@@ -58,7 +58,15 @@ def parse():
                     help="C5 (default) is the metric's workload; C1..C4 time ONE render of that BASELINE.json config: the kernel "
                          "sequence with the plan resident (value), render() from the parameter dict to the float64 result (e2e) "
                          "and the numpy port on one host core (cpu_baseline) -- single GPU only")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the audio the last timed step rendered to DIR/*.npy (float32, at most "
+                         "64 MB; see dump_outputs).  The same arguments give the same inputs, so two builds compare value for value")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes this project's renders; the reference arm keeps none")
+    return args
 
 
 def workload_config(args, extra=None):
@@ -69,6 +77,55 @@ def workload_config(args, extra=None):
     if extra:
         cfg.update(extra)
     return cfg
+
+
+DUMP_RENDER_BYTES = 32 << 20        # whole renders, picked by a fixed seed
+DUMP_SAMPLES = 1 << 22              # float32 values at seeded positions across every render's output (16 MB)
+
+
+def dump_outputs(path, parts, sizes, dist=None):
+    """Writes what a caller of the timed path receives -- float32 stereo audio [frames, 2] per render -- to `path`:
+    render_<i>.npy for whole renders of the sweep picked by a fixed seed (until 32 MB are written) and samples.npy,
+    the values at DUMP_SAMPLES seeded positions of all renders' outputs laid end to end in sweep order.  The picks
+    depend only on `sizes` (float32 values of every render of the sweep, by sweep index), so runs with the same
+    arguments write the same positions however the renders are partitioned.  `parts` = [(BatchRenderer, [sweep index
+    of each of its renders])] for the renders this process holds.  With `dist` (N>1) every rank calls this with its
+    own renders: each writes the picked renders it holds, and rank 0 collects the samples."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    part_of, local = np.full(len(sizes), -1), np.zeros(len(sizes), dtype=np.int64)
+    for j, (b, index) in enumerate(parts):
+        assert np.array_equal(2 * b.tables.out_n.astype(np.int64), sizes[index]), "render lengths differ from `sizes`"
+        part_of[index], local[index] = j, np.arange(len(index))
+    rng = np.random.default_rng(20260)
+    left = DUMP_RENDER_BYTES
+    for i in rng.permutation(len(sizes)):
+        if 4 * sizes[i] <= left:
+            left -= 4 * sizes[i]
+            if part_of[i] >= 0:
+                np.save(os.path.join(path, "render_%05d.npy" % i), parts[part_of[i]][0].output(local[i]).astype(np.float32))
+    ends = np.cumsum(sizes)
+    pos = np.sort(rng.integers(0, int(ends[-1]), min(DUMP_SAMPLES, int(ends[-1]))))
+    i_of = np.searchsorted(ends, pos, side="right")
+    held = np.flatnonzero(part_of[i_of] >= 0)
+    values = np.empty(held.size, dtype=np.float32)
+    for j, (b, _) in enumerate(parts):
+        sel = part_of[i_of[held]] == j
+        i = i_of[held[sel]]
+        at = pos[held[sel]] - (ends - sizes)[i] + 2 * b.tables.out_at[local[i]].astype(np.int64)
+        out = b.outputs_device()
+        values[sel] = out[torch.from_numpy(at).to(out.device)].cpu().numpy()
+    pieces = [(held, values)]
+    if dist is not None:
+        pieces = [None] * dist.get_world_size() if dist.get_rank() == 0 else None
+        dist.gather_object((held, values), pieces, dst=0)
+        if dist.get_rank() != 0:
+            return
+    samples = np.full(pos.size, np.nan, dtype=np.float32)
+    for h, v in pieces:
+        samples[h] = v
+    assert not np.isnan(samples).any(), "some renders of the sweep are held by no rank"
+    np.save(os.path.join(path, "samples.npy"), samples)
 
 
 # ----------------------------------------------------------------------------------------------- clocks
@@ -183,8 +240,6 @@ def run_reference(args):
         v = cpu_pool_throughput(idx, cores)
         if s >= args.warmup:
             vals.append(v)
-        if s >= args.warmup and sum(per_step * FRAMES_PER_RENDER * 2 / x for x in vals) > 150:
-            break
     value = float(np.mean(vals))
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": len(vals),
             "warmup": args.warmup, "ms_per_step": 1e3 * per_step * FRAMES_PER_RENDER * 2 / value, "higher_is_better": True,
@@ -336,6 +391,9 @@ def run_ours(args):
     barrier()
     torch.cuda.profiler.stop()
     wall1 = time.time()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(b, mine[k * per:(k + 1) * per]) for k, b in enumerate(brs)],
+                     np.full(args.renders, 2 * FRAMES_PER_RENDER, dtype=np.int64), dist if world > 1 else None)
     render_only_ms = None
     if use_graph or gather:
         # the same steps without the gather (render only), and one eager pass for the per-stage events: both untimed extras
@@ -547,6 +605,8 @@ def run_single_config(args):
     e1.record()
     torch.cuda.synchronize()
     wall1 = time.time()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(br, [0])], np.array([2 * frames], dtype=np.int64))
     ms = e0.elapsed_time(e1) / args.steps
     launches = (dev.lib.ms_launch_count() - launches0) // args.steps
     clocks = sampler.stop(wall0, wall1)

@@ -436,6 +436,30 @@ def preset_fixture():
     return out
 
 
+def shipped_irs(directory):
+    """The shipped impulse responses the preset fixture carries -- each as the array the reference's on_load_ir rule made
+    of it (main_v2.py:1401-1413: int16 / 32768, mean over channels, normalised to 0.9) -- written back to `directory` as
+    16-bit mono WAV files that this rule maps to exactly that array: the samples are a * peak / 0.9 for the one int16
+    peak that makes every sample an integer.  Returns {path: array}."""
+    import os
+    import wave
+    from conftest import GOLDEN
+    g = np.load(os.path.join(GOLDEN, "presets.npz"))
+    out = {}
+    for key in sorted(k for k in g.files if k.startswith("ir_") and not k.startswith("ir_of_")):
+        a = np.array(g[key])
+        peak = next(q for q in range(1, 32768) if np.max(np.abs(a / 0.9 * q - np.round(a / 0.9 * q))) < 1e-6)
+        path = os.path.join(str(directory), key[3:])
+        with wave.open(path, "wb") as w:
+            w.setnchannels(1)
+            w.setsampwidth(2)
+            w.setframerate(48000)
+            w.writeframes(np.round(a / 0.9 * peak).astype("<i2").tobytes())
+        out[path] = a
+    assert out
+    return out
+
+
 def check_preset(dev, name, fixture=None):
     """One shipped preset through render(): audio against the reference's, progress messages identical, and -- where
     the reference's own output is decided by rounding noise -- the stage-level checks on the device's own input."""

@@ -73,6 +73,10 @@ def test_ir_loader_follows_on_load_ir(tmp_path):
         w.setnchannels(1); w.setsampwidth(3); w.setframerate(48000); w.writeframes(raw)
     a, _ = frontend.read_wav(str(tmp_path / "p24.wav"))
     assert np.array_equal(a, q24.astype(np.float64) / float(2 ** 23))
+    import kernel_checks as K
+    (tmp_path / "irs").mkdir()
+    for path, want in K.shipped_irs(tmp_path / "irs").items():
+        assert np.array_equal(frontend.load_ir_wav(path), want), path
     from oracle import ref_loader
     if ref_loader.available():
         import glob
@@ -84,15 +88,17 @@ def test_ir_loader_follows_on_load_ir(tmp_path):
             assert np.array_equal(frontend.load_ir_wav(f), ref.normalize(s, 0.9)), f
 
 
-def test_shipped_preset_files_merge_like_on_load_preset():
-    from oracle import ref_loader
-    import glob
+def test_shipped_preset_files_merge_like_on_load_preset(tmp_path):
+    """The 27 shipped presets, as the reference's fixture stores them merged (tests/golden/presets.npz): a file with the
+    values that differ from the factory defaults loads to the whole merged set, {**defaults, **file} (main_v2.py:1286-1291)."""
     import json
-    if not ref_loader.available():
-        return
-    files = sorted(glob.glob(os.path.join(ref_loader.REFERENCE_ROOT, "microsound_0.2.1", "presets", "*.json")))
-    assert len(files) == 27
-    for f in files:
-        p = frontend.load_preset(f)
-        raw = json.load(open(f))
-        assert all(p[k] == v for k, v in raw.items()) and set(configs.FACTORY_DEFAULTS) <= set(p)
+    import kernel_checks as K
+    presets = K.preset_fixture()
+    assert len(presets) == 27
+    for name, (merged, *_) in presets.items():
+        merged = {k: v for k, v in merged.items() if not k.startswith("_")}
+        raw = {k: v for k, v in merged.items() if k not in configs.FACTORY_DEFAULTS or configs.FACTORY_DEFAULTS[k] != v}
+        f = tmp_path / (name + ".json")
+        f.write_text(json.dumps(raw))
+        p = frontend.load_preset(str(f))
+        assert all(p[k] == v for k, v in merged.items()) and set(configs.FACTORY_DEFAULTS) <= set(p), name

@@ -1,5 +1,6 @@
 """The oracle (oracle/microsound_np.py) against (a) the unmodified reference where it exists (build
 container) and (b) the golden fixtures the reference produced (tests/golden, oracle/make_golden.py)."""
+import functools
 import os
 
 import numpy as np
@@ -104,22 +105,35 @@ def test_oracle_matches_reference(name, params):
     assert ma["out_sr"] == mb["out_sr"] and ma["design_sr_base"] == mb["design_sr_base"]
 
 
-@needs_ref
+@functools.lru_cache(maxsize=1)
+def _preset_fixture():
+    import kernel_checks as K
+    return K.preset_fixture()
+
+
 def test_oracle_progress_calls_match_reference():
-    ref = ref_loader.load()
-    p = configs.with_defaults(event_process="Poisson", out_dur_s=6.0, grains_per_sec=30.0)
-    a, b = [], []
-    ref.render(p, progress=lambda pct, msg: a.append((pct, msg)))
-    O.render(p, progress=lambda pct, msg: b.append((pct, msg)))
-    assert a == b and len(a) >= 4
+    """The (pct, msg) calls the reference made while rendering the 27 shipped presets (tests/golden/presets.npz)."""
+    longest = 0
+    for name, (p, _, _, _, msgs) in sorted(_preset_fixture().items()):
+        b = []
+        O.render(p, progress=lambda pct, msg: b.append((int(pct), str(msg))))
+        assert b == msgs, name
+        longest = max(longest, len(b))
+    assert longest >= 4
 
 
-@needs_ref
-def test_ir_loader_matches_shipped_files():
-    d = os.path.join(ref_loader.REFERENCE_ROOT, "microsound_0.2.1", "irs")
-    for f in sorted(os.listdir(d)):
-        a = ref_loader.load_ir_wav(os.path.join(d, f))
-        assert a.ndim == 1 and abs(np.max(np.abs(a)) - 0.9) < 1e-12
+def test_ir_loader_matches_shipped_files(tmp_path):
+    """The shipped impulse responses, rebuilt from what the preset fixture stores of them (kernel_checks.shipped_irs),
+    load to the stored arrays; the files themselves too where the reference is present."""
+    import kernel_checks as K
+    for path, want in K.shipped_irs(tmp_path).items():
+        a = ref_loader.load_ir_wav(path)
+        assert a.ndim == 1 and abs(np.max(np.abs(a)) - 0.9) < 1e-12 and np.array_equal(a, want), path
+    if ref_loader.available():
+        d = os.path.join(ref_loader.REFERENCE_ROOT, "microsound_0.2.1", "irs")
+        for f in sorted(os.listdir(d)):
+            a = ref_loader.load_ir_wav(os.path.join(d, f))
+            assert a.ndim == 1 and abs(np.max(np.abs(a)) - 0.9) < 1e-12
 
 
 # ---------------------------------------------------------------- SURVEY 8(f) rows accelerated so far
@@ -149,7 +163,6 @@ def test_wavelet_grain_shorter_than_its_atoms_fails_like_the_reference():
         P.plan_render(configs.with_defaults(gen_mode="Wavelet atoms", time_unfold=1.0, micro_ms=1.0))
 
 
-@needs_ref
 @pytest.mark.parametrize("name", ["opal_airfold", "opal_oval_breath", "basinski_melodic_loop", "basinski_oval_decay",
                                   "soft_ellipse_memory", "micro_carillon", "oval_glass_orbit", "glass_harmonic_arc",
                                   "01_corona_glass_fog", "corona_memory_glass", "melodic_dust_chime", "oval_room_trace",
@@ -159,17 +172,25 @@ def test_wavelet_grain_shorter_than_its_atoms_fails_like_the_reference():
                                   "infra_tone_lattice", "03_wavelet_ice_bloom", "orbital_friction_loop",
                                   "02_friction_lattice", "friction_lattice", "wavelet_mist"])
 def test_oracle_matches_reference_on_shipped_presets(name):
-    """The shipped presets that need only accelerated rows, merged over the factory defaults the way on_load_preset
-    does (main_v2.py:1286-1291), first 1.5 s."""
-    import json
-    ref = ref_loader.load()
-    path = os.path.join(ref_loader.REFERENCE_ROOT, "microsound_0.2.1", "presets", name + ".json")
-    p = configs.with_defaults(json.load(open(path)))
-    p["out_dur_s"] = 1.5
-    if name == "oval_room_trace":
-        p["_ir_audio"] = configs.synth_ir(0.25, 48000, 11, channels=1)
-    if name == "image_grain_hallucination":
-        p["_img_gray"] = np.random.default_rng(5).integers(0, 256, (40, 300)).astype(np.uint8)
-    a, ma = ref.render(p)
-    b, mb = O.render(p)
-    assert np.max(np.abs(a - b)) < TOL and np.max(np.abs(ma["grain_last"] - mb["grain_last"])) < TOL
+    """The shipped presets, merged over the factory defaults the way on_load_preset does (main_v2.py:1286-1291), with
+    the shipped impulse responses: 2 s renders of the reference, every 8th frame stored as float32
+    (tests/golden/presets.npz, oracle/make_golden_presets.py).  The oracle must match to TOL beyond that rounding.
+    Where the reference is present, also every frame and grain_last of its own 1.5 s float64 renders, to TOL."""
+    p, want, step, _, _ = _preset_fixture()[name]
+    b, _ = O.render(p)
+    half_ulp = 0.5 * np.spacing(np.abs(want)).astype(np.float64)
+    assert b[::step].shape == want.shape
+    assert np.max(np.abs(b[::step] - want.astype(np.float64)) - half_ulp) < TOL
+    if ref_loader.available():
+        import json
+        ref = ref_loader.load()
+        path = os.path.join(ref_loader.REFERENCE_ROOT, "microsound_0.2.1", "presets", name + ".json")
+        p = configs.with_defaults(json.load(open(path)))
+        p["out_dur_s"] = 1.5
+        if name == "oval_room_trace":
+            p["_ir_audio"] = configs.synth_ir(0.25, 48000, 11, channels=1)
+        if name == "image_grain_hallucination":
+            p["_img_gray"] = np.random.default_rng(5).integers(0, 256, (40, 300)).astype(np.uint8)
+        a, ma = ref.render(p)
+        b, mb = O.render(p)
+        assert np.max(np.abs(a - b)) < TOL and np.max(np.abs(ma["grain_last"] - mb["grain_last"])) < TOL

@@ -173,7 +173,8 @@ static void bandpass_edge(ms_band_edge& e, double sr, double lo, double hi, doub
     }
 }
 
-struct Item { int64_t n, src, dst; ms_spec_op op; };
+struct Item { int64_t n, src, dst; ms_spec_op op; };         // tables.SPEC_ITEM: exported as it is
+static_assert(sizeof(Item) == 3 * sizeof(int64_t) + sizeof(ms_spec_op), "Item must have no padding");
 struct Plan {
     std::vector<ms_synth_evt> sy1, sy2;
     std::vector<ms_ola_render> ola_r, env_reps;
@@ -632,17 +633,9 @@ void ms_hp_sizes(void* h, int64_t* sizes, int64_t* scalars /*pool_n mono_n frame
     scalars[5] = P->max_out_n; scalars[6] = P->env_n;
     for (int i = 0; i < 7; ++i) scalars[7 + i] = P->alg[i];
 }
-static void put_items(const std::vector<Item>& v, int64_t* n, int64_t* src, int64_t* dst, void* ops) {
-    for (size_t i = 0; i < v.size(); ++i) {
-        n[i] = v[i].n; src[i] = v[i].src; dst[i] = v[i].dst;
-        memcpy((char*)ops + i * sizeof(ms_spec_op), &v[i].op, sizeof(ms_spec_op));
-    }
-}
 void ms_hp_export(void* h, void* sy1, void* sy2, void* ola_r, void* env_reps, void* ola_e, void* fir, void* post,
                   int32_t* tap_off, double* tap_delay, double* tap_raw, int32_t* dust_pos, double* dust_val,
-                  int64_t* tilt_n, int64_t* tilt_src, int64_t* tilt_dst, void* tilt_ops,
-                  int64_t* grain_n, int64_t* grain_src, int64_t* grain_dst, void* grain_ops,
-                  int64_t* rot_n, int64_t* rot_src, int64_t* rot_dst, void* rot_ops,
+                  void* tilt, void* grain, void* rot,
                   int64_t* odd, int64_t* ir_order, int64_t* out_at, int64_t* out_n, int64_t* y_at, int64_t* last, int64_t* srs) {
     Plan* P = (Plan*)h;
     auto cp = [](void* d, const void* s, size_t b) { if (b) memcpy(d, s, b); };
@@ -652,9 +645,8 @@ void ms_hp_export(void* h, void* sy1, void* sy2, void* ola_r, void* env_reps, vo
     cp(post, P->post.data(), P->post.size() * sizeof(ms_post_render));
     cp(tap_off, P->tap_off.data(), P->tap_off.size() * 4); cp(tap_delay, P->tap_delay.data(), P->tap_delay.size() * 8); cp(tap_raw, P->tap_raw.data(), P->tap_raw.size() * 8);
     cp(dust_pos, P->dust_pos.data(), P->dust_pos.size() * 4); cp(dust_val, P->dust_val.data(), P->dust_val.size() * 8);
-    put_items(P->tilt, tilt_n, tilt_src, tilt_dst, tilt_ops);
-    put_items(P->grain, grain_n, grain_src, grain_dst, grain_ops);
-    put_items(P->rot, rot_n, rot_src, rot_dst, rot_ops);
+    cp(tilt, P->tilt.data(), P->tilt.size() * sizeof(Item)); cp(grain, P->grain.data(), P->grain.size() * sizeof(Item));
+    cp(rot, P->rot.data(), P->rot.size() * sizeof(Item));
     cp(odd, P->odd.data(), P->odd.size() * 8); cp(ir_order, P->ir_order.data(), P->ir_order.size() * 8);
     cp(out_at, P->out_at.data(), P->out_at.size() * 8); cp(out_n, P->out_n.data(), P->out_n.size() * 8); cp(y_at, P->y_at.data(), P->y_at.size() * 8);
     cp(last, P->last.data(), P->last.size() * 8); cp(srs, P->srs.data(), P->srs.size() * 8);

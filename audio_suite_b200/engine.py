@@ -212,6 +212,8 @@ class BatchRenderer:
         self.h2d_bytes = getattr(self.dev, "uploaded", 0) + self.dev.lib.ms_h2d_bytes() - up0
 
     # ---- device buffers + native plans -----------------------------------------------------------------
+    cep_stages, plock_stage, imprint_stage = (), None, None          # batches without these stages
+
     def _upload(self, T):
         import os as _os, time as _time
         dev, t, real = self.dev, self.tables, self.real
@@ -223,7 +225,7 @@ class BatchRenderer:
                 _tr.append((name, _time.perf_counter() - _t0))
         self.n_renders, self.n_evt, self.frames = len(t.post), len(t.sy1), t.frames
         self.max_out_n, self.max_h = t.max_out_n, t.max_h
-        self.any_dust, self.any_tilt = t.dust_pos.size > 0, t.tilt[0].size > 0
+        self.any_dust, self.any_tilt = t.dust_pos.size > 0, len(t.tilt) > 0
         self.n_fir = len(t.fir)
         self.pool = dev.empty(t.pool_n, real)
         self.mono = dev.zeros(t.mono_n, real)
@@ -262,138 +264,83 @@ class BatchRenderer:
         if self.any_dust:
             self.d_dpos, self.d_dval = dev.upload(t.dust_pos), dev.upload(t.dust_val.astype(real))
         _mark("uploads")
-        self.tilt_stage = _SpectralStage(dev, self.api, T.pair_jobs(t.tilt), self.pool, self.pool)
-        self.grain_stage = _SpectralStage(dev, self.api, T.pair_jobs(t.grain), self.pool, self.pool)
-        self.rot_stage = _SpectralStage(dev, self.api, T.pair_jobs(t.rot), self.mono, self.mono)
+        stage = lambda jobs, buf: _SpectralStage(dev, self.api, jobs, buf, buf)     # noqa: E731
+        self.tilt_stage = stage(T.pair_jobs(t.tilt), self.pool)
+        self.grain_stage = stage(T.pair_jobs(t.grain), self.pool)
+        self.rot_stage = stage(T.pair_jobs(t.rot), self.mono)
         # resonator bank / waveguide (time domain) and the multiband unfold that follows them
-        self.n_res = self.n_wg = 0
-        self.post_stage = None
-        if t.wg is not None and len(t.wg[0]):
-            rows, lines = t.wg
-            ev = np.zeros(len(rows), np.dtype(_abi.WgEvt))
-            ev["src"], ev["dst"], ev["n"], ev["line_begin"], ev["line_count"] = rows[:, 0], rows[:, 1], rows[:, 2], rows[:, 3], rows[:, 4]
-            ln = np.zeros(len(lines), np.dtype(_abi.WgLine))
-            ln["d"], ln["g"], ln["mix"] = lines[:, 0].astype(np.int64), lines[:, 1], lines[:, 2]
-            self.d_wg_evt, self.d_wg_lines, self.n_wg = dev.upload(ev), dev.upload(ln), len(rows)
-        if t.post_grain is not None and len(t.post_grain[0]):
-            self.post_stage = _SpectralStage(dev, self.api, T.pair_jobs(t.post_grain), self.pool, self.pool)
-        if t.res is not None and len(t.res[0]):
-            rows, decay, modes = t.res
-            ev = np.zeros(len(rows), np.dtype(_abi.ResEvt))
-            ev["src"], ev["dst"], ev["n"], ev["mode_begin"], ev["mode_count"], ev["decay"] = rows[:, 0], rows[:, 1], rows[:, 2], rows[:, 3], rows[:, 4], decay
-            self.d_res_evt, self.d_res_modes, self.n_res = dev.upload(ev), dev.upload(np.ascontiguousarray(modes)), len(rows)
-            self.h_res_evt = ev
-        # cepstral warp: three stages of single-signal jobs around the elementwise steps of ms_cepstral
-        self.cep_stages = None
-        if t.cep is not None and len(t.cep[0]):
-            rows, factor, pre, post = t.cep
-            N = len(rows)
-            n = rows[:, 2]
-            bins = n // 2 + 1
-            xp_len = (2 * bins + 3) // 4 * 4
-            per = xp_len + 2 * ((n + 3) // 4 * 4)
-            base = np.concatenate([[0], np.cumsum(per)])
-            xp, cep, cep2 = base[:-1], base[:-1] + xp_len, base[:-1] + xp_len + (n + 3) // 4 * 4
+        self.n_res, self.n_wg = len(t.res), len(t.wg)
+        if self.n_wg:
+            self.d_wg_evt, self.d_wg_lines = dev.upload(t.wg), dev.upload(t.wg_lines)
+        self.post_stage = stage(T.pair_jobs(t.post_grain), self.pool)
+        if self.n_res:
+            self.d_res_evt, self.d_res_modes, self.h_res_evt = dev.upload(t.res), dev.upload(t.res_modes), t.res
+        # cepstral warp: three stages of single-signal jobs around the elementwise steps of ms_cepstral; the outer one
+        # transforms the grain, the inner two work in a scratch of [spectrum | cepstrum | warped cepstrum] per grain
+        self.n_cep = len(t.cep)
+        if self.n_cep:
+            ev = t.cep.copy()
+            n = ev["n"].astype(np.int64)
+            xp_len, cep_len = (2 * (n // 2 + 1) + 3) // 4 * 4, (n + 3) // 4 * 4
+            base = np.concatenate([[0], np.cumsum(xp_len + 2 * cep_len)])
+            ev["xp"], ev["cep"], ev["cep2"] = base[:-1], base[:-1] + xp_len, base[:-1] + xp_len + cep_len
             self.cep_scratch = dev.empty(int(base[-1]), real)
-
-            def mk_jobs(in_a, out_a, ops=None):
-                jobs = np.zeros(N, np.dtype(_abi.SpecJob))
-                jobs["n"], jobs["in_a"], jobs["out_a"], jobs["in_b"], jobs["out_b"] = n, in_a, out_a, -1, -1
-                if ops is not None:
-                    raw = jobs.view(np.uint8).reshape(N, jobs.dtype.itemsize)
-                    o0 = jobs.dtype.fields["op"][1]
-                    raw[:, o0:o0 + ops.shape[1]] = ops
-                return jobs
-            s1 = _SpectralStage(dev, self.api, mk_jobs(rows[:, 0], rows[:, 1], post), self.pool, self.pool)
-            s2 = _SpectralStage(dev, self.api, mk_jobs(cep, cep), self.cep_scratch, self.cep_scratch)     # inverse only
-            s3 = _SpectralStage(dev, self.api, mk_jobs(cep2, cep2), self.cep_scratch, self.cep_scratch)   # forward only
-            self.cep_stages = (s1, s2, s3)
-            ev = np.zeros(N, np.dtype(_abi.CepEvt))
-            zb = []
+            inner = np.zeros(self.n_cep, T.SPEC_ITEM)
+            inner["n"] = n
+            self.cep_stages = [stage(T.single_jobs(t.cep_items), self.pool)]
+            for at in (ev["cep"], ev["cep2"]):                       # inverse only, forward only
+                inner["src"] = inner["dst"] = at
+                self.cep_stages.append(stage(T.single_jobs(inner), self.cep_scratch))
+            self.cep_zb = []
             for name, st_ in zip(("z1", "z2", "z3"), self.cep_stages):
-                b0, offs = st_.z_table()
-                ev[name] = offs
-                zb.append(b0)
-            ev["xp"], ev["cep"], ev["cep2"], ev["n"], ev["factor"] = xp, cep, cep2, n, factor
-            rawe = ev.view(np.uint8).reshape(N, ev.dtype.itemsize)
-            p0 = ev.dtype.fields["pre"][1]
-            rawe[:, p0:p0 + pre.shape[1]] = pre
-            self.d_cep_evt, self.n_cep, self.cep_max_n, self.cep_zb = dev.upload(ev), N, int(n.max()), zb
-            self.h_cep_evt = ev
+                b0, ev[name] = st_.z_table()
+                self.cep_zb.append(b0)
+            self.d_cep_evt, self.cep_max_n, self.h_cep_evt = dev.upload(ev), int(n.max()), ev
         # partial lock: single-signal jobs from the event's raw transient; low-pass / warp are evaluated by the
         # lock kernel on the forward spectrum, the inverse applies what follows it (multiband)
-        self.plock_stage = None
-        if t.plock is not None and len(t.plock[0]):
-            rows, factor, pre, post = t.plock
-            jobs = np.zeros(len(rows), np.dtype(_abi.SpecJob))
-            jobs["n"], jobs["in_a"], jobs["out_a"], jobs["in_b"], jobs["out_b"] = rows[:, 2], rows[:, 0], rows[:, 1], -1, -1
-            raw = jobs.view(np.uint8).reshape(len(rows), jobs.dtype.itemsize)
-            op0 = jobs.dtype.fields["op"][1]
-            raw[:, op0:op0 + post.shape[1]] = post
-            self.plock_stage = _SpectralStage(dev, self.api, jobs, self.pool, self.pool)
-            zbase, zoffs = self.plock_stage.z_table()
-            ev = np.zeros(len(rows), np.dtype(_abi.PlockEvt))
-            bins = rows[:, 2] // 2 + 1
+        self.n_plock = len(t.plock)
+        if self.n_plock:
+            self.plock_stage = stage(T.single_jobs(t.plock_items), self.pool)
+            ev = t.plock.copy()
+            self.plock_zbase, ev["z"] = self.plock_stage.z_table()
+            bins = ev["n"].astype(np.int64) // 2 + 1
             scr = np.concatenate([[0], np.cumsum((3 * bins + 3) // 4 * 4)])       # 16-byte aligned complex scratch per grain
-            ev["z"], ev["scratch"], ev["n"], ev["top_n"], ev["neigh"], ev["factor"] = zoffs, scr[:-1], rows[:, 2], rows[:, 3], rows[:, 4], factor
-            rawe = ev.view(np.uint8).reshape(len(rows), ev.dtype.itemsize)
-            p0 = ev.dtype.fields["pre"][1]
-            rawe[:, p0:p0 + pre.shape[1]] = pre
-            self.d_plock_evt, self.n_plock = dev.upload(ev), len(rows)
+            ev["scratch"] = scr[:-1]
+            self.d_plock_evt = dev.upload(ev)
             self.plock_scratch = dev.empty(int(scr[-1]), real)
-            self.plock_zbase = zbase
         # event feedback (+ imprint): the events of a render depend on each other, so they are processed rank by rank
         # (rank e of all renders together): feedback kernel, then -- with the imprint on -- forward / one-grain step /
-        # inverse on a spectral stage of that rank's grains
+        # inverse on a spectral stage of that rank's grains; the step keeps one moving average per render (its slot)
         self.seq_ranks = []
-        if t.seq is not None and len(t.seq):
+        if len(t.seq):
             sq = t.seq
-            renders = np.unique(sq[:, 0].astype(np.int64))
-            slot_of = {int(rr): i for i, rr in enumerate(renders)}
-            self.seq_max_bins = int(sq[:, 7].max()) // 2 + 1
+            renders, slot = np.unique(sq["render"], return_inverse=True)
+            self.seq_max_bins = int(sq["fb"]["n_cur"].max()) // 2 + 1
             self.seq_mem = dev.zeros(len(renders) * self.seq_max_bins, real)
             self.seq_prev_bins = dev.zeros(len(renders), np.int32)
-            for e in np.unique(sq[:, 1].astype(np.int64)):
-                rows = sq[sq[:, 1] == e]
-                fbr = rows[rows[:, 5] >= 0]
-                item = {"n_fb": len(fbr), "n_imp": 0}
-                if len(fbr):
-                    ev = np.zeros(len(fbr), np.dtype(_abi.FeedbackEvt))
-                    ev["cur"], ev["prev"], ev["dst"], ev["n_cur"], ev["n_prev"], ev["fb"] = fbr[:, 2], fbr[:, 3], fbr[:, 5], fbr[:, 7], fbr[:, 4], fbr[:, 8]
-                    item["d_fb"], item["fb_max_n"] = dev.upload(ev), int(fbr[:, 7].max())
-                imr = rows[rows[:, 6] >= 0]
-                if len(imr):
-                    src = np.where(imr[:, 5] >= 0, imr[:, 5], imr[:, 2]).astype(np.int64)        # the fed-back grain, or the grain itself at rank 0
-                    jobs = np.zeros(len(imr), np.dtype(_abi.SpecJob))
-                    jobs["n"], jobs["in_a"], jobs["out_a"], jobs["in_b"], jobs["out_b"] = imr[:, 7].astype(np.int64), src, imr[:, 6].astype(np.int64), -1, -1
-                    stg = _SpectralStage(dev, self.api, jobs, self.pool, self.pool)
-                    zbase, zoffs = stg.z_table()
-                    iv = np.zeros(len(imr), np.dtype(_abi.ImprintStepEvt))
-                    iv["z"], iv["n"], iv["amount"], iv["smooth"] = zoffs, imr[:, 7].astype(np.int64), imr[:, 9], imr[:, 10]
-                    iv["slot"] = [slot_of[int(rr)] for rr in imr[:, 0]]
-                    item.update(n_imp=len(imr), stage=stg, zbase=zbase, d_imp=dev.upload(iv), h_imp=iv)
+            for e in np.unique(sq["rank"]):
+                at = sq["rank"] == e
+                fb = sq["fb"][at & (sq["fb"]["dst"] >= 0)]
+                item = {"n_fb": len(fb), "n_imp": 0}
+                if len(fb):
+                    item["d_fb"], item["fb_max_n"] = dev.upload(fb), int(fb["n_cur"].max())
+                at &= sq["imp_item"]["dst"] >= 0
+                if at.any():
+                    stg = stage(T.single_jobs(sq["imp_item"][at]), self.pool)
+                    iv = sq["imp"][at]
+                    zbase, iv["z"] = stg.z_table()
+                    iv["slot"] = slot[at]
+                    item.update(n_imp=len(iv), stage=stg, zbase=zbase, d_imp=dev.upload(iv), h_imp=iv)
                 self.seq_ranks.append(item)
         # spectral imprint: single-signal jobs (Z = the grain's DFT), forward -> per-render moving average -> inverse
-        self.imprint_stage, self.n_imprint_renders = None, 0
+        self.n_imprint_renders = len(t.imprint_r)
         if len(t.imprint):
-            rows = t.imprint
-            jobs = np.zeros(len(rows), np.dtype(_abi.SpecJob))
-            jobs["n"], jobs["in_a"], jobs["out_a"], jobs["in_b"], jobs["out_b"] = rows[:, 3], rows[:, 1], rows[:, 2], -1, -1
-            self.imprint_stage = _SpectralStage(dev, self.api, jobs, self.pool, self.pool)
-            zbase, zoffs = self.imprint_stage.z_table()
-            ev = np.zeros(len(rows), np.dtype(_abi.ImprintEvt))
-            ev["z"], ev["n"] = zoffs, rows[:, 3]
-            renders = np.unique(rows[:, 0])
-            first = np.searchsorted(rows[:, 0], renders, side="left")
-            last = np.searchsorted(rows[:, 0], renders, side="right")
-            rr = np.zeros(len(renders), np.dtype(_abi.ImprintRender))
-            rr["ev_begin"], rr["ev_end"] = first, last
-            rr["amount"], rr["smooth"] = t.imprint_par[renders, 0], t.imprint_par[renders, 1]
-            self.d_imp_evt, self.d_imp_render = dev.upload(ev), dev.upload(rr)
-            self.h_imp_evt, self.h_imp_render = ev, rr
-            self.n_imprint_renders = len(renders)
-            self.imprint_max_bins = int(rows[:, 3].max()) // 2 + 1
-            self.imprint_zbase = zbase
+            self.imprint_stage = stage(T.single_jobs(t.imprint_items), self.pool)
+            ev = t.imprint.copy()
+            self.imprint_zbase, ev["z"] = self.imprint_stage.z_table()
+            self.d_imp_evt, self.d_imp_render = dev.upload(ev), dev.upload(t.imprint_r)
+            self.h_imp_evt, self.h_imp_render = ev, t.imprint_r
+            self.imprint_max_bins = int(ev["n"].max()) // 2 + 1
         _mark("spectral_create")
         self.fir_handle = C.c_void_p(None)
         if self.n_fir:
@@ -444,7 +391,7 @@ class BatchRenderer:
                 mark("tilt_spectral")
             self.grain_stage.run()
             mark("grain_spectral")
-            if self.cep_stages is not None:
+            if self.n_cep:
                 s1, s2, s3 = self.cep_stages
                 zp = [C.c_void_p(dev.ptr(s_.ws).value + b0) for s_, b0 in zip(self.cep_stages, self.cep_zb)]
                 args = (dev.ptr(self.d_cep_evt), self.n_cep, self.cep_max_n, zp[0], zp[1], zp[2], dev.ptr(self.cep_scratch), st)
@@ -458,7 +405,7 @@ class BatchRenderer:
                 probe("cep_y")
                 s1.inverse()
                 mark("cepstral_warp")
-            if self.plock_stage is not None:
+            if self.n_plock:
                 self.plock_stage.forward()
                 zptr = C.c_void_p(dev.ptr(self.plock_stage.ws).value + self.plock_zbase)
                 _check(dev, lib.ms_partial_lock(dev.ptr(self.d_plock_evt), self.n_plock, zptr, dev.ptr(self.plock_scratch), st))
@@ -472,8 +419,7 @@ class BatchRenderer:
             if self.n_wg:
                 _check(dev, lib.ms_waveguide(dev.ptr(self.d_wg_evt), self.n_wg, dev.ptr(self.d_wg_lines), dev.ptr(self.pool), st))
             if self.n_res or self.n_wg:
-                if self.post_stage is not None:
-                    self.post_stage.run()
+                self.post_stage.run()
                 mark("resonator_waveguide")
             if self.seq_ranks:
                 self.seq_prev_bins.fill_(-1) if hasattr(self.seq_prev_bins, "fill_") else self.seq_prev_bins.fill(-1)
@@ -563,7 +509,7 @@ class BatchRenderer:
     def meta(self, r):
         t = self.tables
         m = dict(out_sr=int(t.srs[r, 0]), design_sr_base=int(t.srs[r, 1]), micro_last=None, grain_last=None)
-        micro, grain, n = (int(v) for v in t.last[r])
+        micro, grain, n = t.last[r].tolist()
         if n > 0:
             m["micro_last"] = np.asarray(self.dev.download(self.pool, micro, n)).astype(np.float64)
             m["grain_last"] = np.asarray(self.dev.download(self.pool, grain, n)).astype(np.float64)
@@ -571,7 +517,7 @@ class BatchRenderer:
 
     def close(self):
         for s in (self.tilt_stage, self.grain_stage, self.rot_stage, self.imprint_stage, self.plock_stage, self.post_stage) + \
-                tuple(self.cep_stages or ()) + tuple(it["stage"] for it in getattr(self, "seq_ranks", []) if it["n_imp"]):
+                tuple(self.cep_stages) + tuple(it["stage"] for it in getattr(self, "seq_ranks", []) if it["n_imp"]):
             if s is not None:
                 s.close()
         if self.fir_handle:

@@ -28,7 +28,7 @@ FIELDS = ("base_sr", "out_dur_s", "time_unfold", "peak", "sat_drive", "stereo_on
 _MODE = {m: float(i) for i, m in enumerate(BASIC_MODES)}
 _PROCESS = {"Single": 0.0, "Poisson": 1.0}
 _OFF_FLAGS = ("partial_lock_on", "cep_warp_on", "res_bank_on", "wg_on", "event_feedback_on", "spectral_imprint_on")
-_HP_NAMES = ("sy", "ola_r", "env_reps", "ola_e", "fir", "post", "taps", "dust", "tilt", "grain", "rot", "odd", "irs")
+_HP_NAMES = ("sy1", "ola_r", "env_reps", "ola_e", "fir", "post", "tap_off", "dust_pos", "tilt", "grain", "rot", "odd", "irs")   # ms_hp_sizes
 
 _lib = None
 
@@ -47,7 +47,7 @@ def lib():
             l.ms_hp_error.restype = C.c_char_p
             l.ms_hp_error.argtypes = [C.c_void_p, C.POINTER(C.c_int)]
             l.ms_hp_sizes.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
-            l.ms_hp_export.argtypes = [C.c_void_p] * 32
+            l.ms_hp_export.argtypes = [C.c_void_p] * 23
             l.ms_hp_free.argtypes = [C.c_void_p]
             l.ms_hp_pcg64_seed.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
             l.ms_hp_draws.argtypes = [C.c_int64, C.c_int, C.c_uint64, C.c_int, C.c_void_p]
@@ -214,42 +214,21 @@ def plan_chunk(params_list, threads=1):
         sc = np.zeros(14, np.int64)
         l.ms_hp_sizes(h, sizes.ctypes.data, sc.ctypes.data)
         n = dict(zip(_HP_NAMES, sizes.tolist()))
-        OPB = T._SPEC_OP_BYTES
         t = T.Tables()
-        t.sy1, t.sy2 = T._recs(_abi.SynthEvt, n["sy"]), T._recs(_abi.SynthEvt, n["sy"])
-        t.ola_r, t.env_reps = T._recs(_abi.OlaRender, n["ola_r"]), T._recs(_abi.OlaRender, n["env_reps"])
-        t.ola_e, t.fir, t.post = T._recs(_abi.OlaEvt, n["ola_e"]), T._recs(_abi.FirRender, n["fir"]), T._recs(_abi.PostRender, n["post"])
-        t.tap_off = np.zeros(n["taps"], np.int32)
-        delay, raw = np.zeros(n["taps"]), np.zeros(n["taps"])
-        t.dust_pos, t.dust_val = np.zeros(n["dust"], np.int32), np.zeros(n["dust"])
-        items = {}
-        for k in ("tilt", "grain", "rot"):
-            items[k] = (np.zeros(n[k], np.int64), np.zeros(n[k], np.int64), np.zeros(n[k], np.int64), np.zeros((n[k], OPB), np.uint8))
-        t.odd = np.zeros((n["odd"], 4), np.int64)
-        ir_order = np.zeros(n["irs"], np.int64)
+        n["sy2"], n["dust_val"] = n["sy1"], n["dust_pos"]
+        for k in ("sy1", "sy2", "ola_r", "env_reps", "ola_e", "fir", "post", "tap_off", "dust_pos", "dust_val", "tilt", "grain", "rot", "odd"):
+            setattr(t, k, np.zeros(n[k], getattr(t, k).dtype))
+        delay, raw, ir_order = np.zeros(n["tap_off"]), np.zeros(n["tap_off"]), np.zeros(n["irs"], np.int64)
         t.out_at, t.out_n, t.y_at = np.zeros(R, np.int64), np.zeros(R, np.int64), np.zeros(R, np.int64)
-        t.last, t.srs = np.zeros((R, 3), np.int64), np.zeros((R, 2), np.int64)
-        ptr = lambda a: a.ctypes.data          # noqa: E731
-        args = [t.sy1, t.sy2, t.ola_r, t.env_reps, t.ola_e, t.fir, t.post, t.tap_off, delay, raw, t.dust_pos, t.dust_val]
-        for k in ("tilt", "grain", "rot"):
-            args += list(items[k])
-        args += [t.odd, ir_order, t.out_at, t.out_n, t.y_at, t.last, t.srs]
-        l.ms_hp_export(h, *[ptr(a) for a in args])
+        t.last, t.srs = np.zeros(R, T.LAST), np.zeros((R, 2), np.int64)
+        args = [t.sy1, t.sy2, t.ola_r, t.env_reps, t.ola_e, t.fir, t.post, t.tap_off, delay, raw, t.dust_pos, t.dust_val,
+                t.tilt, t.grain, t.rot, t.odd, ir_order, t.out_at, t.out_n, t.y_at, t.last, t.srs]
+        l.ms_hp_export(h, *[a.ctypes.data for a in args])
     finally:
         l.ms_hp_free(h)
     # gains *= exp(-delays * 42) (main_v2.py:415) with numpy's own exp, as the reference computes it
     t.tap_gain = raw * np.exp(-delay * 42.0)
     t.irs = np.concatenate([np.ones(1) if k == -2 else irs[k] for k in ir_order.tolist()]).astype(np.float64) if n["irs"] else np.zeros(0)
-    t.tilt, t.grain, t.rot = items["tilt"], items["grain"], items["rot"]
-    t.atoms, t.atom_shift = np.zeros((0, 4)), np.zeros(0, np.int32)
-    z8 = np.zeros((0, OPB), np.uint8)
-    t.plock = (np.zeros((0, 5), np.int64), np.zeros(0), z8, z8)
-    t.cep = (np.zeros((0, 3), np.int64), np.zeros(0), z8, z8)
-    t.res = (np.zeros((0, 5), np.int64), np.zeros(0), np.zeros((0, 3)))
-    t.wg = (np.zeros((0, 5), np.int64), np.zeros((0, 3)))
-    t.seq = np.zeros((0, 11))
-    t.post_grain = (np.zeros(0, np.int64), np.zeros(0, np.int64), np.zeros(0, np.int64), z8)
-    t.imprint, t.imprint_par = np.zeros((0, 4), np.int64), np.full((R, 2), np.nan)
     t.pool_n, t.mono_n, t.frames, t.h_total, t.max_h, t.max_out_n, t.env_n = (int(v) for v in sc[:7])
     t.alg = dict(zip(("synth", "tilt_spectral", "grain_spectral", "overlap_add", "fir_in", "fir_taps", "post"), (int(v) for v in sc[7:])))
     return t

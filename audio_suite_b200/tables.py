@@ -2,9 +2,13 @@
 
 `pack_chunk(plans)` lays a list of render plans out in chunk-local coordinates (every offset starts at
 0) and returns plain numpy arrays, so chunks can be built by worker processes and pickled cheaply;
-`merge_chunks` concatenates them, shifts every offset field by the chunk's base in its buffer, and pairs
-the spectral jobs across the whole batch (two signals of equal length share one complex transform).
-A single in-process chunk goes through exactly the same code.
+`merge_chunks` concatenates them and shifts every offset field (RELOC) by the chunk's base in its buffer.
+`pair_jobs` / `single_jobs` turn spectral items into the device's job records (two signals of equal
+length share one complex transform).  A single in-process chunk goes through exactly the same code.
+
+Every table is a record array with the layout of its struct in include/microsound_b200.h (SpecItem:
+`struct Item` of csrc/ms_hostplan.cpp), so it is uploaded as it stands.  Fields only the device
+workspace can supply (the `z*` spectrum offsets, scratch offsets) stay 0 here and are filled on upload.
 
 Buffers (offsets in elements): pool (real; per-event signals), mono (real; per chunk:
 [OLA plane | FIR plane | right channels / odd-length scratch]), out (float32 frames), hpool (real;
@@ -14,7 +18,7 @@ from __future__ import annotations
 
 import math
 import os
-from dataclasses import dataclass, field
+from dataclasses import dataclass, field, fields
 
 import numpy as np
 
@@ -24,9 +28,30 @@ _SPEC_OP_BYTES = np.dtype(_abi.SpecOp).itemsize
 _SPEC_JOB = np.dtype(_abi.SpecJob)
 _ZERO_OP = np.zeros(_SPEC_OP_BYTES, np.uint8)
 
+# one spectral work item: a signal of n samples from pool[src] to pool[dst] through one operator
+SPEC_ITEM = np.dtype([("n", np.int64), ("src", np.int64), ("dst", np.int64), ("op", np.uint8, (_SPEC_OP_BYTES,))])
+# odd-length stereo: rolled copy of mono[y_at : y_at + n] by dr into mono[scratch]
+ODD = np.dtype([("y_at", np.int64), ("scratch", np.int64), ("n", np.int64), ("dr", np.int64)])
+# per render: pool offsets of the last event's raw and final grain (-1 if none), its length
+LAST = np.dtype([("micro", np.int64), ("grain", np.int64), ("n", np.int64)])
+# one event of a render with event feedback, processed rank by rank: feedback from the previous event's final grain
+# (fb.dst = -1 at rank 0), then the imprint step (imp_item.dst = -1 when the imprint is off or the grain is short)
+SEQ = np.dtype([("render", np.int64), ("rank", np.int64), ("fb", np.dtype(_abi.FeedbackEvt)),
+                ("imp", np.dtype(_abi.ImprintStepEvt)), ("imp_item", SPEC_ITEM)])
+
 
 def _recs(ctype, n):
     return np.zeros(n, dtype=np.dtype(ctype))
+
+
+def _structs(ctype, rows):
+    """ctypes structs -> record array of their bytes (padding included)."""
+    return np.frombuffer(bytearray(b"".join(map(bytes, rows))), np.dtype(ctype)) if rows else _recs(ctype, 0)
+
+
+def spec_items(rows):
+    """[(n, src, dst, SpecOp or None)] -> SPEC_ITEM array"""
+    return np.array([(n, s, d, _ZERO_OP if op is None else np.frombuffer(bytes(op), np.uint8)) for n, s, d, op in rows], SPEC_ITEM)
 
 
 _BESSEL = {}
@@ -56,66 +81,96 @@ def bessel_coeffs(theta, K=_abi.POST_K):
     return out
 
 
-class _Items:
-    """Spectral work items (n, in, out, operator bytes) of one stage."""
-
-    def __init__(self):
-        self.n, self.src, self.dst, self.ops = [], [], [], []
-
-    def add(self, n, src, dst, op):
-        self.n.append(n)
-        self.src.append(src)
-        self.dst.append(dst)
-        self.ops.append(bytes(op))
-
-    def arrays(self):
-        k = len(self.n)
-        ops = np.frombuffer(b"".join(self.ops), dtype=np.uint8).reshape(k, _SPEC_OP_BYTES) if k else np.zeros((0, _SPEC_OP_BYTES), np.uint8)
-        return (np.asarray(self.n, np.int64), np.asarray(self.src, np.int64), np.asarray(self.dst, np.int64), ops)
+def _empty(dtype, *shape):
+    return field(default_factory=lambda: np.zeros((0,) + shape, dtype))
 
 
 @dataclass
 class Tables:
-    sy1: np.ndarray = None
-    sy2: np.ndarray = None
-    ola_r: np.ndarray = None
-    env_reps: np.ndarray = None     # one OlaRender per shared envelope table (its .env = table offset)
+    sy1: np.ndarray = _empty(_abi.SynthEvt)
+    sy2: np.ndarray = _empty(_abi.SynthEvt)
+    ola_r: np.ndarray = _empty(_abi.OlaRender)
+    env_reps: np.ndarray = _empty(_abi.OlaRender)    # one OlaRender per shared envelope table (its .env = table offset)
     env_n: int = 0
-    ola_e: np.ndarray = None
-    fir: np.ndarray = None
-    post: np.ndarray = None
-    tap_off: np.ndarray = None
-    tap_gain: np.ndarray = None
-    irs: np.ndarray = None
-    dust_pos: np.ndarray = None
-    dust_val: np.ndarray = None
-    atoms: np.ndarray = None        # wavelet atoms, float64 [N, 4]
-    atom_shift: np.ndarray = None   # int32 [N]
-    seq: np.ndarray = None          # event-sequential tail (renders with event feedback), rows float64:
-                                    # render, rank, cur, prev (-1: none), n_prev, fb_dst (-1), imp_dst (-1), n, fb, amount, smooth
-    wg: tuple = None                # (rows int64 [N, 5] = src, dst, n, line_begin, line_count ; lines float64 [L, 3])
-    res: tuple = None               # (rows int64 [N, 5] = src, dst, n, mode_begin, mode_count ; decay [N] ; modes float64 [M, 3])
-    post_grain: tuple = None        # spectral items applied after the resonator bank (multiband): (n, src, dst, ops)
-    cep: tuple = None               # (rows int64 [N, 3] = src, dst, n ; factor [N] ; pre ops [N, B] ; post ops [N, B])
-    plock: tuple = None             # (rows int64 [N, 5] = src, dst, n, top_n, neigh ; factor [N] ; pre ops [N, B] ; post ops [N, B])
-    imprint: np.ndarray = None      # rows per imprinted event, in event order per render: render, pool_in, pool_out, n
-    imprint_par: np.ndarray = None  # per render: amount, smooth (nan when off)
-    tilt: tuple = None          # (n, src, dst, ops)
-    grain: tuple = None
-    rot: tuple = None
-    odd: np.ndarray = None      # rows: y_at, scratch, n, dr   (odd-length stereo)
+    ola_e: np.ndarray = _empty(_abi.OlaEvt)
+    fir: np.ndarray = _empty(_abi.FirRender)
+    post: np.ndarray = _empty(_abi.PostRender)
+    tap_off: np.ndarray = _empty(np.int32)
+    tap_gain: np.ndarray = _empty(np.float64)
+    irs: np.ndarray = _empty(np.float64)
+    dust_pos: np.ndarray = _empty(np.int32)
+    dust_val: np.ndarray = _empty(np.float64)
+    atoms: np.ndarray = _empty(np.float64, 4)        # wavelet atoms, float64 [N, 4]
+    atom_shift: np.ndarray = _empty(np.int32)
+    seq: np.ndarray = _empty(SEQ)                    # events of renders with event feedback, in render / event order
+    wg: np.ndarray = _empty(_abi.WgEvt)
+    wg_lines: np.ndarray = _empty(_abi.WgLine)
+    res: np.ndarray = _empty(_abi.ResEvt)
+    res_modes: np.ndarray = _empty(_abi.ResMode)
+    post_grain: np.ndarray = _empty(SPEC_ITEM)       # spectral items applied after the resonator bank (multiband)
+    cep: np.ndarray = _empty(_abi.CepEvt)            # cepstral warp (`pre` operator filled) ...
+    cep_items: np.ndarray = _empty(SPEC_ITEM)        # ... and its outer forward / inverse transform
+    plock: np.ndarray = _empty(_abi.PlockEvt)        # partial lock (`pre` operator filled) ...
+    plock_items: np.ndarray = _empty(SPEC_ITEM)      # ... and its outer transforms
+    imprint: np.ndarray = _empty(_abi.ImprintEvt)    # spectral imprint without feedback, in event order per render ...
+    imprint_items: np.ndarray = _empty(SPEC_ITEM)
+    imprint_r: np.ndarray = _empty(_abi.ImprintRender)
+    tilt: np.ndarray = _empty(SPEC_ITEM)
+    grain: np.ndarray = _empty(SPEC_ITEM)
+    rot: np.ndarray = _empty(SPEC_ITEM)
+    odd: np.ndarray = _empty(ODD)
     pool_n: int = 0
     mono_n: int = 0
     frames: int = 0
     h_total: int = 0
     max_h: int = 0
     max_out_n: int = 0
-    out_at: np.ndarray = None   # per render: first frame
-    out_n: np.ndarray = None
-    y_at: np.ndarray = None
-    last: np.ndarray = None     # per render: micro_at, grain_at, n of the last event (-1 if none)
-    srs: np.ndarray = None      # per render: base_sr, design_sr_base
-    alg: dict = field(default_factory=dict)   # algorithmic element counts per stage (SURVEY 8d)
+    out_at: np.ndarray = _empty(np.int64)            # per render: first frame
+    out_n: np.ndarray = _empty(np.int64)
+    y_at: np.ndarray = _empty(np.int64)
+    last: np.ndarray = _empty(LAST)
+    srs: np.ndarray = _empty(np.int64, 2)            # per render: base_sr, design_sr_base
+    alg: dict = field(default_factory=dict)          # algorithmic element counts per stage (SURVEY 8d)
+
+
+# Every offset field of the tables: (table, field) -> (buffer it indexes, whether -1 means "none" and stays -1).
+# Field None: the table is a plain per-render array of offsets.
+RELOC = {
+    ("sy1", "out"): ("pool", False), ("sy1", "dust_begin"): ("dust", False), ("sy1", "atom_begin"): ("atoms", False),
+    ("sy2", "out"): ("pool", False), ("sy2", "aux"): ("pool", False),
+    ("ola_r", "out"): ("mono", False), ("ola_r", "ev_begin"): ("ola_e", False), ("ola_r", "ev_end"): ("ola_e", False),
+    ("ola_r", "env"): ("env", True), ("env_reps", "env"): ("env", False),
+    ("ola_e", "grain"): ("pool", False),
+    ("fir", "ir"): ("irs", False), ("fir", "h"): ("h", False), ("fir", "tap_begin"): ("taps", False), ("fir", "tap_end"): ("taps", False),
+    ("fir", "x"): ("mono", False), ("fir", "y"): ("mono", False),
+    ("post", "y"): ("mono", False), ("post", "rbuf"): ("mono", False), ("post", "out"): ("frames", False),
+    ("seq", "render"): ("renders", False), ("seq", "fb.cur"): ("pool", False), ("seq", "fb.prev"): ("pool", True),
+    ("seq", "fb.dst"): ("pool", True), ("seq", "imp_item.src"): ("pool", False), ("seq", "imp_item.dst"): ("pool", True),
+    ("wg", "src"): ("pool", False), ("wg", "dst"): ("pool", False), ("wg", "line_begin"): ("wg_lines", False),
+    ("res", "src"): ("pool", False), ("res", "dst"): ("pool", False), ("res", "mode_begin"): ("res_modes", False),
+    ("imprint_r", "ev_begin"): ("imprint", False), ("imprint_r", "ev_end"): ("imprint", False),
+    ("odd", "y_at"): ("mono", False), ("odd", "scratch"): ("mono", False),
+    ("out_at", None): ("frames", False), ("y_at", None): ("mono", False),
+    ("last", "micro"): ("pool", True), ("last", "grain"): ("pool", True),
+}
+for _t, _buf in (("tilt", "pool"), ("grain", "pool"), ("post_grain", "pool"), ("cep_items", "pool"), ("plock_items", "pool"),
+                 ("imprint_items", "pool"), ("rot", "mono")):
+    RELOC[(_t, "src")] = RELOC[(_t, "dst")] = (_buf, False)
+
+# size of each buffer in a chunk: the base of the next chunk's offsets
+BUFFERS = {
+    "pool": lambda t: t.pool_n, "mono": lambda t: t.mono_n, "frames": lambda t: t.frames, "h": lambda t: t.h_total,
+    "env": lambda t: t.env_n, "ola_e": lambda t: len(t.ola_e), "taps": lambda t: len(t.tap_off), "irs": lambda t: len(t.irs),
+    "dust": lambda t: len(t.dust_pos), "atoms": lambda t: len(t.atom_shift), "res_modes": lambda t: len(t.res_modes),
+    "wg_lines": lambda t: len(t.wg_lines), "imprint": lambda t: len(t.imprint), "renders": lambda t: len(t.post),
+}
+
+
+def column(arr, name):
+    """arr["a"]["b"] for name "a.b"; arr itself for None."""
+    for f in (name.split(".") if name else ()):
+        arr = arr[f]
+    return arr
 
 
 def pack_chunk(plans) -> Tables:
@@ -125,20 +180,20 @@ def pack_chunk(plans) -> Tables:
     ola_r, post = _recs(_abi.OlaRender, R), _recs(_abi.PostRender, R)
     ola_e = []
     fir = []
-    tilt, grain, rot = _Items(), _Items(), _Items()
+    tilt, grain, rot, post_grain = [], [], [], []
     dust_pos, dust_val, n_dust = [], [], 0
     atoms, atom_shift, n_atoms = [], [], 0
-    imprint_rows, imprint_par = [], np.full((R, 2), np.nan)
-    pl_rows, pl_factor, pl_pre, pl_post = [], [], [], []
-    cp_rows, cp_factor, cp_pre, cp_post = [], [], [], []
-    rs_rows, rs_decay, rs_modes, n_modes = [], [], [], 0
-    wg_rows, wg_lines, n_lines = [], [], 0
-    seq_rows = []
-    post_grain = _Items()
+    imprint, imprint_items, imprint_r = [], [], []
+    plock, plock_items, cep, cep_items = [], [], [], []
+    res, res_modes, n_modes = [], [], 0
+    wg, wg_lines, n_lines = [], [], 0
+    seq = []
     tap_off, tap_gain, n_taps = [], [], 0
     irs, ir_index, n_ir = [], {}, 0
     pool_n = mono_n = h_total = max_h = 0
-    mono_at, last = [], np.full((R, 3), -1, np.int64)
+    mono_at = []
+    last = np.zeros(R, LAST)
+    last[:] = (-1, -1, -1)
     fir_of = {}
     alg = dict(synth=0, tilt_spectral=0, grain_spectral=0, overlap_add=0, fir_in=0, fir_taps=0, post=0)
     env_seen = {}
@@ -151,6 +206,7 @@ def pack_chunk(plans) -> Tables:
         d_end = min(n, a + d) if d > 0 else a
         sus_end = max(d_end, n - rel)
         ev_begin = len(ola_e)
+        imp_begin = len(imprint)
         max_len = 0
         x_begin, x_end = n, 0
         prev_final, prev_n, rank = -1, 0, 0
@@ -188,7 +244,7 @@ def pack_chunk(plans) -> Tables:
                 raw, tilted = pool_n, pool_n + ev.n
                 pool_n += 2 * ev.n
                 out1, mode2, aux2 = raw, ev.mode, tilted
-                tilt.add(ev.n, raw, tilted, ev.tilt)
+                tilt.append((ev.n, raw, tilted, ev.tilt))
                 alg["tilt_spectral"] += 2 * ev.n
             common = (s_hi, s_lo, i_hi, i_lo, ev.n)
             tail = (ev.fade, ev.sigma)
@@ -202,39 +258,34 @@ def pack_chunk(plans) -> Tables:
             if ev.cep is not None:
                 g_at = pool_n
                 pool_n += ev.n
-                cp_rows.append((micro, g_at, ev.n))
-                cp_factor.append(ev.cep[0])
-                cp_pre.append(bytes(ev.cep[1]))
-                cp_post.append(bytes(ev.cep[2]))
+                cep.append(_abi.CepEvt(n=ev.n, factor=ev.cep[0], pre=ev.cep[1]))
+                cep_items.append((ev.n, micro, g_at, ev.cep[2]))
                 alg["grain_spectral"] += 2 * ev.n * (1 + int(ev.cep[1].lp_on) + (1 if ev.cep[1].warp_exp else 0)
                                                      + int(ev.cep[2].stretch_on) + (1 if ev.cep[2].n_bands else 0))
             if ev.plock is not None:
                 pl_src = g_at                      # the raw transient, or the cepstrally warped grain
                 g_at = pool_n
                 pool_n += ev.n
-                pl_rows.append((pl_src, g_at, ev.n, ev.plock[1], ev.plock[2]))
-                pl_factor.append(ev.plock[0])
-                pl_pre.append(bytes(ev.plock[3]))
-                pl_post.append(bytes(ev.spec))
+                plock.append(_abi.PlockEvt(n=ev.n, top_n=ev.plock[1], neigh=ev.plock[2], factor=ev.plock[0], pre=ev.plock[3]))
+                plock_items.append((ev.n, pl_src, g_at, ev.spec))
                 alg["grain_spectral"] += 2 * ev.n * (1 + int(ev.plock[3].lp_on) + (1 if ev.plock[3].warp_exp else 0) + (1 if ev.spec.n_bands else 0))
             elif ev.cep is None and ev.spec is not None:
                 g_at = pool_n
                 pool_n += ev.n
-                grain.add(ev.n, micro, g_at, ev.spec)
+                grain.append((ev.n, micro, g_at, ev.spec))
                 alg["grain_spectral"] += 2 * ev.n * (int(ev.spec.lp_on) + int(ev.spec.stretch_on) + (1 if ev.spec.n_bands else 0)
                                                      + (1 if ev.spec.warp_exp else 0))
             if ev.res is not None:
                 r_at = pool_n                      # the resonator reads the grain so far and writes a new one
                 pool_n += ev.n
-                rs_rows.append((g_at, r_at, ev.n, n_modes, len(ev.res[0])))
-                rs_decay.append(ev.res[1])
-                rs_modes.append(ev.res[0])
+                res.append(_abi.ResEvt(src=g_at, dst=r_at, n=ev.n, mode_begin=n_modes, mode_count=len(ev.res[0]), decay=ev.res[1]))
+                res_modes.append(ev.res[0])
                 n_modes += len(ev.res[0])
                 g_at = r_at
             if ev.wg is not None:
                 w_at = pool_n                      # the combs run in place on a copy of the grain so far
                 pool_n += ev.n
-                wg_rows.append((g_at, w_at, ev.n, n_lines, len(ev.wg)))
+                wg.append(_abi.WgEvt(src=g_at, dst=w_at, n=ev.n, line_begin=n_lines, line_count=len(ev.wg)))
                 wg_lines.append(ev.wg)
                 n_lines += len(ev.wg)
                 g_at = w_at
@@ -242,7 +293,7 @@ def pack_chunk(plans) -> Tables:
                 if ev.spec_b is not None:
                     b_at = pool_n
                     pool_n += ev.n
-                    post_grain.add(ev.n, g_at, b_at, ev.spec_b)
+                    post_grain.append((ev.n, g_at, b_at, ev.spec_b))
                     alg["grain_spectral"] += 2 * ev.n
                     g_at = b_at
             last[r] = (micro, g_at, ev.n)
@@ -257,16 +308,17 @@ def pack_chunk(plans) -> Tables:
                 if imp_on:
                     imp_dst = pool_n
                     pool_n += ev.n
-                    g_at = imp_dst
-                seq_rows.append((r, rank, cur, prev_final, prev_n, fb_dst, imp_dst, ev.n, rp.feedback,
-                                 rp.imprint[0] if imp_on else 0.0, rp.imprint[1] if imp_on else 0.0))
+                amount, smooth = rp.imprint if imp_on else (0.0, 0.0)
+                seq.append((r, rank, (cur, prev_final, fb_dst, ev.n, prev_n, rp.feedback), (0, ev.n, 0, amount, smooth),
+                            (ev.n, g_at, imp_dst, _ZERO_OP)))       # the imprint reads the fed-back grain, or the grain itself
+                g_at = imp_dst if imp_on else g_at
                 prev_final, prev_n, rank = g_at, ev.n, rank + 1
             elif rp.imprint is not None and ev.n >= 64 and rp.imprint[0] > 0:         # M:570: short grains / amount <= 0 pass through
                 src = g_at
                 g_at = pool_n                      # imprinted grain (grain_last keeps the grain before it, M:729)
                 pool_n += ev.n
-                imprint_rows.append((r, src, g_at, ev.n))
-                imprint_par[r] = rp.imprint
+                imprint.append(_abi.ImprintEvt(n=ev.n))
+                imprint_items.append((ev.n, src, g_at, None))
             if ev.placed:
                 ola_e.append((g_at + ev.offset, ev.start, ev.length, ev.amp))
                 max_len = max(max_len, ev.length)
@@ -276,6 +328,8 @@ def pack_chunk(plans) -> Tables:
                 x_end = max(x_end, ev.start + ev.length)
                 alg["overlap_add"] += ev.length
             e += 1
+        if len(imprint) > imp_begin:
+            imprint_r.append(_abi.ImprintRender(imp_begin, len(imprint), *rp.imprint))
         env_key = (n, a, d_end, sus_end, 1 if (rel > 0 and n > sus_end) else 0,
                    1.0 / a if a > 0 else 0.0, 1.0 / (d_end - a) if d_end > a else 0.0,
                    1.0 / (n - sus_end - 1) if n - sus_end > 1 else 0.0, S, curve)
@@ -324,9 +378,7 @@ def pack_chunk(plans) -> Tables:
     frames = 0
     odd = []
     out_at, out_n, y_at = np.zeros(R, np.int64), np.zeros(R, np.int64), np.zeros(R, np.int64)
-    fir_arr = _recs(_abi.FirRender, len(fir))
-    for i, f in enumerate(fir):
-        fir_arr[i] = f
+    fir_arr = np.array(fir, np.dtype(_abi.FirRender))
     for r, rp in enumerate(plans):
         n = rp.out_n
         y = mono_at[r]
@@ -345,7 +397,7 @@ def pack_chunk(plans) -> Tables:
                 odd.append((y, 2 * plane + extra, n, dr))
                 op = _abi.SpecOp()
                 op.kind, op.alpha = _abi.OP_ROT, rp.stereo_theta
-                rot.add(n, 2 * plane + extra, 2 * plane + extra + n, op)
+                rot.append((n, 2 * plane + extra, 2 * plane + extra + n, op))
                 extra += 2 * n
         post[r] = (y, frames, rbuf, n, mode, dl, dr, rp.drive, 1.0 / math.tanh(rp.drive) if rp.drive > 0 else 1.0, rp.peak, coef)
         out_at[r], out_n[r], y_at[r] = frames, n, y
@@ -359,37 +411,29 @@ def pack_chunk(plans) -> Tables:
             ola_r["env"][members] = env_n
             reps.append(ola_r[members[0]].copy())
             env_n += int(key[0])
-    env_reps = np.array(reps, dtype=ola_r.dtype) if reps else np.zeros(0, dtype=ola_r.dtype)
     t = Tables()
-    t.env_reps, t.env_n = env_reps, env_n
+    if reps:
+        t.env_reps = np.array(reps, dtype=ola_r.dtype)
+    t.env_n = env_n
     t.sy1, t.sy2, t.ola_r, t.post, t.fir = sy1, sy2, ola_r, post, fir_arr
-    t.ola_e = _recs(_abi.OlaEvt, len(ola_e))
-    for i, rec in enumerate(ola_e):
-        t.ola_e[i] = rec
-    t.tap_off = np.concatenate(tap_off).astype(np.int32) if tap_off else np.zeros(0, np.int32)
-    t.tap_gain = np.concatenate(tap_gain).astype(np.float64) if tap_gain else np.zeros(0)
-    t.irs = np.concatenate(irs).astype(np.float64) if irs else np.zeros(0)
-    t.dust_pos = np.concatenate(dust_pos).astype(np.int32) if dust_pos else np.zeros(0, np.int32)
-    t.dust_val = np.concatenate(dust_val).astype(np.float64) if dust_val else np.zeros(0)
-    t.atoms = np.concatenate(atoms).astype(np.float64) if atoms else np.zeros((0, 4))
-    t.atom_shift = np.concatenate(atom_shift).astype(np.int32) if atom_shift else np.zeros(0, np.int32)
-    npl = len(pl_rows)
-    t.plock = (np.asarray(pl_rows, np.int64).reshape(-1, 5), np.asarray(pl_factor, np.float64),
-               np.frombuffer(b"".join(pl_pre), np.uint8).reshape(npl, _SPEC_OP_BYTES) if npl else np.zeros((0, _SPEC_OP_BYTES), np.uint8),
-               np.frombuffer(b"".join(pl_post), np.uint8).reshape(npl, _SPEC_OP_BYTES) if npl else np.zeros((0, _SPEC_OP_BYTES), np.uint8))
-    t.res = (np.asarray(rs_rows, np.int64).reshape(-1, 5), np.asarray(rs_decay, np.float64),
-             np.concatenate(rs_modes) if rs_modes else np.zeros((0, 3)))
-    t.seq = np.asarray(seq_rows, np.float64).reshape(-1, 11)
-    t.wg = (np.asarray(wg_rows, np.int64).reshape(-1, 5), np.concatenate(wg_lines) if wg_lines else np.zeros((0, 3)))
-    t.post_grain = post_grain.arrays()
-    ncp = len(cp_rows)
-    t.cep = (np.asarray(cp_rows, np.int64).reshape(-1, 3), np.asarray(cp_factor, np.float64),
-             np.frombuffer(b"".join(cp_pre), np.uint8).reshape(ncp, _SPEC_OP_BYTES) if ncp else np.zeros((0, _SPEC_OP_BYTES), np.uint8),
-             np.frombuffer(b"".join(cp_post), np.uint8).reshape(ncp, _SPEC_OP_BYTES) if ncp else np.zeros((0, _SPEC_OP_BYTES), np.uint8))
-    t.imprint = np.asarray(imprint_rows, np.int64).reshape(-1, 4)
-    t.imprint_par = imprint_par
-    t.tilt, t.grain, t.rot = tilt.arrays(), grain.arrays(), rot.arrays()
-    t.odd = np.asarray(odd, np.int64).reshape(-1, 4)
+    t.ola_e = np.array(ola_e, np.dtype(_abi.OlaEvt))
+    for name, parts in (("tap_off", tap_off), ("tap_gain", tap_gain), ("irs", irs), ("dust_pos", dust_pos), ("dust_val", dust_val),
+                        ("atoms", atoms), ("atom_shift", atom_shift)):
+        if parts:
+            setattr(t, name, np.concatenate(parts).astype(getattr(t, name).dtype))
+    t.cep, t.cep_items = _structs(_abi.CepEvt, cep), spec_items(cep_items)
+    t.plock, t.plock_items = _structs(_abi.PlockEvt, plock), spec_items(plock_items)
+    t.res = _structs(_abi.ResEvt, res)
+    if res_modes:
+        t.res_modes = np.ascontiguousarray(np.concatenate(res_modes), np.float64).view(t.res_modes.dtype).reshape(-1)
+    t.wg, t.wg_lines = _structs(_abi.WgEvt, wg), _recs(_abi.WgLine, n_lines)
+    if wg_lines:
+        lines = np.concatenate(wg_lines)
+        t.wg_lines["d"], t.wg_lines["g"], t.wg_lines["mix"] = lines[:, 0], lines[:, 1], lines[:, 2]
+    t.seq = np.array(seq, SEQ)
+    t.imprint, t.imprint_items, t.imprint_r = _structs(_abi.ImprintEvt, imprint), spec_items(imprint_items), _structs(_abi.ImprintRender, imprint_r)
+    t.tilt, t.grain, t.rot, t.post_grain = spec_items(tilt), spec_items(grain), spec_items(rot), spec_items(post_grain)
+    t.odd = np.array(odd, ODD)
     t.pool_n, t.mono_n, t.frames, t.h_total, t.max_h = pool_n, 2 * plane + extra, frames, h_total, max_h
     t.max_out_n = max((rp.out_n for rp in plans), default=0)
     t.out_at, t.out_n, t.y_at, t.last = out_at, out_n, y_at, last
@@ -398,120 +442,55 @@ def pack_chunk(plans) -> Tables:
     return t
 
 
-def _shift(arr, fields, base):
-    if arr.size and base:
-        for f in fields:
-            arr[f] += base
-
-
 def merge_chunks(chunks) -> Tables:
+    """One Tables of consecutive chunks: tables concatenated, offsets shifted by the chunk's base in their buffer.
+    The chunks themselves are left as they are."""
     if len(chunks) == 1:
         return chunks[0]
     m = Tables()
-    pool_b = mono_b = frame_b = h_b = tap_b = ir_b = dust_b = olae_b = env_b = atom_b = render_b = 0
-    parts = {k: [] for k in ("sy1", "sy2", "ola_r", "env_reps", "ola_e", "fir", "post", "tap_off", "tap_gain", "irs", "dust_pos", "dust_val",
-                             "atoms", "atom_shift", "imprint", "imprint_par", "seq", "odd", "out_at", "out_n", "y_at", "last", "srs")}
-    items = {k: [[], [], [], []] for k in ("tilt", "grain", "rot", "post_grain")}
-    rs_parts, mode_b = [[], [], []], 0
-    wg_parts, line_b = [[], []], 0
-    pl_parts = [[], [], [], []]
-    cp_parts = [[], [], [], []]
-    alg = {}
+    for f in fields(Tables):
+        if f.name != "alg" and isinstance(getattr(m, f.name), np.ndarray):
+            setattr(m, f.name, np.concatenate([getattr(c, f.name) for c in chunks]))
+    bases = {buf: np.cumsum([0] + [size(c) for c in chunks[:-1]]) for buf, size in BUFFERS.items()}
+
+    def shift(table, buf):
+        return np.repeat(bases[buf], [len(getattr(c, table)) for c in chunks])
+    for (table, name), (buf, keep_none) in RELOC.items():
+        col, add = column(getattr(m, table), name), shift(table, buf)
+        col += np.where(col >= 0, add, 0) if keep_none else add
+    # sy1.aux is a pool offset only for these generators (the scratch they synthesise through); 0 for the others
+    m.sy1["aux"] += np.where(np.isin(m.sy1["mode"], (P.MODE_SCANLINE, P.MODE_CHAOS, P.MODE_STICK)), shift("sy1", "pool"), 0)
+    for k in ("pool_n", "mono_n", "frames", "h_total", "env_n"):
+        setattr(m, k, sum(getattr(c, k) for c in chunks))
+    m.max_h, m.max_out_n = max(c.max_h for c in chunks), max(c.max_out_n for c in chunks)
     for c in chunks:
-        _shift(c.sy1, ("out",), pool_b)
-        if c.sy1.size and pool_b:
-            c.sy1["aux"] += np.where((c.sy1["mode"] == P.MODE_SCANLINE) | (c.sy1["mode"] == P.MODE_CHAOS) | (c.sy1["mode"] == P.MODE_STICK), pool_b, 0)
-        _shift(c.sy1, ("dust_begin",), dust_b)
-        _shift(c.sy1, ("atom_begin",), atom_b)
-        if c.imprint.size:
-            c.imprint[:, 0] += render_b
-            c.imprint[:, 1:3] += pool_b
-        if c.seq.size:
-            c.seq[:, 0] += render_b
-            for col in (2, 3, 5, 6):
-                c.seq[:, col] += np.where(c.seq[:, col] >= 0, pool_b, 0)
-        if c.plock[0].size:
-            c.plock[0][:, 0:2] += pool_b
-        if c.cep[0].size:
-            c.cep[0][:, 0:2] += pool_b
-        for i in range(4):
-            pl_parts[i].append(c.plock[i])
-            cp_parts[i].append(c.cep[i])
-        _shift(c.sy2, ("out", "aux"), pool_b)
-        _shift(c.ola_r, ("out",), mono_b)
-        _shift(c.ola_r, ("ev_begin", "ev_end"), olae_b)
-        if env_b:
-            c.ola_r["env"] += np.where(c.ola_r["env"] >= 0, env_b, 0)
-            c.env_reps["env"] += env_b
-        _shift(c.ola_e, ("grain",), pool_b)
-        _shift(c.fir, ("ir",), ir_b)
-        _shift(c.fir, ("h",), h_b)
-        _shift(c.fir, ("tap_begin", "tap_end"), tap_b)
-        _shift(c.fir, ("x", "y"), mono_b)
-        _shift(c.post, ("y", "rbuf"), mono_b)
-        _shift(c.post, ("out",), frame_b)
-        if c.odd.size:
-            c.odd[:, 0:2] += mono_b
-        c.out_at += frame_b
-        c.y_at += mono_b
-        if c.last.size:
-            c.last[:, 0:2] += np.where(c.last[:, 0:2] >= 0, pool_b, 0)
-        for k in parts:
-            parts[k].append(getattr(c, k))
-        if c.res[0].size:
-            c.res[0][:, 0:2] += pool_b
-            c.res[0][:, 3] += mode_b
-        for i in range(3):
-            rs_parts[i].append(c.res[i])
-        mode_b += len(c.res[2])
-        if c.wg[0].size:
-            c.wg[0][:, 0:2] += pool_b
-            c.wg[0][:, 3] += line_b
-        wg_parts[0].append(c.wg[0])
-        wg_parts[1].append(c.wg[1])
-        line_b += len(c.wg[1])
-        for k, base in (("tilt", pool_b), ("grain", pool_b), ("rot", mono_b), ("post_grain", pool_b)):
-            n, s, d, ops = getattr(c, k)
-            items[k][0].append(n)
-            items[k][1].append(s + base)
-            items[k][2].append(d + base)
-            items[k][3].append(ops)
         for k, v in c.alg.items():
-            alg[k] = alg.get(k, 0) + v
-        pool_b += c.pool_n
-        mono_b += c.mono_n
-        frame_b += c.frames
-        h_b += c.h_total
-        tap_b += c.tap_off.size
-        ir_b += c.irs.size
-        dust_b += c.dust_pos.size
-        olae_b += c.ola_e.size
-        env_b += c.env_n
-        atom_b += c.atom_shift.size
-        render_b += len(c.post)
-        m.max_h = max(m.max_h, c.max_h)
-        m.max_out_n = max(m.max_out_n, c.max_out_n)
-    for k in parts:
-        setattr(m, k, np.concatenate(parts[k]))
-    for k in items:
-        setattr(m, k, tuple(np.concatenate(x) for x in items[k]))
-    m.plock = tuple(np.concatenate(x) for x in pl_parts)
-    m.res = tuple(np.concatenate(x) for x in rs_parts)
-    m.wg = tuple(np.concatenate(x) for x in wg_parts)
-    m.cep = tuple(np.concatenate(x) for x in cp_parts)
-    m.pool_n, m.mono_n, m.frames, m.h_total, m.alg, m.env_n = pool_b, mono_b, frame_b, h_b, alg, env_b
+            m.alg[k] = m.alg.get(k, 0) + v
     return m
 
 
+def _op_bytes(jobs, i):
+    """Raw bytes of jobs["op"][:, i] (SpecOp has nested structs: operators are copied as bytes)."""
+    op0 = _SPEC_JOB.fields["op"][1] + i * _SPEC_OP_BYTES
+    return jobs.view(np.uint8).reshape(len(jobs), _SPEC_JOB.itemsize)[:, op0:op0 + _SPEC_OP_BYTES]
+
+
+def single_jobs(items):
+    """SPEC_ITEM array -> one SpecJob per item, in item order (for stages that address each job's spectrum)."""
+    jobs = np.zeros(len(items), _SPEC_JOB)
+    jobs["n"], jobs["in_a"], jobs["out_a"], jobs["in_b"], jobs["out_b"] = items["n"], items["src"], items["dst"], -1, -1
+    _op_bytes(jobs, 0)[:] = items["op"]
+    return jobs
+
+
 def pair_jobs(items):
-    """(n, src, dst, ops) -> SpecJob record array.  Two signals of equal n share one complex transform;
+    """SPEC_ITEM array -> SpecJob record array.  Two signals of equal n share one complex transform;
     the leftover of an odd group rides alone."""
-    n, src, dst, ops = items
-    k = n.size
+    k = len(items)
     if k == 0:
         return np.zeros(0, _SPEC_JOB)
-    order = np.argsort(n, kind="stable")
-    n, src, dst, ops = n[order], src[order], dst[order], ops[order]
+    items = items[np.argsort(items["n"], kind="stable")]
+    n, src, dst, ops = items["n"], items["src"], items["dst"], items["op"]
     starts = np.flatnonzero(np.r_[True, n[1:] != n[:-1]])
     pos = np.arange(k) - np.repeat(starts, np.diff(np.r_[starts, k]))      # index inside its equal-n group
     first = pos % 2 == 0
@@ -521,15 +500,13 @@ def pair_jobs(items):
     b = a + 1
     paired = has_partner[a]
     jobs = np.zeros(a.size, _SPEC_JOB)
-    raw = jobs.view(np.uint8).reshape(a.size, _SPEC_JOB.itemsize)
     jobs["n"] = n[a]
     jobs["in_a"], jobs["out_a"] = src[a], dst[a]
     bb = np.where(paired, np.minimum(b, k - 1), 0)
     jobs["in_b"] = np.where(paired, src[bb], -1)
     jobs["out_b"] = np.where(paired, dst[bb], -1)
-    op0 = _SPEC_JOB.fields["op"][1]
-    raw[:, op0:op0 + _SPEC_OP_BYTES] = ops[a]
-    raw[:, op0 + _SPEC_OP_BYTES:op0 + 2 * _SPEC_OP_BYTES] = np.where(paired[:, None], ops[bb], _ZERO_OP[None, :])
+    _op_bytes(jobs, 0)[:] = ops[a]
+    _op_bytes(jobs, 1)[:] = np.where(paired[:, None], ops[bb], _ZERO_OP[None, :])
     return jobs
 
 

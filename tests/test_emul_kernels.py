@@ -105,6 +105,13 @@ def test_pooled_planning_matches_in_process(emul, monkeypatch):
                                       ("Resonant strike", 30.0), ("Skewed transient", 25.0), ("Gaussian click", 30.0),
                                       ("Resonant strike", 25.0)])]
     ps[3]["base_sr"], ps[3]["out_dur_s"] = 44100, 0.05003          # odd length -> FFT rotation path
+    # the stages outside the native planner's family, split across pieces
+    extra = dict(event_process="Poisson", out_dur_s=0.15, grains_per_sec=30.0, micro_ms=2.0, er_cloud_on=False, bandlimit_on=False)
+    ps += [configs.with_defaults(extra, seed=40, cep_warp_on=True, cep_factor=1.2, gen_mode="Resonant strike"),
+           configs.with_defaults(extra, seed=41, res_bank_on=True, wg_on=True, wg_max_ms=1.0, partial_lock_on=True, partial_stretch=1.1,
+                                 unfold_mode="Multi-band unfold", gen_mode="Stick–slip friction"),
+           configs.with_defaults(extra, seed=42, event_feedback_on=True, spectral_imprint_on=True, res_bank_on=True, gen_mode="Gaussian click"),
+           configs.with_defaults(extra, seed=43, spectral_imprint_on=True, gen_mode="Wavelet atoms")]
     one = engine.render_batch(ps, device=emul)
     streamed = engine.render_batch(ps, device=emul, chunk=5, workers=3, piece=2)     # slices of 5 = pieces of 2+2+1, 2
     ramped = engine.render_batch(ps, device=emul, chunk=[1, 2, 3], workers=2, piece=2)  # slice schedule 1, 2, 3, 3: short first slices

@@ -145,6 +145,11 @@ public:
     int filter_compose(const std::vector<FftJob>& jobs, const FftJob* jobs_dev, ms_stream_t st, size_t lo = 0, size_t hi = (size_t)-1) { return run(jobs, jobs_dev, st, 5, lo, hi); }
     // overlap-save: two blocks per job, multiplied by `bspec`, valid outputs stored
     int overlap_save(const std::vector<FftJob>& jobs, const FftJob* jobs_dev, ms_stream_t st, size_t lo = 0, size_t hi = (size_t)-1) { return run(jobs, jobs_dev, st, 4, lo, hi); }
+    // partitioned overlap-save (ms_fir_long.cuh), direct lengths only.  Forward: two blocks of real input as re / im (LD_OLS:
+    // in_a / in_b at p0_a / p0_b, zero outside [0, ols_n)) -> natural-order spectrum * out_scale at `cout`.  Inverse: the
+    // natural-order swap(Y) at `cin` -> its transform, i.e. swap(M * IFFT(Y)) -> valid outputs of both blocks (ST_OLS).
+    int ols_forward(const std::vector<FftJob>& jobs, const FftJob* jobs_dev, ms_stream_t st) { return run(jobs, jobs_dev, st, 6); }
+    int ols_inverse(const std::vector<FftJob>& jobs, const FftJob* jobs_dev, ms_stream_t st) { return run(jobs, jobs_dev, st, 7); }
 
 private:
     std::mutex mu_;
@@ -405,7 +410,8 @@ private:
         return cs;
     }
 
-    // what: 0 forward (pair -> Z), 1 inverse (spec(Z) -> pair), 2 c2c test path
+    // what: 0 forward (pair -> Z), 1 inverse (spec(Z) -> pair), 2 c2c test path, 3 / 5 filter spectra, 4 overlap-save,
+    // 6 / 7 forward / inverse of the partitioned overlap-save
     int run(const std::vector<FftJob>& jobs, const FftJob* jobs_dev, ms_stream_t st, int what, size_t lo = 0, size_t hi = (size_t)-1) {
         const size_t end = std::min(hi, jobs.size());
         size_t b = lo;
@@ -449,6 +455,15 @@ private:
                     if (!rc) rc = launch_rows<LD_WORK, MODE_CONV, ST_WORK>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd);
                     if (!rc) rc = launch_cols<LD_WORK, ST_OLS, 0>(C.ept, C.gx, gy, C.nthr, C.smem, st, jd);
                 } else MS_FAIL("overlap-save needs a direct length");
+            } else if (what == 6 || what == 7) {
+                if (cls == 0) rc = what == 6 ? launch_rows<LD_OLS, MODE_NAT, ST_CPX>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd)
+                                             : launch_rows<LD_CPX, MODE_NAT, ST_OLS>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd);
+                else if (cls == 1) {
+                    rc = what == 6 ? launch_cols<LD_OLS, ST_WORK, 1>(C.ept, C.gx, gy, C.nthr, C.smem, st, jd)
+                                   : launch_cols<LD_CPX, ST_WORK, 1>(C.ept, C.gx, gy, C.nthr, C.smem, st, jd);
+                    if (!rc) rc = what == 6 ? launch_rows<LD_WORK, MODE_NAT, ST_CPX>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd)
+                                            : launch_rows<LD_WORK, MODE_NAT, ST_OLS>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd);
+                } else MS_FAIL("partitioned overlap-save needs a direct length");
             } else if (what == 2) {
                 if (cls == 0) rc = launch_rows<LD_CPX, MODE_NAT, ST_CPX>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd);
                 else if (cls == 1) {

@@ -145,13 +145,16 @@ def _marshal(params_list):
     gs = _get_side
     for r, p in enumerate(params_list):
         ir, dig = p.get("_ir_audio"), p.get("_ir_digest")
-        key = gs(p) + (id(ir), id(dig), widths[r])
+        cap = p.get("space_ir_tap_cap", P.IR_TAP_CAP)           # optional key: not in the itemgetter
+        if cap.__class__ is not int or cap < 1:
+            cap = P.ir_tap_cap(p)
+        key = gs(p) + (cap, id(ir), id(dig), widths[r])
         k = uniq_of.get(key)
         if k is None:
-            gen_mode, unfold_mode, process, l0, l1, l2, l3, ir_on, max_samps, _, _, w = key
+            gen_mode, unfold_mode, process, l0, l1, l2, l3, ir_on, max_samps, _, _, _, w = key
             ir_id = -1.0
             if ir_on:
-                taps = dig["taps"] if dig is not None else (P._ir_taps(ir, int(max_samps)) if ir is not None else None)
+                taps = dig["taps"] if dig is not None else (P._ir_taps(ir, int(max_samps), cap) if ir is not None else None)
                 if taps is not None:
                     j = ir_of.get(id(taps))
                     if j is None or irs[j] is not taps:

@@ -20,7 +20,8 @@ from . import _abi
 from .configs import BASIC_MODES
 
 DESIGN_SR_CAP = 30_000_000          # M:597, M:646
-IR_TAP_CAP = 8192                   # M:443
+IR_TAP_CAP = 8192                   # M:443: default of the optional key `space_ir_tap_cap`
+IR_TAP_LIMIT = 1 << 21              # most IR taps the FIR stage takes (ms_fir_*: 10 s at 192 kHz)
 
 MODE_GAUSS, MODE_DUST, MODE_NOISE, MODE_SKEW, MODE_RES, MODE_PLAIN, MODE_WAVELET, MODE_IRFRAG, MODE_SCANLINE, MODE_SILENT, MODE_CHAOS, MODE_STICK = range(12)
 WAVELET_FLOOR = 128                 # M:319
@@ -255,7 +256,7 @@ class RenderPlan:
     feedback: Optional[float] = None        # event_feedback_amt when event feedback is on (M:731-734)
     er_offs: Optional[np.ndarray] = None    # int32 tap delays (0 < off < out_n)
     er_gains: Optional[np.ndarray] = None   # float64
-    ir: Optional[np.ndarray] = None         # float64 mono taps (<= 8192) or None
+    ir: Optional[np.ndarray] = None         # float64 mono taps (<= space_ir_tap_cap) or None
     stereo_on: bool = False
     stereo_dl: int = 0
     stereo_dr: int = 0
@@ -284,6 +285,7 @@ def check_supported(params):
 def plan_render(params) -> RenderPlan:
     """Scalar half of render() (M:589-646, 742-753, 760-781)."""
     check_supported(params)
+    cap = ir_tap_cap(params)
     base_sr = int(params["base_sr"])
     out_dur = float(params["out_dur_s"])
     out_n = int(max(1, round(out_dur * base_sr)))
@@ -438,7 +440,7 @@ def plan_render(params) -> RenderPlan:
         if digest is not None:
             rp.ir = digest["taps"]
         elif ir_audio is not None:
-            rp.ir = _ir_taps(ir_audio, int(params["space_ir_max_samps"]))
+            rp.ir = _ir_taps(ir_audio, int(params["space_ir_max_samps"]), cap)
     if params["stereo_on"] and out_n >= 64:   # M:426: shorter outputs are duplicated
         w = float(min(max(float(params["stereo_width"]), 0.0), 1.0))
         rp.stereo_on = True
@@ -465,18 +467,34 @@ def array_signature(a):
     return (id(a), a.shape, a.dtype.str, float(np.sum(flat[::step], dtype=np.float64)), float(flat[-1]) if flat.size else 0.0)
 
 
-def _ir_taps(ir, max_samps):
+def ir_tap_cap(params):
+    """The optional key `space_ir_tap_cap`: how many rows of the IR convolve_ir_short keeps (M:443 keeps 8192, the
+    default).  An int >= 1, or None for no cap beyond `space_ir_max_samps`.  Caps above 8192 are an EXTENSION of the
+    reference: the FIR stage then runs its partitioned route, checked against float64 convolution."""
+    cap = params.get("space_ir_tap_cap", IR_TAP_CAP)
+    if cap is None:
+        return None
+    if isinstance(cap, (bool, np.bool_)) or not isinstance(cap, (int, np.integer)) or cap < 1:
+        raise ValueError(f"space_ir_tap_cap must be an int >= 1 or None, not {cap!r}")
+    return int(cap)
+
+
+def _ir_taps(ir, max_samps, cap=IR_TAP_CAP):
     """convolve_ir_short's view of the IR (M:438-443): None if the slice has fewer than 8 values, else the
-    float64 mono mix of its first 8192 rows.  Cached per IR object: a sweep shares one IR."""
-    key = (array_signature(ir), max_samps)
+    float64 mono mix of its first `cap` rows (None: all of them).  Cached per IR object: a sweep shares one IR.
+    More than IR_TAP_LIMIT kept taps raise ValueError: the FIR stage does not take them."""
+    key = (array_signature(ir), max_samps, cap)
     hit = _TAPS_CACHE.get(key)
     if hit is not None and hit[0] is ir:
         return hit[1]
     h = np.asarray(ir)[:max_samps]
     taps = None
     if h.size >= 8:                           # size counts both channels of a 2-D IR
-        h = h[:IR_TAP_CAP].astype(np.float64)         # the mono mix is row-wise, so cut to 8192 rows first
+        h = (h if cap is None else h[:cap]).astype(np.float64)      # the mono mix is row-wise, so cut to `cap` rows first
         taps = h.mean(axis=1) if h.ndim > 1 else h
+        if taps.size > IR_TAP_LIMIT:
+            raise ValueError(f"an impulse response of {taps.size} taps is outside the accelerated path "
+                             f"(at most {IR_TAP_LIMIT}; lower space_ir_tap_cap or space_ir_max_samps)")
     if len(_TAPS_CACHE) > 64:
         _TAPS_CACHE.clear()
     _TAPS_CACHE[key] = (ir, taps)
@@ -611,7 +629,7 @@ def _plan_dust(ev, density):
 def _slim_params(p):
     """Copy of a parameter dict for the planning workers: the impulse response is replaced by what the planner
     keeps of it -- `_ir_digest = {"taps": convolve_ir_short's view (M:439-443: float64 mono mix of the first
-    min(space_ir_max_samps, 8192) rows, None when that slice has fewer than 8 values), "frag": gen_ir_fragment's
+    min(space_ir_max_samps, space_ir_tap_cap) rows, None when that slice has fewer than 8 values), "frag": gen_ir_fragment's
     source (M:335-340: the float64 mono mix of the WHOLE response, None when it has fewer than 32 values)}` -- so a
     multi-second stereo IR is not pickled per render and both size tests are made on the original array.  The
     digests are cached per IR object, so renders sharing an IR share the arrays (one pickle memo entry per piece)."""
@@ -623,6 +641,6 @@ def _slim_params(p):
     frag = None
     if p["gen_mode"] == "IR fragment" and np.asarray(ir).size >= 32:
         frag = _mono64(ir)
-    taps = _ir_taps(ir, int(p["space_ir_max_samps"])) if p["space_ir_on"] else None
+    taps = _ir_taps(ir, int(p["space_ir_max_samps"]), ir_tap_cap(p)) if p["space_ir_on"] else None
     q["_ir_digest"] = {"taps": taps, "frag": frag}
     return q

@@ -219,8 +219,12 @@ typedef struct {
     int32_t x_begin, x_end;   /* support of the input: samples outside [x_begin, x_end) are exactly zero */
     int32_t _pad;
 } ms_fir_render;
-/* The cloud and the IR are both causal LTI filters: the library keeps the spectrum of every distinct IR
- * (computed once in ms_fir_create) and composes IRspec * (1 + FFT(cloud taps)) per render in ms_fir_run. */
+/* The cloud and the IR are both causal LTI filters.  Route by row: ir_len <= 8192 -- the library keeps the spectrum of
+ * every distinct IR (computed once in ms_fir_create) and composes IRspec * (1 + FFT(cloud taps)) per render;
+ * 8192 < ir_len <= 2^21 (EXTENSION: the reference cuts at 8192) -- the cloud runs first as its own pass into the workspace,
+ * then the IR as uniformly partitioned overlap-save with partition spectra computed once per distinct (ir, ir_len,
+ * partition length), using only min(ir_len, out_n - x_begin) taps (the others cannot reach y[:out_n]).  A batch may mix
+ * both; longer IRs fail in ms_fir_workspace_bytes / ms_fir_create.  ms_fir_run allocates nothing and never synchronises. */
 /* ms_fir_workspace_bytes_f32 / ms_fir_workspace_bytes_f64: declared below by MS_DECLARE_API */
 /* ms_fir_create_f32 / ms_fir_create_f64: declared below by MS_DECLARE_API */
 /* ms_fir_run_f32 / ms_fir_run_f64: declared below by MS_DECLARE_API */

@@ -163,8 +163,46 @@ MS_DEV_NOINLINE void fir_fold_row0(const int* MS_RESTRICT rp, const real* MS_RES
 // one pass of eight rows: fetch, FFT, * H, swap, FFT, twiddle, back.  row0 + slot = global row of tile slot `slot`
 // (slot_zero >= 0: that slot holds row 0 instead); this warp works on slot `my`, whose filter row is IRspec[row] *
 // (1 + E) with E = sE[erow] (rev: reversed and conjugated); own_e: the warp first transforms its E row in place.
+// (second half of a pass) v = this warp's row spectrum: * H (filter `filt`), swap, inverse, twiddle, tile back into S
+MS_DEV void fir_p2_filter_store(cpx* v, const cpx* filt, const FirTables& T, cpx* S, cpx* sB, const cpx* swE, int row0, int slot_zero,
+                                int my, int row, int rev, int taps, const Ctx& c) {
+    const int lane = c.tid & 31;
+    cpx* sw = sB + my * FF_RS;
+    {
+        const cpx* f = filt + (size_t)row * FF_N + lane;
+#pragma unroll
+        for (int m = 0; m < 8; ++m) {
+            cpx h = __ldg(&f[32 * m]);
+            if (taps) {
+                const int k2 = lane + 32 * m;
+                const cpx e = rev ? c_conj(swE[ms_pad(FF_N - 1 - k2)]) : swE[ms_pad(k2)];
+                h = c_mul(h, mk(e.x + (real)1.0, e.y));
+            }
+            v[m] = c_swap(c_mul(v[m], h));
+        }
+    }
+    c.syncwarp();
+    warp_fft256(v, sw, T.tw, lane, c);                      // inverse over k2 (swapped domain): index n2' = lane + 32 m
+    twiddle_row(v, T, row, lane);
+    c.syncwarp();
+#pragma unroll
+    for (int m = 0; m < 8; ++m) sw[ms_pad(lane + 32 * m)] = v[m];
+    c.sync();
+    {
+        const int rr = c.tid & 7;
+        const int rw = rr == slot_zero ? 0 : row0 + rr;
+        cpx* dst = S + (size_t)(c.tid >> 3) * FF_N + rw;
+#pragma unroll
+        for (int i = 0; i < FF_N * FF_TILE / FF_NTHR; ++i) dst[(size_t)(FF_NTHR / 8) * FF_N * i] = sB[rr * FF_RS + ms_pad((c.tid >> 3) + (FF_NTHR / 8) * i)];
+    }
+    c.sync();
+}
+// PAIR (space_ir_stereo, two rows equal on the input side): the row spectrum is filtered twice -- by U.filt back into S,
+// by filt_r into S_r -- from one tile fetch, one E transform and one forward row FFT.  Each channel's arithmetic is that
+// of a lone unit with its filter, so each result is bit-identical to it.
+template <bool PAIR>
 MS_DEV void fir_p2_pass(const FirUnit& U, const FirTables& T, cpx* S, cpx* sB, cpx* sE, int row0, int slot_zero, int my, int erow, int rev,
-                        int own_e, int taps, const Ctx& c) {
+                        int own_e, int taps, const Ctx& c, const cpx* filt_r = nullptr, cpx* S_r = nullptr) {
     const int lane = c.tid & 31;
     cpx v[8];
     {   // the tile: S[n2][rows of the pass] -> sB[slot][n2]   (all loads in flight before the first store)
@@ -194,36 +232,18 @@ MS_DEV void fir_p2_pass(const FirUnit& U, const FirTables& T, cpx* S, cpx* sB, c
     for (int q = 0; q < 8; ++q) v[q] = sw[ms_pad(lane + 32 * q)];
     c.syncwarp();
     warp_fft256(v, sw, T.tw, lane, c);                      // v[m] = Z[row][k2 = lane + 32 m]
-    {
-        const cpx* f = U.filt + (size_t)row * FF_N + lane;
+    if (PAIR) {
+        cpx z[8];
 #pragma unroll
-        for (int m = 0; m < 8; ++m) {
-            cpx h = __ldg(&f[32 * m]);
-            if (taps) {
-                const int k2 = lane + 32 * m;
-                const cpx e = rev ? c_conj(swE[ms_pad(FF_N - 1 - k2)]) : swE[ms_pad(k2)];
-                h = c_mul(h, mk(e.x + (real)1.0, e.y));
-            }
-            v[m] = c_swap(c_mul(v[m], h));
-        }
+        for (int m = 0; m < 8; ++m) z[m] = v[m];
+        fir_p2_filter_store(v, U.filt, T, S, sB, swE, row0, slot_zero, my, row, rev, taps, c);
+        fir_p2_filter_store(z, filt_r, T, S_r, sB, swE, row0, slot_zero, my, row, rev, taps, c);
+    } else {
+        fir_p2_filter_store(v, U.filt, T, S, sB, swE, row0, slot_zero, my, row, rev, taps, c);
     }
-    c.syncwarp();
-    warp_fft256(v, sw, T.tw, lane, c);                      // inverse over k2 (swapped domain): index n2' = lane + 32 m
-    twiddle_row(v, T, row, lane);
-    c.syncwarp();
-#pragma unroll
-    for (int m = 0; m < 8; ++m) sw[ms_pad(lane + 32 * m)] = v[m];
-    c.sync();
-    {
-        const int rr = c.tid & 7;
-        const int rw = rr == slot_zero ? 0 : row0 + rr;
-        cpx* dst = S + (size_t)(c.tid >> 3) * FF_N + rw;
-#pragma unroll
-        for (int i = 0; i < FF_N * FF_TILE / FF_NTHR; ++i) dst[(size_t)(FF_NTHR / 8) * FF_N * i] = sB[rr * FF_RS + ms_pad((c.tid >> 3) + (FF_NTHR / 8) * i)];
-    }
-    c.sync();
 }
-MS_DEV void fir_p2_tile(const FirUnit& U, const FirTables& T, cpx* S, int tile, const Ctx& c) {
+template <bool PAIR>
+MS_DEV void fir_p2_tile(const FirUnit& U, const FirTables& T, cpx* S, int tile, const Ctx& c, const cpx* filt_r = nullptr, cpx* S_r = nullptr) {
     cpx* sB = (cpx*)c.smem;                                 // transposing tile + exchange rows
     cpx* sE = sB + FF_TILE * FF_RS;                         // E rows of pass A (natural order k2)
     const int warp = c.tid >> 5;
@@ -232,12 +252,13 @@ MS_DEV void fir_p2_tile(const FirUnit& U, const FirTables& T, cpx* S, int tile, 
     const int taps = U.tap_res >= 0;
     if (taps) { fir_fold_taps(T.res_ptr + U.tap_res, T.tap_off, T.tap_gain, sE, k_first, c.tid); }
     // pass A: rows k_first + w, each warp its own E row
-    fir_p2_pass(U, T, S, sB, sE, k_first, -1, warp, warp, 0, 1, taps, c);
+    fir_p2_pass<PAIR>(U, T, S, sB, sE, k_first, -1, warp, warp, 0, 1, taps, c, filt_r, S_r);
     // pass B: partners 256 - (k_first + w) = rowB0 + (7 - w); in the last tile slot 0 (row 128 again) takes row 0
     const int rowB0 = FF_N - (k_first + 7);
     if (taps && last) { fir_fold_row0(T.res_ptr + U.tap_res, T.tap_gain, sE + 7 * FF_RS, c.tid); }
     const int slot = 7 - warp;
-    fir_p2_pass(U, T, S, sB, sE, rowB0, last ? 0 : -1, slot, warp, (last && warp == 7) ? 0 : 1, (last && warp == 7) ? 1 : 0, taps, c);
+    fir_p2_pass<PAIR>(U, T, S, sB, sE, rowB0, last ? 0 : -1, slot, warp, (last && warp == 7) ? 0 : 1, (last && warp == 7) ? 1 : 0, taps, c,
+                      filt_r, S_r);
 }
 
 // ---- phase 3: inverse columns, valid outputs ------------------------------------------------------------------
@@ -273,8 +294,15 @@ MS_DEV void fir_phase_body(int phase, const FirUnit* MS_RESTRICT units, FirTable
     const FirUnit& U = units[c.by];
     cpx* S = scratch + (size_t)c.by * (FF_N * FF_N);
     if (phase == 1) fir_p1_tile(U, T, S, c.bx, c);
-    else if (phase == 2) fir_p2_tile(U, T, S, c.bx, c);
+    else if (phase == 2) fir_p2_tile<false>(U, T, S, c.bx, c);
     else fir_p3_tile(U, T, S, c.bx, c);
+}
+// phase 2 of pair units (space_ir_stereo): unit c.by is a left channel whose right channel is unit c.by + pair_off, with
+// scratch block c.by + pair_off.  P1 ran for the left unit only; P3 runs for both.
+MS_DEV void fir_p2_pair_body(const FirUnit* MS_RESTRICT units, int pair_off, FirTables T, cpx* scratch, const Ctx& c) {
+    const FirUnit& U = units[c.by];
+    fir_p2_tile<true>(U, T, scratch + (size_t)c.by * (FF_N * FF_N), c.bx, c, units[c.by + pair_off].filt,
+                      scratch + (size_t)(c.by + pair_off) * (FF_N * FF_N));
 }
 
 // ---- reflection taps sorted by residue (off mod 256), once per plan ------------------------------------------------
@@ -340,7 +368,7 @@ __global__ void __launch_bounds__(FF_NTHR, 3) fir_cluster_kernel(const FirUnit* 
         const FirUnit& U = units[u];
         for (int t = rank; t < FF_TILES; t += CL) fir_p1_tile(U, T, S, t, c);
         ff_cluster_sync();
-        for (int t = rank; t < FF_TILES2; t += CL) fir_p2_tile(U, T, S, t, c);
+        for (int t = rank; t < FF_TILES2; t += CL) fir_p2_tile<false>(U, T, S, t, c);
         ff_cluster_sync();
         for (int t = rank; t < FF_TILES; t += CL) fir_p3_tile(U, T, S, t, c);
     }

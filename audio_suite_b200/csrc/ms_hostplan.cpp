@@ -121,7 +121,7 @@ enum { F_base_sr, F_out_dur_s, F_time_unfold, F_peak, F_sat_drive, F_stereo_on, 
        F_mb_b1, F_mb_b2, F_mb_b3, F_mb_u1, F_mb_u2, F_mb_u3, F_mb_roll, F_bandlimit_on, F_bandlimit_out_hz, F_bandlimit_roll_hz,
        F_event_process, F_grains_per_sec, F_max_grains, F_grain_amp_rand, F_grain_offset_on, F_grain_offset_max_ms,
        F_lane_density, F_lane_unfold, F_lane_cutoff, F_lane_stretch, F_er_cloud_on, F_er_taps, F_er_max_ms, F_space_ir_on, F_ir_id,
-       F_env_a, F_env_d, F_env_s, F_env_r, F_env_curve, F_bessel_id, F_COUNT };
+       F_ir_r_id, F_env_a, F_env_d, F_env_s, F_env_r, F_env_curve, F_bessel_id, F_COUNT };
 enum { MODE_GAUSS = 0, MODE_DUST = 1, MODE_NOISE = 2, MODE_SKEW = 3, MODE_RES = 4, MODE_PLAIN = 5 };
 
 struct Lanes { const int64_t* ptr; const double* t; const double* v; };
@@ -198,11 +198,11 @@ static bool same_env(const EnvKey& k, const EnvKey& o) {
 
 // per-render scalars that the second (sequential) pass needs
 struct Scal {
-    std::vector<int64_t> mono_at, fir_of, st_dl, st_dr;
+    std::vector<int64_t> mono_at, fir_of, fir_r_of, st_dl, st_dr;      // fir_r_of: the right channel's row (space_ir_stereo), or -1
     std::vector<int> stereo_on, bessel_id;
     std::vector<double> st_theta, drive, peak;
     void resize(size_t n) {
-        mono_at.resize(n); fir_of.assign(n, -1); st_dl.resize(n); st_dr.resize(n); stereo_on.resize(n); bessel_id.resize(n);
+        mono_at.resize(n); fir_of.assign(n, -1); fir_r_of.assign(n, -1); st_dl.resize(n); st_dr.resize(n); stereo_on.resize(n); bessel_id.resize(n);
         st_theta.resize(n); drive.resize(n); peak.resize(n);
     }
 };
@@ -431,6 +431,13 @@ static int plan_range(Plan& P, Scal& SC, const double* rows, int r0, int r1, con
             fr.x_begin = (int32_t)std::min(x_begin, x_end); fr.x_end = (int32_t)x_end;
             fir_of[r] = (int64_t)P.fir.size();
             P.fir.push_back(fr);
+            const int ir_r_id = ir_id >= 0 ? (int)p[F_ir_r_id] : -1;
+            if (ir_r_id >= 0) {                               // space_ir_stereo: the right channel's row differs only in ir and y
+                P.alg[4] += has_er ? 4 * n_out : 2 * n_out; P.alg[5] += ir_len[ir_r_id];
+                fr.ir = ir_r_id;
+                SC.fir_r_of[r] = (int64_t)P.fir.size();
+                P.fir.push_back(fr);
+            }
             P.h_total += h_len; P.max_h = std::max(P.max_h, h_len);
         }
         mono_at[r] = P.mono_n;
@@ -492,6 +499,7 @@ static void append_part(Plan& P, Scal& S, const Plan& Q, const Scal& QS, std::ve
         P.last.push_back(Q.last[3 * r + 2]);
         S.mono_at.push_back(QS.mono_at[r] + mono_b);
         S.fir_of.push_back(QS.fir_of[r] < 0 ? -1 : QS.fir_of[r] + fir_b);
+        S.fir_r_of.push_back(QS.fir_r_of[r] < 0 ? -1 : QS.fir_r_of[r] + fir_b);
     }
     append(P.out_n, Q.out_n); append(P.srs, Q.srs);
     append(S.stereo_on, QS.stereo_on); append(S.st_dl, QS.st_dl); append(S.st_dr, QS.st_dr); append(S.st_theta, QS.st_theta);
@@ -519,7 +527,27 @@ static void finish_plan(Plan& P, const Scal& S, const double* bessel, int n_coef
         ms_post_render& po = P.post[r];
         memset(&po, 0, sizeof po);
         int mode = 0; int64_t dl = 0, dr = 0, rbuf = 0;
-        if (stereo_on[r]) {
+        if (S.fir_r_of[r] >= 0) {
+            // space_ir_stereo: [yR | right] (even n), [yR | rolled copy | right] (odd n), [yR] (no stereo diffusion)
+            const int64_t y_r = 2 * plane + extra;
+            P.fir[(size_t)S.fir_r_of[r]].y = y_r;
+            extra += n;
+            if (!stereo_on[r]) {
+                mode = 2; rbuf = y_r;
+            } else if (n % 2 == 0) {
+                mode = 3; rbuf = y_r + n; dl = st_dl[r]; dr = st_dr[r];
+                const double* cf = bessel + (size_t)bessel_id[r] * n_coef;
+                for (int k = 0; k < n_coef && k < 2 * MS_POST_K + 1; ++k) po.coef[k] = cf[k];
+                extra += n;
+            } else {
+                mode = 2; rbuf = y_r + 2 * n; dl = st_dl[r]; dr = st_dr[r];
+                P.odd.push_back(y_r); P.odd.push_back(y_r + n); P.odd.push_back(n); P.odd.push_back(dr);
+                Item it; it.n = n; it.src = y_r + n; it.dst = y_r + 2 * n; memset(&it.op, 0, sizeof it.op);
+                it.op.kind = MS_OP_ROT; it.op.alpha = st_theta[r];
+                P.rot.push_back(it);
+                extra += 2 * n;
+            }
+        } else if (stereo_on[r]) {
             dl = st_dl[r]; dr = st_dr[r];
             if (n % 2 == 0) {
                 mode = 1; rbuf = 2 * plane + extra;

@@ -199,8 +199,8 @@ MS_DEV void post_max_body(const PostRender* MS_RESTRICT renders, real* mono, uns
     real* res = red + OLA_NTHR;                      // OLA_TILE results, stream order
     const int len = t1 - t0;
     real m = (real)0.;
-    if (mode == 1) {
-        post_right_tile(R, y, t0, len, win, coef, res, c);
+    if (mode == 1 || mode == 3) {                    // mode 3: the right channel is made from the n samples before rbuf
+        post_right_tile(R, mode == 3 ? mono + R.rbuf - n : y, t0, len, win, coef, res, c);
         real yv[OLA_TILE / OLA_NTHR];
 #pragma unroll
         for (int q = 0; q < OLA_TILE / OLA_NTHR; ++q) { const int j = c.tid + OLA_NTHR * q; yv[q] = j < len ? y[t0 + j] : (real)0.; }
@@ -229,7 +229,7 @@ MS_DEV void post_max_body(const PostRender* MS_RESTRICT renders, real* mono, uns
 #endif
     }
 }
-// pass 2: write interleaved stereo, clipped and scaled to the requested peak
+// pass 2: write interleaved stereo, clipped and scaled to the requested peak (modes 1-3 read the right channel at rbuf)
 MS_DEV void post_write_body(const PostRender* MS_RESTRICT renders, const real* MS_RESTRICT mono, const unsigned long long* MS_RESTRICT maxbits,
                             float2* MS_RESTRICT out, const Ctx& c) {
     const PostRender& R = renders[c.by];

@@ -74,13 +74,15 @@ def read_wav(path):
     return a, int(sr)
 
 
-def load_ir_wav(path):
+def load_ir_wav(path, stereo=False):
     """What on_load_ir hands to render() as `_ir_audio` (main_v2.py:1401-1413): the file as float64, the mean over
     its channels, normalised to a 0.9 peak (normalize, main_v2.py:26-29: untouched when silent).  The file's sample
-    rate is ignored, as in the reference (it is only displayed there)."""
+    rate is ignored, as in the reference (it is only displayed there).  `stereo=True` (EXTENSION, for
+    `space_ir_stereo`) keeps every channel, float64 [frames, channels], with one gain for all of them so that their
+    balance stays as recorded; a one-channel file gives the same 1-D array either way."""
     a, _ = read_wav(path)
     a = a.astype(np.float64)
-    if a.ndim > 1:
+    if a.ndim > 1 and not stereo:
         a = a.mean(axis=1)
     m = float(np.max(np.abs(a))) if a.size else 0.0
     return a if m <= 0 else a * (0.9 / m)

@@ -24,7 +24,7 @@ FIELDS = ("base_sr", "out_dur_s", "time_unfold", "peak", "sat_drive", "stereo_on
           "mb_b1", "mb_b2", "mb_b3", "mb_u1", "mb_u2", "mb_u3", "mb_roll", "bandlimit_on", "bandlimit_out_hz", "bandlimit_roll_hz",
           "event_process", "grains_per_sec", "max_grains", "grain_amp_rand", "grain_offset_on", "grain_offset_max_ms",
           "bp_density", "bp_unfold", "bp_cutoff", "bp_stretch", "er_cloud_on", "er_taps", "er_max_ms", "space_ir_on", "_ir",
-          "env_a", "env_d", "env_s", "env_r", "env_curve", "_bessel")
+          "_ir_r", "env_a", "env_d", "env_s", "env_r", "env_curve", "_bessel")
 _MODE = {m: float(i) for i, m in enumerate(BASIC_MODES)}
 _PROCESS = {"Single": 0.0, "Poisson": 1.0}
 _OFF_FLAGS = ("partial_lock_on", "cep_warp_on", "res_bank_on", "wg_on", "event_feedback_on", "spectral_imprint_on")
@@ -138,6 +138,13 @@ def _marshal(params_list):
                 i = lane_of[text] = float(len(lanes))
                 lanes.append(pts)
         return i
+
+    def ir_index(taps):
+        j = ir_of.get(id(taps))
+        if j is None or irs[j] is not taps:
+            j = ir_of[id(taps)] = len(irs)
+            irs.append(taps)
+        return float(j)
     # the non-numeric fields: one small tuple per render; a sweep repeats the same strings / IR object, so the converted
     # values are memoised per distinct tuple (arrays enter by id(); the objects themselves are kept alive by `params_list`)
     uniq, uniq_of, idx = [], {}, []
@@ -145,22 +152,26 @@ def _marshal(params_list):
     gs = _get_side
     for r, p in enumerate(params_list):
         ir, dig = p.get("_ir_audio"), p.get("_ir_digest")
-        cap = p.get("space_ir_tap_cap", P.IR_TAP_CAP)           # optional key: not in the itemgetter
+        cap = p.get("space_ir_tap_cap", P.IR_TAP_CAP)           # optional keys: not in the itemgetter
         if cap.__class__ is not int or cap < 1:
             cap = P.ir_tap_cap(p)
-        key = gs(p) + (cap, id(ir), id(dig), widths[r])
+        stereo = p.get("space_ir_stereo", False)
+        if stereo.__class__ is not bool:
+            stereo = P.ir_stereo(p)
+        key = gs(p) + (cap, stereo, id(ir), id(dig), widths[r])
         k = uniq_of.get(key)
         if k is None:
-            gen_mode, unfold_mode, process, l0, l1, l2, l3, ir_on, max_samps, _, _, _, w = key
-            ir_id = -1.0
+            gen_mode, unfold_mode, process, l0, l1, l2, l3, ir_on, max_samps, _, _, _, _, w = key
+            ir_id = ir_r_id = -1.0
             if ir_on:
-                taps = dig["taps"] if dig is not None else (P._ir_taps(ir, int(max_samps), cap) if ir is not None else None)
-                if taps is not None:
-                    j = ir_of.get(id(taps))
-                    if j is None or irs[j] is not taps:
-                        j = ir_of[id(taps)] = len(irs)
-                        irs.append(taps)
-                    ir_id = float(j)
+                if dig is not None:
+                    pair = dig["taps"], dig.get("taps_r")
+                else:
+                    pair = P.ir_pair(ir, int(max_samps), cap, stereo) if ir is not None else (None, None)
+                if pair[0] is not None:
+                    ir_id = ir_index(pair[0])
+                    if pair[1] is not None:
+                        ir_r_id = ir_index(pair[1])
             theta = (0.0 if w < 0.0 else 1.0 if w > 1.0 else float(w)) * 0.9
             b = bess_of.get(theta)
             if b is None:
@@ -170,9 +181,9 @@ def _marshal(params_list):
             if gen_mode not in _MODE or process not in _PROCESS:
                 raise Unsupported(r)
             uniq.append((_MODE[gen_mode], 0.0 if unfold_mode == _CLASSIC else 1.0, _PROCESS[process],
-                         lane_id(l0), lane_id(l1), lane_id(l2), lane_id(l3), ir_id, b))
+                         lane_id(l0), lane_id(l1), lane_id(l2), lane_id(l3), ir_id, ir_r_id, b))
         idx.append(k)
-    rows[:, _SIDE_COL] = np.array(uniq, dtype=np.float64).reshape(len(uniq), 9)[np.array(idx, dtype=np.intp)]
+    rows[:, _SIDE_COL] = np.array(uniq, dtype=np.float64).reshape(len(uniq), len(_SIDE_COL))[np.array(idx, dtype=np.intp)]
     lane_ptr = np.zeros(len(lanes) + 1, np.int64)
     for i, pts in enumerate(lanes):
         lane_ptr[i + 1] = lane_ptr[i] + len(pts)
@@ -184,7 +195,7 @@ def _marshal(params_list):
     return rows, lane_ptr, lane_t, lane_v, irs, ir_len, btab
 
 
-_SIDE_COL = [FIELDS.index(k) for k in ("gen_mode", "unfold_mode", "event_process", "bp_density", "bp_unfold", "bp_cutoff", "bp_stretch", "_ir", "_bessel")]
+_SIDE_COL = [FIELDS.index(k) for k in ("gen_mode", "unfold_mode", "event_process", "bp_density", "bp_unfold", "bp_cutoff", "bp_stretch", "_ir", "_ir_r", "_bessel")]
 
 
 def default_threads():

@@ -256,7 +256,8 @@ class RenderPlan:
     feedback: Optional[float] = None        # event_feedback_amt when event feedback is on (M:731-734)
     er_offs: Optional[np.ndarray] = None    # int32 tap delays (0 < off < out_n)
     er_gains: Optional[np.ndarray] = None   # float64
-    ir: Optional[np.ndarray] = None         # float64 mono taps (<= space_ir_tap_cap) or None
+    ir: Optional[np.ndarray] = None         # float64 mono taps (<= space_ir_tap_cap) or None; with ir_r: the left channel
+    ir_r: Optional[np.ndarray] = None       # space_ir_stereo with a two-column IR: float64 right-channel taps, else None
     stereo_on: bool = False
     stereo_dl: int = 0
     stereo_dr: int = 0
@@ -286,6 +287,7 @@ def plan_render(params) -> RenderPlan:
     """Scalar half of render() (M:589-646, 742-753, 760-781)."""
     check_supported(params)
     cap = ir_tap_cap(params)
+    stereo_ir = ir_stereo(params)
     base_sr = int(params["base_sr"])
     out_dur = float(params["out_dur_s"])
     out_n = int(max(1, round(out_dur * base_sr)))
@@ -438,9 +440,9 @@ def plan_render(params) -> RenderPlan:
         rp.er_offs, rp.er_gains = offs[keep].astype(np.int32), gains[keep]
     if params["space_ir_on"]:
         if digest is not None:
-            rp.ir = digest["taps"]
+            rp.ir, rp.ir_r = digest["taps"], digest.get("taps_r")
         elif ir_audio is not None:
-            rp.ir = _ir_taps(ir_audio, int(params["space_ir_max_samps"]), cap)
+            rp.ir, rp.ir_r = ir_pair(ir_audio, int(params["space_ir_max_samps"]), cap, stereo_ir)
     if params["stereo_on"] and out_n >= 64:   # M:426: shorter outputs are duplicated
         w = float(min(max(float(params["stereo_width"]), 0.0), 1.0))
         rp.stereo_on = True
@@ -477,6 +479,46 @@ def ir_tap_cap(params):
     if isinstance(cap, (bool, np.bool_)) or not isinstance(cap, (int, np.integer)) or cap < 1:
         raise ValueError(f"space_ir_tap_cap must be an int >= 1 or None, not {cap!r}")
     return int(cap)
+
+
+def ir_stereo(params):
+    """The optional key `space_ir_stereo` (EXTENSION; the reference mixes every IR to mono, M:438-445): True convolves
+    the render with each channel of a two-column IR separately (`ir_pair`).  Only a bool (numpy's included) is taken."""
+    on = params.get("space_ir_stereo", False)
+    if not isinstance(on, (bool, np.bool_)):
+        raise ValueError(f"space_ir_stereo must be a bool, not {on!r}")
+    return bool(on)
+
+
+_PAIR_CACHE = {}
+
+
+def ir_pair(ir, max_samps, cap=IR_TAP_CAP, stereo=False):
+    """(left taps, right taps) of the IR: (`_ir_taps`, None) unless `stereo` and the IR has two columns; then the
+    reference's slice, "< 8 values" test and cut to `cap` rows, and instead of the mono mix column 0 and column 1 as
+    contiguous float64 arrays, each at most IR_TAP_LIMIT taps.  More than two columns raise ValueError.  Cached per IR
+    object, so a sweep shares one pair of arrays (and one copy of each in the IR pool of its tables)."""
+    a = np.asarray(ir)
+    if stereo and (a.ndim > 2 or (a.ndim == 2 and a.shape[1] > 2)):
+        raise ValueError(f"space_ir_stereo takes an impulse response of one or two channels, not shape {a.shape}")
+    if not stereo or a.ndim < 2 or a.shape[1] == 1:
+        return _ir_taps(ir, max_samps, cap), None
+    key = (array_signature(ir), max_samps, cap)
+    hit = _PAIR_CACHE.get(key)
+    if hit is not None and hit[0] is ir:
+        return hit[1]
+    h = a[:max_samps]
+    pair = (None, None)
+    if h.size >= 8:                           # the reference's test: size counts both channels
+        h = h if cap is None else h[:cap]
+        if h.shape[0] > IR_TAP_LIMIT:
+            raise ValueError(f"an impulse response of {h.shape[0]} taps per channel is outside the accelerated path "
+                             f"(at most {IR_TAP_LIMIT}; lower space_ir_tap_cap or space_ir_max_samps)")
+        pair = (np.array(h[:, 0], dtype=np.float64), np.array(h[:, 1], dtype=np.float64))
+    if len(_PAIR_CACHE) > 64:
+        _PAIR_CACHE.clear()
+    _PAIR_CACHE[key] = (ir, pair)
+    return pair
 
 
 def _ir_taps(ir, max_samps, cap=IR_TAP_CAP):
@@ -630,7 +672,8 @@ def _slim_params(p):
     """Copy of a parameter dict for the planning workers: the impulse response is replaced by what the planner
     keeps of it -- `_ir_digest = {"taps": convolve_ir_short's view (M:439-443: float64 mono mix of the first
     min(space_ir_max_samps, space_ir_tap_cap) rows, None when that slice has fewer than 8 values), "frag": gen_ir_fragment's
-    source (M:335-340: the float64 mono mix of the WHOLE response, None when it has fewer than 32 values)}` -- so a
+    source (M:335-340: the float64 mono mix of the WHOLE response, None when it has fewer than 32 values), "taps_r": the
+    right channel under space_ir_stereo (`ir_pair`; "taps" is then the left one), else None}` -- so a
     multi-second stereo IR is not pickled per render and both size tests are made on the original array.  The
     digests are cached per IR object, so renders sharing an IR share the arrays (one pickle memo entry per piece)."""
     ir = p.get("_ir_audio")
@@ -641,6 +684,6 @@ def _slim_params(p):
     frag = None
     if p["gen_mode"] == "IR fragment" and np.asarray(ir).size >= 32:
         frag = _mono64(ir)
-    taps = _ir_taps(ir, int(p["space_ir_max_samps"]), ir_tap_cap(p)) if p["space_ir_on"] else None
-    q["_ir_digest"] = {"taps": taps, "frag": frag}
+    taps, taps_r = ir_pair(ir, int(p["space_ir_max_samps"]), ir_tap_cap(p), ir_stereo(p)) if p["space_ir_on"] else (None, None)
+    q["_ir_digest"] = {"taps": taps, "taps_r": taps_r, "frag": frag}
     return q

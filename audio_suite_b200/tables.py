@@ -11,7 +11,7 @@ Every table is a record array with the layout of its struct in include/microsoun
 workspace can supply (the `z*` spectrum offsets, scratch offsets) stay 0 here and are filled on upload.
 
 Buffers (offsets in elements): pool (real; per-event signals), mono (real; per chunk:
-[OLA plane | FIR plane | right channels / odd-length scratch]), out (float32 frames), hpool (real;
+[OLA plane | FIR plane | right channels / odd-length scratch / right-channel FIR outputs]), out (float32 frames), hpool (real;
 combined FIR taps), taps (reflection delays/gains), irs (deduplicated IR taps), dust (impulses).
 """
 from __future__ import annotations
@@ -194,7 +194,18 @@ def pack_chunk(plans) -> Tables:
     mono_at = []
     last = np.zeros(R, LAST)
     last[:] = (-1, -1, -1)
-    fir_of = {}
+    fir_of, fir_r_of = {}, {}
+
+    def ir_slot(h):
+        """(offset, length) of taps `h` in the deduplicated IR pool"""
+        nonlocal n_ir
+        key = h.ctypes.data if h.flags.owndata else h.tobytes()
+        hit = ir_index.get(key)
+        if hit is None or (not isinstance(key, bytes) and hit[2] is not h):
+            hit = ir_index[key] = (n_ir, h.size, h)
+            irs.append(h)
+            n_ir += h.size
+        return hit
     alg = dict(synth=0, tilt_spectral=0, grain_spectral=0, overlap_add=0, fir_in=0, fir_taps=0, post=0)
     env_seen = {}
     e = 0
@@ -340,12 +351,7 @@ def pack_chunk(plans) -> Tables:
         has_er = rp.er_offs is not None and rp.er_offs.size > 0
         if has_er or rp.ir is not None:
             if rp.ir is not None:
-                key = rp.ir.ctypes.data if rp.ir.flags.owndata else rp.ir.tobytes()
-                hit = ir_index.get(key)
-                if hit is None or (not isinstance(key, bytes) and hit[2] is not rp.ir):
-                    hit = ir_index[key] = (n_ir, rp.ir.size, rp.ir)
-                    irs.append(rp.ir)
-                    n_ir += rp.ir.size
+                hit = ir_slot(rp.ir)
                 alg["fir_in"] += 2 * n
                 alg["fir_taps"] += rp.ir.size
             else:
@@ -369,6 +375,11 @@ def pack_chunk(plans) -> Tables:
                 x_begin = 1                      # env[0] = 0 ** curve = 0 (main_v2.py:181-182)
             fir_of[r] = len(fir)
             fir.append((ir_at, ir_len, h_len, h_total, t0, n_taps, mono_n, 0, n, min(x_begin, x_end), x_end, 0))
+            if rp.ir_r is not None:              # space_ir_stereo: the right channel's row differs only in `ir` and `y`
+                fir_r_of[r] = len(fir)
+                fir.append((ir_slot(rp.ir_r)[0],) + fir[-1][1:])
+                alg["fir_in"] += 2 * n * (2 if has_er else 1)
+                alg["fir_taps"] += rp.ir_r.size
             h_total += h_len
             max_h = max(max_h, h_len)
         mono_at.append(mono_n)
@@ -387,7 +398,26 @@ def pack_chunk(plans) -> Tables:
             fir_arr[fir_of[r]]["y"] = y
         mode, dl, dr, rbuf = 0, 0, 0, 0
         coef = np.zeros(2 * _abi.POST_K + 1)
-        if rp.stereo_on:
+        if r in fir_r_of:
+            # space_ir_stereo: the right channel's FIR output yR opens the render's extra region, the right channel
+            # proper is made from it: [yR | right] (even n, Bessel FIR in the max pass), [yR | rolled copy | right]
+            # (odd n), or [yR] itself (no stereo diffusion)
+            y_r = 2 * plane + extra
+            fir_arr[fir_r_of[r]]["y"] = y_r
+            extra += n
+            if not rp.stereo_on:
+                mode, rbuf = 2, y_r
+            elif n % 2 == 0:
+                mode, coef, rbuf, dl, dr = 3, bessel_coeffs(rp.stereo_theta), y_r + n, rp.stereo_dl, rp.stereo_dr
+                extra += n
+            else:
+                mode, rbuf, dl, dr = 2, y_r + 2 * n, rp.stereo_dl, rp.stereo_dr
+                odd.append((y_r, y_r + n, n, dr))
+                op = _abi.SpecOp()
+                op.kind, op.alpha = _abi.OP_ROT, rp.stereo_theta
+                rot.append((n, y_r + n, y_r + 2 * n, op))
+                extra += 2 * n
+        elif rp.stereo_on:
             dl, dr = rp.stereo_dl, rp.stereo_dr
             if n % 2 == 0:
                 mode, coef, rbuf = 1, bessel_coeffs(rp.stereo_theta), 2 * plane + extra     # right channel, written by the max pass

@@ -235,9 +235,11 @@ typedef struct {
 typedef struct {
     int64_t y;                /* mono input offset */
     int64_t out;              /* output offset in frames */
-    int64_t rbuf;             /* offset in `mono` of the right channel: written by ms_post (mode 1), read (mode 2) */
+    int64_t rbuf;             /* offset in `mono` of the right channel: written by ms_post (modes 1, 3), read (mode 2) */
     int32_t n;
-    int32_t stereo_mode;      /* 0 duplicate, 1 Bessel FIR (even n), 2 precomputed */
+    int32_t stereo_mode;      /* 0 duplicate, 1 Bessel FIR of y (even n), 2 precomputed, 3 Bessel FIR (even n) of the n
+                                 samples at rbuf - n (a second mono signal: the right channel's own FIR output under
+                                 space_ir_stereo), written at rbuf; the left channel is roll(y, dl) in modes 1-3 */
     int32_t dl, dr;
     double drive, inv_tanh_drive, peak;
     double coef[2 * MS_POST_K + 1];  /* J_m(theta), m = -K..K */

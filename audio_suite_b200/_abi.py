@@ -118,6 +118,11 @@ class PostRender(C.Structure):
                 ("coef", C.c_double * (2 * POST_K + 1))]
 
 
+class ExportRender(C.Structure):
+    _fields_ = [("out", C.c_int64), ("out_end", C.c_int64), ("bank", C.c_int64), ("bank_end", C.c_int64),
+                ("rate", C.c_int32 * 4)]             # up, down, half, taps per phase
+
+
 _P, _I, _Z = C.c_void_p, C.c_int, C.c_size_t
 _COMMON = {
     "ms_version": (C.c_int, []),
@@ -159,6 +164,7 @@ _STAGES = {
     "ms_fir_run": (_I, [_P, _P]),
     "ms_fir_destroy": (None, [_P]),
     "ms_post": (_I, [_P, _I, _I, _P, _P, _P, _P]),
+    "ms_post_export": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P, _P]),
     "ms_roll": (_I, [_P, _P, _I, _I, _P]),
     "ms_polyphase_decimate": (_I, [_P, C.c_int64, _I, _I, _P, _I, _I, _P, C.c_int64, _P]),
 }

@@ -20,6 +20,7 @@
 #include <algorithm>
 #include <atomic>
 #include <thread>
+#include <numeric>
 #include "../../include/microsound_b200.h"
 #include "ms_zig_exp_tables.h"
 
@@ -121,7 +122,7 @@ enum { F_base_sr, F_out_dur_s, F_time_unfold, F_peak, F_sat_drive, F_stereo_on, 
        F_mb_b1, F_mb_b2, F_mb_b3, F_mb_u1, F_mb_u2, F_mb_u3, F_mb_roll, F_bandlimit_on, F_bandlimit_out_hz, F_bandlimit_roll_hz,
        F_event_process, F_grains_per_sec, F_max_grains, F_grain_amp_rand, F_grain_offset_on, F_grain_offset_max_ms,
        F_lane_density, F_lane_unfold, F_lane_cutoff, F_lane_stretch, F_er_cloud_on, F_er_taps, F_er_max_ms, F_space_ir_on, F_ir_id,
-       F_ir_r_id, F_env_a, F_env_d, F_env_s, F_env_r, F_env_curve, F_bessel_id, F_COUNT };
+       F_ir_r_id, F_env_a, F_env_d, F_env_s, F_env_r, F_env_curve, F_bessel_id, F_export_sr, F_COUNT };
 enum { MODE_GAUSS = 0, MODE_DUST = 1, MODE_NOISE = 2, MODE_SKEW = 3, MODE_RES = 4, MODE_PLAIN = 5 };
 
 struct Lanes { const int64_t* ptr; const double* t; const double* v; };
@@ -186,7 +187,9 @@ struct Plan {
     std::vector<Item> tilt, grain, rot;
     std::vector<int64_t> odd;                       // rows of 4: y_at, scratch, n, dr
     std::vector<int64_t> out_at, out_n, y_at, last, srs, ir_order;
-    int64_t pool_n, mono_n, frames, h_total, max_h, max_out_n, env_n, n_ir;
+    std::vector<ms_export_render> exp;              // renders with export_sr: resampler rows ...
+    std::vector<int64_t> export_of, ratios, bank_at; // ... their render indices; distinct (up, down) in order of first use
+    int64_t pool_n, mono_n, frames, h_total, max_h, max_out_n, env_n, n_ir, n_bank;
     int64_t alg[7];                                 // synth, tilt_spectral, grain_spectral, overlap_add, fir_in, fir_taps, post
     std::string error; int error_render;
 };
@@ -199,9 +202,11 @@ static bool same_env(const EnvKey& k, const EnvKey& o) {
 // per-render scalars that the second (sequential) pass needs
 struct Scal {
     std::vector<int64_t> mono_at, fir_of, fir_r_of, st_dl, st_dr;      // fir_r_of: the right channel's row (space_ir_stereo), or -1
+    std::vector<int64_t> ex_up, ex_down;                                 // export_sr as up / down in lowest terms (0: none)
     std::vector<int> stereo_on, bessel_id;
     std::vector<double> st_theta, drive, peak;
     void resize(size_t n) {
+        ex_up.assign(n, 0); ex_down.assign(n, 0);
         mono_at.resize(n); fir_of.assign(n, -1); fir_r_of.assign(n, -1); st_dl.resize(n); st_dr.resize(n); stereo_on.resize(n); bessel_id.resize(n);
         st_theta.resize(n); drive.resize(n); peak.resize(n);
     }
@@ -454,6 +459,8 @@ static int plan_range(Plan& P, Scal& SC, const double* rows, int r0, int r1, con
             st_theta[r] = w * 0.9;
         }
         drive[r] = p[F_sat_drive]; peak[r] = p[F_peak]; bessel_id[r] = (int)p[F_bessel_id];
+        const long long ex_sr = (long long)p[F_export_sr];          // validated by plan.export_ratio; 0: none
+        if (ex_sr > 0) { const long long g = std::gcd(base_sr, ex_sr); SC.ex_up[r] = ex_sr / g; SC.ex_down[r] = base_sr / g; }
         P.out_n[r] = n_out;
     }
     return 0;
@@ -504,6 +511,7 @@ static void append_part(Plan& P, Scal& S, const Plan& Q, const Scal& QS, std::ve
     append(P.out_n, Q.out_n); append(P.srs, Q.srs);
     append(S.stereo_on, QS.stereo_on); append(S.st_dl, QS.st_dl); append(S.st_dr, QS.st_dr); append(S.st_theta, QS.st_theta);
     append(S.drive, QS.drive); append(S.peak, QS.peak); append(S.bessel_id, QS.bessel_id);
+    append(S.ex_up, QS.ex_up); append(S.ex_down, QS.ex_down);
     P.pool_n += Q.pool_n; P.mono_n += Q.mono_n; P.h_total += Q.h_total;
     P.max_h = std::max(P.max_h, Q.max_h); P.max_out_n = std::max(P.max_out_n, Q.max_out_n);
     for (int k = 0; k < 7; ++k) P.alg[k] += Q.alg[k];
@@ -565,8 +573,23 @@ static void finish_plan(Plan& P, const Scal& S, const double* bessel, int n_coef
         }
         po.y = y; po.out = P.frames; po.rbuf = rbuf; po.n = (int32_t)n; po.stereo_mode = mode; po.dl = (int32_t)dl; po.dr = (int32_t)dr;
         po.drive = drive[r]; po.inv_tanh_drive = drive[r] > 0 ? 1.0 / tanh(drive[r]) : 1.0; po.peak = peak[r];
+        // export_sr: ceil(n up / down) frames through the polyphase bank of the ratio (decimate.polyphase_bank fills the pool)
+        int64_t n_x = n;
+        if (S.ex_up[r] > 0) {
+            const int64_t up = S.ex_up[r], down = S.ex_down[r], half = 10 * std::max(up, down);
+            const int64_t taps = half / up + (up - 1 + half) / up + 1;
+            n_x = (n * up + down - 1) / down;
+            size_t k = 0;
+            for (; k < P.bank_at.size(); ++k) if (P.ratios[2 * k] == up && P.ratios[2 * k + 1] == down) break;
+            if (k == P.bank_at.size()) { P.ratios.push_back(up); P.ratios.push_back(down); P.bank_at.push_back(P.n_bank); P.n_bank += up * taps; }
+            ms_export_render e;
+            e.out = P.frames; e.out_end = P.frames + n_x; e.bank = P.bank_at[k]; e.bank_end = P.bank_at[k] + up * taps;
+            e.rate[0] = (int32_t)up; e.rate[1] = (int32_t)down; e.rate[2] = (int32_t)half; e.rate[3] = (int32_t)taps;
+            P.exp.push_back(e); P.export_of.push_back(r);
+        }
         P.out_at[r] = P.frames; P.y_at[r] = y;
-        P.frames += n;
+        P.frames += n_x;
+        P.out_n[r] = n_x;
         P.alg[6] += n;
     }
     // ---- envelopes shared by several renders are tabulated once
@@ -592,7 +615,7 @@ static void finish_plan(Plan& P, const Scal& S, const double* bessel, int n_coef
 // A slice in blocks of HP_BLOCK renders, the blocks handed out to `threads` threads and appended in order.
 static const int HP_BLOCK = 32;
 static int plan_chunk(Plan& P, const double* rows, int R, const Lanes& L, const int64_t* ir_len, const double* bessel, int n_coef, int threads) {
-    P.pool_n = P.mono_n = P.frames = P.h_total = P.max_h = P.max_out_n = P.env_n = P.n_ir = 0;
+    P.pool_n = P.mono_n = P.frames = P.h_total = P.max_h = P.max_out_n = P.env_n = P.n_ir = P.n_bank = 0;
     memset(P.alg, 0, sizeof P.alg);
     const int nb = (R + HP_BLOCK - 1) / HP_BLOCK;
     std::vector<Plan> parts((size_t)nb); std::vector<Scal> scal((size_t)nb);
@@ -649,14 +672,15 @@ void* ms_hp_plan(const double* rows, int n_renders, const int64_t* lane_ptr, con
 }
 const char* ms_hp_error(void* h, int* render) { Plan* P = (Plan*)h; *render = P->error_render; return P->error.c_str(); }
 // sizes: element counts of every exported array, in the order of ms_hp_export
-enum { HP_SY, HP_OLA_R, HP_ENV_REPS, HP_OLA_E, HP_FIR, HP_POST, HP_TAPS, HP_DUST, HP_TILT, HP_GRAIN, HP_ROT, HP_ODD, HP_IRS, HP_NSIZES };
+enum { HP_SY, HP_OLA_R, HP_ENV_REPS, HP_OLA_E, HP_FIR, HP_POST, HP_TAPS, HP_DUST, HP_TILT, HP_GRAIN, HP_ROT, HP_ODD, HP_IRS, HP_EXPORT,
+       HP_RATIOS, HP_NSIZES };
 void ms_hp_sizes(void* h, int64_t* sizes, int64_t* scalars /*pool_n mono_n frames h_total max_h max_out_n env_n, alg[7]*/) {
     Plan* P = (Plan*)h;
     sizes[HP_SY] = (int64_t)P->sy1.size(); sizes[HP_OLA_R] = (int64_t)P->ola_r.size(); sizes[HP_ENV_REPS] = (int64_t)P->env_reps.size();
     sizes[HP_OLA_E] = (int64_t)P->ola_e.size(); sizes[HP_FIR] = (int64_t)P->fir.size(); sizes[HP_POST] = (int64_t)P->post.size();
     sizes[HP_TAPS] = (int64_t)P->tap_off.size(); sizes[HP_DUST] = (int64_t)P->dust_pos.size(); sizes[HP_TILT] = (int64_t)P->tilt.size();
     sizes[HP_GRAIN] = (int64_t)P->grain.size(); sizes[HP_ROT] = (int64_t)P->rot.size(); sizes[HP_ODD] = (int64_t)P->odd.size() / 4;
-    sizes[HP_IRS] = (int64_t)P->ir_order.size();
+    sizes[HP_IRS] = (int64_t)P->ir_order.size(); sizes[HP_EXPORT] = (int64_t)P->exp.size(); sizes[HP_RATIOS] = (int64_t)P->bank_at.size();
     scalars[0] = P->pool_n; scalars[1] = P->mono_n; scalars[2] = P->frames; scalars[3] = P->h_total; scalars[4] = P->max_h;
     scalars[5] = P->max_out_n; scalars[6] = P->env_n;
     for (int i = 0; i < 7; ++i) scalars[7 + i] = P->alg[i];
@@ -664,7 +688,8 @@ void ms_hp_sizes(void* h, int64_t* sizes, int64_t* scalars /*pool_n mono_n frame
 void ms_hp_export(void* h, void* sy1, void* sy2, void* ola_r, void* env_reps, void* ola_e, void* fir, void* post,
                   int32_t* tap_off, double* tap_delay, double* tap_raw, int32_t* dust_pos, double* dust_val,
                   void* tilt, void* grain, void* rot,
-                  int64_t* odd, int64_t* ir_order, int64_t* out_at, int64_t* out_n, int64_t* y_at, int64_t* last, int64_t* srs) {
+                  int64_t* odd, int64_t* ir_order, int64_t* out_at, int64_t* out_n, int64_t* y_at, int64_t* last, int64_t* srs,
+                  void* exp, int64_t* export_of, int64_t* ratios) {
     Plan* P = (Plan*)h;
     auto cp = [](void* d, const void* s, size_t b) { if (b) memcpy(d, s, b); };
     cp(sy1, P->sy1.data(), P->sy1.size() * sizeof(ms_synth_evt)); cp(sy2, P->sy2.data(), P->sy2.size() * sizeof(ms_synth_evt));
@@ -678,6 +703,8 @@ void ms_hp_export(void* h, void* sy1, void* sy2, void* ola_r, void* env_reps, vo
     cp(odd, P->odd.data(), P->odd.size() * 8); cp(ir_order, P->ir_order.data(), P->ir_order.size() * 8);
     cp(out_at, P->out_at.data(), P->out_at.size() * 8); cp(out_n, P->out_n.data(), P->out_n.size() * 8); cp(y_at, P->y_at.data(), P->y_at.size() * 8);
     cp(last, P->last.data(), P->last.size() * 8); cp(srs, P->srs.data(), P->srs.size() * 8);
+    cp(exp, P->exp.data(), P->exp.size() * sizeof(ms_export_render)); cp(export_of, P->export_of.data(), P->export_of.size() * 8);
+    cp(ratios, P->ratios.data(), P->ratios.size() * 8);
 }
 void ms_hp_free(void* h) { delete (Plan*)h; }
 }

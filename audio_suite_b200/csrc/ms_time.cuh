@@ -259,6 +259,94 @@ MS_DEV void post_write_body(const PostRender* MS_RESTRICT renders, const real* M
         if (i < t1) o[i] = make_float2((float)(soft_clip(lv[q], drive, inv_t) * scale), (float)(soft_clip(rv[q], drive, inv_t) * scale));
     }
 }
+// ---- EXTENSION: export sample rate, the write pass of an exporting render (include/microsound_b200.h, ms_post_export) ----
+// out[m] = sum_s x[q + s] bank[p][s + A], q = (m down) div up, p = (m down) mod up, x = soft_clip(.) * scale of each channel
+// (zero outside [0, n)).  grid = (ceil(max output frames / EXP_TILE), renders), OLA_NTHR threads; a thread owns the outputs
+// m0 + tid + OLA_NTHR k (stores of a warp are consecutive float2).  The tile's input window -- both channels, clipped and
+// scaled on load -- goes through shared memory in rounds of EXP_CH frames; every output adds the taps that fall in the
+// round, in ascending s, into the same two accumulators, so the sum does not depend on the rounds (heavy decimation
+// spans many rounds: at 1/640 a tile of outputs reads 655360 input frames).  One bank load (read through L1) feeds both
+// channels.  Products m down reach 4e10 (C4 at 640/147): 64-bit until the offsets inside the tile.
+typedef ms_export_render ExportRender;
+#define EXP_TILE 1024                // output frames per CTA
+#define EXP_CH 2048                  // input frames per round of the staged window
+MS_DEV void post_export_body(const PostRender* MS_RESTRICT renders, const ExportRender* MS_RESTRICT exps, const real* MS_RESTRICT mono,
+                             const unsigned long long* MS_RESTRICT maxbits, const real* MS_RESTRICT bank, float2* MS_RESTRICT out,
+                             const Ctx& c) {
+    const PostRender& R = renders[c.by];
+    const ExportRender E = exps[c.by];
+    const long long out_n = E.out_end - E.out;
+    const long long m0 = (long long)c.bx * EXP_TILE;
+    if (m0 >= out_n) return;
+    const int cnt = (int)(out_n - m0 < EXP_TILE ? out_n - m0 : EXP_TILE);
+    const long long up = E.rate[0], down = E.rate[1];
+    const int taps = E.rate[3], A = E.rate[2] / E.rate[0];
+    const int n = R.n, mode = R.stereo_mode;
+    union { double f; unsigned long long u; } cv; cv.u = maxbits[c.by];
+    const real drive = (real)R.drive, inv_t = (real)R.inv_tanh_drive;
+    const real top = soft_clip((real)cv.f, drive, inv_t);
+    const real scale = top > (real)0. ? (real)R.peak / top : (real)1.0;
+    const real* y = mono + R.y;
+    const real* rsrc = mode ? mono + R.rbuf : y;
+    const int dlm = mode ? wrap_idx((long long)R.dl, n) : 0;           // left channel = roll(y, dl)
+    const long long w0 = m0 * down / up - A;                            // input frame of window slot 0
+    const int wlen = (int)((m0 + cnt - 1) * down / up + (taps - A) - w0);
+    constexpr int NQ = EXP_TILE / OLA_NTHR, NL = EXP_CH / OLA_NTHR;
+    int rq[NQ];                                  // window slot of q(m), -1: no output
+    const real* tp[NQ];                          // taps of the output's phase, at s = 0
+    real aL[NQ], aR[NQ];
+#pragma unroll
+    for (int k = 0; k < NQ; ++k) {
+        const int i = c.tid + OLA_NTHR * k;
+        const long long md = (m0 + i) * down, q = md / up;
+        rq[k] = i < cnt ? (int)(q - w0) : -1;
+        tp[k] = bank + E.bank + (md - q * up) * taps + A;
+        aL[k] = aR[k] = (real)0.;
+    }
+    real* wl = (real*)c.smem;                    // EXP_CH frames of each channel
+    real* wr = wl + EXP_CH;
+    for (int c0 = 0; c0 < wlen; c0 += EXP_CH) {
+        const int clen = wlen - c0 < EXP_CH ? wlen - c0 : EXP_CH;
+        // every load of the round is issued before the first store
+        real lv[NL], rv[NL];
+#pragma unroll
+        for (int k = 0; k < NL; ++k) {
+            const int j = c.tid + OLA_NTHR * k;
+            const long long J = w0 + c0 + j;
+            lv[k] = rv[k] = (real)0.;
+            if (j < clen && J >= 0 && J < n) {
+                int li = (int)J - dlm; if (li < 0) li += n;
+                lv[k] = y[li];
+                rv[k] = rsrc[J];
+            }
+        }
+        if (c0) c.sync();                        // the previous round has been read
+#pragma unroll
+        for (int k = 0; k < NL; ++k) {
+            const int j = c.tid + OLA_NTHR * k;
+            if (j < clen) { wl[j] = soft_clip(lv[k], drive, inv_t) * scale; wr[j] = soft_clip(rv[k], drive, inv_t) * scale; }
+        }
+        c.sync();
+#pragma unroll
+        for (int k = 0; k < NQ; ++k) {
+            if (rq[k] < 0) continue;
+            const int d = rq[k] - c0;            // slot of x[q] in this round
+            const int s_lo = -A > -d ? -A : -d;
+            const int s_hi = taps - 1 - A < clen - 1 - d ? taps - 1 - A : clen - 1 - d;
+            real l = aL[k], r = aR[k];
+            for (int s = s_lo; s <= s_hi; ++s) {
+                const real h = __ldg(&tp[k][s]);
+                l += h * wl[d + s];
+                r += h * wr[d + s];
+            }
+            aL[k] = l; aR[k] = r;
+        }
+    }
+    float2* o = out + E.out + m0;
+#pragma unroll
+    for (int k = 0; k < NQ; ++k)
+        if (rq[k] >= 0) o[c.tid + OLA_NTHR * k] = make_float2((float)aL[k], (float)aR[k]);
+}
 // circular shift used by the odd-length stereo path: dst[i] = src[(i + shift) mod n]
 MS_DEV void roll_body(const real* MS_RESTRICT src, real* MS_RESTRICT dst, int n, int shift, const Ctx& c) {
     for (int i = c.bx * c.nthr + c.tid; i < n; i += c.nthr * 64) dst[i] = src[wrap_idx((long long)i + shift, n)];

@@ -14,13 +14,39 @@ import numpy as np
 from . import _abi
 
 
-def design_taps(q, half_len_per_q=10, beta=5.0):
-    """The low-pass resample_poly(x, 1, q) designs: firwin(2 * 10 q + 1, 1 / q, window=('kaiser', 5.0)), restated with
-    numpy (windowed sinc, unit DC gain).  Returns float64 taps of odd length."""
-    half = half_len_per_q * int(q)
+def resample_taps(up, down, half_len_per_q=10, beta=5.0):
+    """The filter resample_poly(x, up, down) designs: up * firwin(2 * 10 q + 1, 1 / q, window=('kaiser', 5.0)) with
+    q = max(up, down), restated with numpy (windowed sinc, unit DC gain before the factor up).  Float64 taps of odd length."""
+    q = max(int(up), int(down))
+    half = half_len_per_q * q
     m = np.arange(-half, half + 1, dtype=np.float64)
     h = (1.0 / q) * np.sinc(m / q) * np.kaiser(2 * half + 1, beta)
-    return h / np.sum(h)
+    return int(up) * (h / np.sum(h))
+
+
+def design_taps(q, half_len_per_q=10, beta=5.0):
+    """The low-pass resample_poly(x, 1, q) designs (resample_taps with up = 1)."""
+    return resample_taps(1, q, half_len_per_q, beta)
+
+
+_BANKS = {}
+
+
+def polyphase_bank(up, down):
+    """resample_taps(up, down) as the polyphase bank ms_post_export reads (include/microsound_b200.h): float64
+    [up, taps], row p holding g[p + half - s up] for s = -A .. taps - 1 - A (zero outside g), A = half // up.
+    Returns (half, taps, bank); cached per ratio, so a sweep shares one bank."""
+    key = (int(up), int(down))
+    hit = _BANKS.get(key)
+    if hit is None:
+        g = resample_taps(*key)
+        half = (len(g) - 1) // 2
+        u = key[0]
+        a, b = half // u, (u - 1 + half) // u
+        k = np.arange(u)[:, None] + half - np.arange(-a, b + 1)[None, :] * u
+        bank = np.where((k >= 0) & (k <= 2 * half), g[np.clip(k, 0, 2 * half)], 0.0)
+        hit = _BANKS[key] = (half, a + b + 1, np.ascontiguousarray(bank))
+    return hit
 
 
 def upfirdn_decimate(x, h, q, device, precision="f64"):

@@ -13,6 +13,7 @@ Stage order (one batched launch sequence for all renders):
   overlap-add placement + ADSR                                   ms_overlap_add
   reflection cloud (+) impulse response as one FIR, overlap-save ms_fir_*
   stereo diffusion, soft clip, normalise                         ms_post
+  [... and for renders with `export_sr`: resampled to that rate]  ms_post_export
 """
 from __future__ import annotations
 
@@ -260,7 +261,20 @@ class BatchRenderer:
         self.n_env = len(t.env_reps)
         self.envpool = dev.empty(max(1, t.env_n), real)
         self.d_env_reps = dev.upload(t.env_reps) if self.n_env else None
-        self.d_post = dev.upload(t.post)
+        # export_sr: the renders that have one run ms_post_export instead of ms_post, on the maxbits after the plain ones
+        self.n_export = len(t.export)
+        if self.n_export:
+            exporting = np.zeros(self.n_renders, bool)
+            exporting[t.export_of] = True
+            plain = t.post[~exporting]
+            self.n_plain, self.max_n_plain = len(plain), int(plain["n"].max()) if len(plain) else 0
+            self.d_post = dev.upload(plain) if len(plain) else None
+            self.d_post_export, self.d_export = dev.upload(t.post[t.export_of]), dev.upload(t.export)
+            self.d_bank = dev.upload(t.bank.astype(real))
+            self.max_n_export = int(t.post["n"][t.export_of].max())
+            self.max_out_export = int((t.export["out_end"] - t.export["out"]).max())
+        else:
+            self.d_post = dev.upload(t.post)
         if self.any_dust:
             self.d_dpos, self.d_dval = dev.upload(t.dust_pos), dev.upload(t.dust_val.astype(real))
         _mark("uploads")
@@ -458,8 +472,16 @@ class BatchRenderer:
             for (y_at, scratch, n, dr) in self.tables.odd.tolist():
                 _check(dev, lib.ms_roll(C.c_void_p(base + isz * y_at), C.c_void_p(base + isz * scratch), n, dr, st))
             self.rot_stage.run()
-        _check(dev, lib.ms_post(dev.ptr(self.d_post), self.n_renders, self.max_out_n, dev.ptr(self.mono),
-                                dev.ptr(self.maxbits), dev.ptr(self.out), st))
+        if not self.n_export:
+            _check(dev, lib.ms_post(dev.ptr(self.d_post), self.n_renders, self.max_out_n, dev.ptr(self.mono),
+                                    dev.ptr(self.maxbits), dev.ptr(self.out), st))
+        else:
+            if self.n_plain:
+                _check(dev, lib.ms_post(dev.ptr(self.d_post), self.n_plain, self.max_n_plain, dev.ptr(self.mono),
+                                        dev.ptr(self.maxbits), dev.ptr(self.out), st))
+            mb = C.c_void_p(dev.ptr(self.maxbits).value + 8 * self.n_plain)
+            _check(dev, lib.ms_post_export(dev.ptr(self.d_post_export), dev.ptr(self.d_export), self.n_export, self.max_n_export,
+                                           self.max_out_export, dev.ptr(self.mono), mb, dev.ptr(self.d_bank), dev.ptr(self.out), st))
         mark("post")
 
     # ---- CUDA graph ------------------------------------------------------------------------------------
@@ -491,7 +513,7 @@ class BatchRenderer:
 
     # ---- results ---------------------------------------------------------------------------------------
     def output(self, r):
-        """float32 [out_n, 2] of render r (host copy)."""
+        """float32 [out_n, 2] of render r (host copy; out_n frames at its export rate, if any)."""
         n = int(self.tables.out_n[r])
         return self.dev.download(self.out, 2 * int(self.tables.out_at[r]), 2 * n).reshape(n, 2)
 
@@ -509,6 +531,10 @@ class BatchRenderer:
     def meta(self, r):
         t = self.tables
         m = dict(out_sr=int(t.srs[r, 0]), design_sr_base=int(t.srs[r, 1]), micro_last=None, grain_last=None)
+        at = np.flatnonzero(t.export_of == r)
+        if at.size:                                  # export_sr = base_sr * up / down, exactly
+            up, down = t.export["rate"][at[0], :2].tolist()
+            m["out_sr"] = m["out_sr"] * up // down
         micro, grain, n = t.last[r].tolist()
         if n > 0:
             m["micro_last"] = np.asarray(self.dev.download(self.pool, micro, n)).astype(np.float64)
@@ -678,15 +704,16 @@ def _render_batch(params_list, device=None, precision="auto", host_out=None, chu
             br.close()
         return outs
     torch = dev.torch
-    # frames of the whole batch (main_v2.py:590), memoised per distinct (duration, rate): a sweep repeats a few values
+    # frames of the whole batch (main_v2.py:590; at the export rate of renders with `export_sr`), memoised per distinct
+    # (duration, rate, export rate): a sweep repeats a few values
     import operator
     frames_of, get_dur = {}, operator.itemgetter("out_dur_s", "base_sr")
     total = 0
     for p in params_list:
-        key = get_dur(p)
+        key = get_dur(p) + (p.get("export_sr"),)
         f = frames_of.get(key)
         if f is None:
-            f = frames_of[key] = int(max(1, round(float(key[0]) * int(key[1]))))
+            f = frames_of[key] = P.export_frames(int(max(1, round(float(key[0]) * int(key[1])))), P.export_ratio(p))
         total += f
     if host_out is None:
         host_out = torch.empty(2 * total, dtype=torch.float32).pin_memory()

@@ -17,6 +17,7 @@ import struct
 import numpy as np
 
 from .configs import FACTORY_DEFAULTS
+from .plan import export_ratio
 
 
 def load_preset(source, ir_audio=None, img_gray=None):
@@ -136,6 +137,7 @@ def write_wav_float32(path, audio, sample_rate):
 
 def batch_render(base_params, seeds, unfolds, stretches, folder, device=None, precision="auto", progress=None):
     """The batch dialog's sweep (main_v2.py:1524-1593) through the streamed GPU batch: returns [(reference name, path)].
+    With `export_sr` in the parameters the files are written, and named, at that rate.
     `progress(done, total, name)` mirrors the dialog's progress bar / status line."""
     from . import engine
     plist = batch_params(base_params, seeds, unfolds, stretches)
@@ -143,9 +145,10 @@ def batch_render(base_params, seeds, unfolds, stretches, folder, device=None, pr
     outs = engine.render_batch(plist, device=device, precision=precision)
     written, total = [], max(1, len(plist))
     for i, (p, audio) in enumerate(zip(plist, outs)):
-        name = batch_name(p["seed"], p["time_unfold"], p["partial_stretch"], int(p["base_sr"]))
+        out_sr = int(p["base_sr"]) if export_ratio(p) is None else int(p["export_sr"])      # the optional key `export_sr`
+        name = batch_name(p["seed"], p["time_unfold"], p["partial_stretch"], out_sr)
         path = os.path.join(folder, name + ".wav")
-        write_wav_float32(path, audio, int(p["base_sr"]))
+        write_wav_float32(path, audio, out_sr)
         written.append((name, path))
         if progress:
             progress(i + 1, total, name)

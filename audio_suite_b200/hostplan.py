@@ -13,7 +13,7 @@ import os
 
 import numpy as np
 
-from . import _abi, plan as P
+from . import _abi, decimate, plan as P
 from .configs import BASIC_MODES
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -24,11 +24,11 @@ FIELDS = ("base_sr", "out_dur_s", "time_unfold", "peak", "sat_drive", "stereo_on
           "mb_b1", "mb_b2", "mb_b3", "mb_u1", "mb_u2", "mb_u3", "mb_roll", "bandlimit_on", "bandlimit_out_hz", "bandlimit_roll_hz",
           "event_process", "grains_per_sec", "max_grains", "grain_amp_rand", "grain_offset_on", "grain_offset_max_ms",
           "bp_density", "bp_unfold", "bp_cutoff", "bp_stretch", "er_cloud_on", "er_taps", "er_max_ms", "space_ir_on", "_ir",
-          "_ir_r", "env_a", "env_d", "env_s", "env_r", "env_curve", "_bessel")
+          "_ir_r", "env_a", "env_d", "env_s", "env_r", "env_curve", "_bessel", "export_sr")
 _MODE = {m: float(i) for i, m in enumerate(BASIC_MODES)}
 _PROCESS = {"Single": 0.0, "Poisson": 1.0}
 _OFF_FLAGS = ("partial_lock_on", "cep_warp_on", "res_bank_on", "wg_on", "event_feedback_on", "spectral_imprint_on")
-_HP_NAMES = ("sy1", "ola_r", "env_reps", "ola_e", "fir", "post", "tap_off", "dust_pos", "tilt", "grain", "rot", "odd", "irs")   # ms_hp_sizes
+_HP_NAMES = ("sy1", "ola_r", "env_reps", "ola_e", "fir", "post", "tap_off", "dust_pos", "tilt", "grain", "rot", "odd", "irs", "export", "ratios")   # ms_hp_sizes
 
 _lib = None
 
@@ -47,7 +47,7 @@ def lib():
             l.ms_hp_error.restype = C.c_char_p
             l.ms_hp_error.argtypes = [C.c_void_p, C.POINTER(C.c_int)]
             l.ms_hp_sizes.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
-            l.ms_hp_export.argtypes = [C.c_void_p] * 23
+            l.ms_hp_export.argtypes = [C.c_void_p] * 26
             l.ms_hp_free.argtypes = [C.c_void_p]
             l.ms_hp_pcg64_seed.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
             l.ms_hp_draws.argtypes = [C.c_int64, C.c_int, C.c_uint64, C.c_int, C.c_void_p]
@@ -158,6 +158,9 @@ def _marshal(params_list):
         stereo = p.get("space_ir_stereo", False)
         if stereo.__class__ is not bool:
             stereo = P.ir_stereo(p)
+        ex = p.get("export_sr")                                  # optional key, 0 = none (also when equal to base_sr)
+        if ex is not None:
+            rows[r, _EXPORT_COL] = 0.0 if P.export_ratio(p) is None else float(ex)
         key = gs(p) + (cap, stereo, id(ir), id(dig), widths[r])
         k = uniq_of.get(key)
         if k is None:
@@ -195,6 +198,7 @@ def _marshal(params_list):
     return rows, lane_ptr, lane_t, lane_v, irs, ir_len, btab
 
 
+_EXPORT_COL = FIELDS.index("export_sr")
 _SIDE_COL = [FIELDS.index(k) for k in ("gen_mode", "unfold_mode", "event_process", "bp_density", "bp_unfold", "bp_cutoff", "bp_stretch", "_ir", "_ir_r", "_bessel")]
 
 
@@ -235,14 +239,17 @@ def plan_chunk(params_list, threads=1):
         delay, raw, ir_order = np.zeros(n["tap_off"]), np.zeros(n["tap_off"]), np.zeros(n["irs"], np.int64)
         t.out_at, t.out_n, t.y_at = np.zeros(R, np.int64), np.zeros(R, np.int64), np.zeros(R, np.int64)
         t.last, t.srs = np.zeros(R, T.LAST), np.zeros((R, 2), np.int64)
+        t.export, t.export_of, ratios = np.zeros(n["export"], t.export.dtype), np.zeros(n["export"], np.int64), np.zeros((n["ratios"], 2), np.int64)
         args = [t.sy1, t.sy2, t.ola_r, t.env_reps, t.ola_e, t.fir, t.post, t.tap_off, delay, raw, t.dust_pos, t.dust_val,
-                t.tilt, t.grain, t.rot, t.odd, ir_order, t.out_at, t.out_n, t.y_at, t.last, t.srs]
+                t.tilt, t.grain, t.rot, t.odd, ir_order, t.out_at, t.out_n, t.y_at, t.last, t.srs, t.export, t.export_of, ratios]
         l.ms_hp_export(h, *[a.ctypes.data for a in args])
     finally:
         l.ms_hp_free(h)
     # gains *= exp(-delays * 42) (main_v2.py:415) with numpy's own exp, as the reference computes it
     t.tap_gain = raw * np.exp(-delay * 42.0)
     t.irs = np.concatenate([np.ones(1) if k == -2 else irs[k] for k in ir_order.tolist()]).astype(np.float64) if n["irs"] else np.zeros(0)
+    if len(ratios):                       # the banks are designed in numpy, as the Python planner does (bit-identical pools)
+        t.bank = np.concatenate([decimate.polyphase_bank(u, d)[2].reshape(-1) for u, d in ratios.tolist()])
     t.pool_n, t.mono_n, t.frames, t.h_total, t.max_h, t.max_out_n, t.env_n = (int(v) for v in sc[:7])
     t.alg = dict(zip(("synth", "tilt_spectral", "grain_spectral", "overlap_add", "fir_in", "fir_taps", "post"), (int(v) for v in sc[7:])))
     return t

@@ -22,6 +22,7 @@ from .configs import BASIC_MODES
 DESIGN_SR_CAP = 30_000_000          # M:597, M:646
 IR_TAP_CAP = 8192                   # M:443: default of the optional key `space_ir_tap_cap`
 IR_TAP_LIMIT = 1 << 21              # most IR taps the FIR stage takes (ms_fir_*: 10 s at 192 kHz)
+EXPORT_RATIO_LIMIT = 640            # largest up or down of `export_sr` / base_sr in lowest terms (filter of 12801 taps)
 
 MODE_GAUSS, MODE_DUST, MODE_NOISE, MODE_SKEW, MODE_RES, MODE_PLAIN, MODE_WAVELET, MODE_IRFRAG, MODE_SCANLINE, MODE_SILENT, MODE_CHAOS, MODE_STICK = range(12)
 WAVELET_FLOOR = 128                 # M:319
@@ -264,6 +265,7 @@ class RenderPlan:
     stereo_theta: float = 0.0
     drive: float = 1.0
     peak: float = 0.98
+    export: Optional[tuple] = None          # (up, down) of the optional key `export_sr`, or None: delivered at base_sr
     progress_msgs: list = field(default_factory=list)
 
 
@@ -288,6 +290,7 @@ def plan_render(params) -> RenderPlan:
     check_supported(params)
     cap = ir_tap_cap(params)
     stereo_ir = ir_stereo(params)
+    export = export_ratio(params)
     base_sr = int(params["base_sr"])
     out_dur = float(params["out_dur_s"])
     out_n = int(max(1, round(out_dur * base_sr)))
@@ -451,6 +454,7 @@ def plan_render(params) -> RenderPlan:
         rp.stereo_theta = w * 0.9
     rp.drive = float(params["sat_drive"])
     rp.peak = float(params["peak"])
+    rp.export = export
     return rp
 
 
@@ -488,6 +492,32 @@ def ir_stereo(params):
     if not isinstance(on, (bool, np.bool_)):
         raise ValueError(f"space_ir_stereo must be a bool, not {on!r}")
     return bool(on)
+
+
+def export_ratio(params):
+    """The optional key `export_sr` (EXTENSION; the reference delivers every render at base_sr): the rate the output is
+    resampled to after the normalisation, as scipy.signal.resample_poly(x, up, down) does it.  Returns (up, down) in
+    lowest terms, or None when the key is absent, None or equal to int(base_sr).  Only an int >= 1 (numpy's included, not
+    a bool) is taken, with up and down at most EXPORT_RATIO_LIMIT."""
+    sr = params.get("export_sr", None)
+    if sr is None:
+        return None
+    if isinstance(sr, (bool, np.bool_)) or not isinstance(sr, (int, np.integer)) or sr < 1:
+        raise ValueError(f"export_sr must be an int >= 1 or None, not {sr!r}")
+    base, sr = int(params["base_sr"]), int(sr)
+    if sr == base:
+        return None
+    g = math.gcd(base, sr)
+    up, down = sr // g, base // g
+    if max(up, down) > EXPORT_RATIO_LIMIT:
+        raise ValueError(f"export_sr {sr} from base_sr {base} is the ratio {up}/{down}: up and down must be at most "
+                         f"{EXPORT_RATIO_LIMIT}")
+    return up, down
+
+
+def export_frames(n, ratio):
+    """Frames of a render of n frames at base_sr after the export resampler: ceil(n up / down)."""
+    return n if ratio is None else -(-n * ratio[0] // ratio[1])
 
 
 _PAIR_CACHE = {}

@@ -11,8 +11,9 @@ Every table is a record array with the layout of its struct in include/microsoun
 workspace can supply (the `z*` spectrum offsets, scratch offsets) stay 0 here and are filled on upload.
 
 Buffers (offsets in elements): pool (real; per-event signals), mono (real; per chunk:
-[OLA plane | FIR plane | right channels / odd-length scratch / right-channel FIR outputs]), out (float32 frames), hpool (real;
-combined FIR taps), taps (reflection delays/gains), irs (deduplicated IR taps), dust (impulses).
+[OLA plane | FIR plane | right channels / odd-length scratch / right-channel FIR outputs]), out (float32 frames, at the
+export rate of renders with `export_sr`), hpool (real; combined FIR taps), taps (reflection delays/gains), irs
+(deduplicated IR taps), dust (impulses), bank (polyphase banks of the export resampler, one per ratio and chunk).
 """
 from __future__ import annotations
 
@@ -22,7 +23,7 @@ from dataclasses import dataclass, field, fields
 
 import numpy as np
 
-from . import _abi, plan as P
+from . import _abi, decimate, plan as P
 
 _SPEC_OP_BYTES = np.dtype(_abi.SpecOp).itemsize
 _SPEC_JOB = np.dtype(_abi.SpecJob)
@@ -119,6 +120,9 @@ class Tables:
     grain: np.ndarray = _empty(SPEC_ITEM)
     rot: np.ndarray = _empty(SPEC_ITEM)
     odd: np.ndarray = _empty(ODD)
+    export: np.ndarray = _empty(_abi.ExportRender)   # renders with an export rate, in render order ...
+    export_of: np.ndarray = _empty(np.int64)         # ... and their render indices
+    bank: np.ndarray = _empty(np.float64)            # polyphase banks of the export resampler (decimate.polyphase_bank)
     pool_n: int = 0
     mono_n: int = 0
     frames: int = 0
@@ -126,7 +130,7 @@ class Tables:
     max_h: int = 0
     max_out_n: int = 0
     out_at: np.ndarray = _empty(np.int64)            # per render: first frame
-    out_n: np.ndarray = _empty(np.int64)
+    out_n: np.ndarray = _empty(np.int64)             # per render: frames (at the export rate, if any)
     y_at: np.ndarray = _empty(np.int64)
     last: np.ndarray = _empty(LAST)
     srs: np.ndarray = _empty(np.int64, 2)            # per render: base_sr, design_sr_base
@@ -151,6 +155,8 @@ RELOC = {
     ("imprint_r", "ev_begin"): ("imprint", False), ("imprint_r", "ev_end"): ("imprint", False),
     ("odd", "y_at"): ("mono", False), ("odd", "scratch"): ("mono", False),
     ("out_at", None): ("frames", False), ("y_at", None): ("mono", False),
+    ("export", "out"): ("frames", False), ("export", "out_end"): ("frames", False),
+    ("export", "bank"): ("bank", False), ("export", "bank_end"): ("bank", False), ("export_of", None): ("renders", False),
     ("last", "micro"): ("pool", True), ("last", "grain"): ("pool", True),
 }
 for _t, _buf in (("tilt", "pool"), ("grain", "pool"), ("post_grain", "pool"), ("cep_items", "pool"), ("plock_items", "pool"),
@@ -163,6 +169,7 @@ BUFFERS = {
     "env": lambda t: t.env_n, "ola_e": lambda t: len(t.ola_e), "taps": lambda t: len(t.tap_off), "irs": lambda t: len(t.irs),
     "dust": lambda t: len(t.dust_pos), "atoms": lambda t: len(t.atom_shift), "res_modes": lambda t: len(t.res_modes),
     "wg_lines": lambda t: len(t.wg_lines), "imprint": lambda t: len(t.imprint), "renders": lambda t: len(t.post),
+    "bank": lambda t: len(t.bank),
 }
 
 
@@ -389,6 +396,7 @@ def pack_chunk(plans) -> Tables:
     frames = 0
     odd = []
     out_at, out_n, y_at = np.zeros(R, np.int64), np.zeros(R, np.int64), np.zeros(R, np.int64)
+    export, export_of, banks, bank_at, n_bank = [], [], [], {}, 0
     fir_arr = np.array(fir, np.dtype(_abi.FirRender))
     for r, rp in enumerate(plans):
         n = rp.out_n
@@ -430,8 +438,18 @@ def pack_chunk(plans) -> Tables:
                 rot.append((n, 2 * plane + extra, 2 * plane + extra + n, op))
                 extra += 2 * n
         post[r] = (y, frames, rbuf, n, mode, dl, dr, rp.drive, 1.0 / math.tanh(rp.drive) if rp.drive > 0 else 1.0, rp.peak, coef)
-        out_at[r], out_n[r], y_at[r] = frames, n, y
-        frames += n
+        n_x = P.export_frames(n, rp.export)
+        if rp.export is not None:                # export_sr: the output is resampled by up / down through the ratio's bank
+            half, taps, bk = decimate.polyphase_bank(*rp.export)
+            at = bank_at.get(rp.export)
+            if at is None:
+                at = bank_at[rp.export] = n_bank
+                banks.append(bk.reshape(-1))
+                n_bank += bk.size
+            export.append((frames, frames + n_x, at, at + bk.size, rp.export + (half, taps)))
+            export_of.append(r)
+        out_at[r], out_n[r], y_at[r] = frames, n_x, y
+        frames += n_x
         alg["post"] += n
     # envelopes shared by several renders are tabulated once (ms_adsr_tables) instead of one pow() per sample
     env_n = 0
@@ -464,6 +482,9 @@ def pack_chunk(plans) -> Tables:
     t.imprint, t.imprint_items, t.imprint_r = _structs(_abi.ImprintEvt, imprint), spec_items(imprint_items), _structs(_abi.ImprintRender, imprint_r)
     t.tilt, t.grain, t.rot, t.post_grain = spec_items(tilt), spec_items(grain), spec_items(rot), spec_items(post_grain)
     t.odd = np.array(odd, ODD)
+    if export:
+        t.export, t.export_of = np.array(export, t.export.dtype), np.array(export_of, np.int64)
+        t.bank = np.concatenate(banks)
     t.pool_n, t.mono_n, t.frames, t.h_total, t.max_h = pool_n, 2 * plane + extra, frames, h_total, max_h
     t.max_out_n = max((rp.out_n for rp in plans), default=0)
     t.out_at, t.out_n, t.y_at, t.last = out_at, out_n, y_at, last

@@ -246,6 +246,23 @@ typedef struct {
 } ms_post_render;
 /* ms_post_f32 / ms_post_f64: declared below by MS_DECLARE_API */
 /* ms_roll_f32 / ms_roll_f64: declared below by MS_DECLARE_API */
+/* EXTENSION (the reference delivers every render at base_sr): an export sample rate.  ms_post_export runs the max pass of
+ * ms_post (the same kernel) on the renders of `dev_renders`, then, instead of its write pass, resamples each channel of the
+ * clipped and normalised signal x = soft_clip(.) * scale, in the working precision, by up / down as
+ * scipy.signal.resample_poly(x, up, down) defines it:
+ *     out[m] = sum_j x[j] g[m down - j up + half],  0 <= m < ceil(n up / down),
+ * g = up * firwin(2 half + 1, 1 / max(up, down), window=("kaiser", 5.0)), half = 10 max(up, down), g zero outside
+ * [0, 2 half].  The filter arrives as a polyphase bank: phase p = (m down) mod up holds `taps` = rate[3] coefficients,
+ * entry s + A of phase p being g[p + half - s up] (zero outside g) for s = -A .. taps - 1 - A, A = half / up; with
+ * q = (m down) div up, out[m] = sum_s x[q + s] bank[p][s + A].  The output is interleaved float32 stereo at `out`; there is
+ * no renormalisation after the resampler, so inter-sample peaks may exceed `peak`.  Row i of dev_export belongs to row i of
+ * dev_renders.  max_n: largest n, max_out_n: largest out_end - out.  Allocates nothing, never synchronises. */
+typedef struct {
+    int64_t out, out_end;     /* output frames [out, out_end) */
+    int64_t bank, bank_end;   /* the render's polyphase bank in the bank pool: up * taps coefficients */
+    int32_t rate[4];          /* up, down, half, taps per phase */
+} ms_export_render;
+/* ms_post_export_f32 / ms_post_export_f64: declared below by MS_DECLARE_API */
 
 /* ---- EXTENSION, not on the reference's path (SURVEY a14): band-limited polyphase decimation.  render() never decimates:
  *      the rate change is a relabel (main_v2.py:489-490), the band-limit is lowpass_fft (main_v2.py:39-59).  This stage
@@ -299,6 +316,8 @@ typedef struct {
     void ms_fir_destroy##SFX(void* handle); \
     int ms_post##SFX(const ms_post_render* dev_renders, int n_renders, int max_n, REAL* mono, uint64_t* maxbits, \
     float* out, void* stream); \
+    int ms_post_export##SFX(const ms_post_render* dev_renders, const ms_export_render* dev_export, int n_renders, int max_n, \
+    int max_out_n, REAL* mono, uint64_t* maxbits, const REAL* bank, float* out, void* stream); \
     int ms_roll##SFX(const REAL* src, REAL* dst, int n, int shift, void* stream); \
     int ms_polyphase_decimate##SFX(const REAL* x, int64_t x_stride, int n, int n_signals, const REAL* h, int taps, int q, \
     REAL* y, int64_t y_stride, void* stream);

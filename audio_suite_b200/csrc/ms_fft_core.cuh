@@ -208,12 +208,12 @@ MS_DEV cpx* tile_fft(cpx* a, cpx* b, const TileGeom& g, const RadixPlan& p, cons
 
 // (The generic passes stay ping-pong: run in place, a thread must hold ALL its butterflies of a pass in registers at
 //  once -- 8..10 double-complex values for the radix 4/5/3/2 passes -- and at the 64-register budget that spills:
-//  measured grain stage 17.2 -> 20.8 ms.  The static 256-point tiles are radix 8 (+ one radix-4 pass) and gain.)
-// ---- in-place pass (static 256 x 256 tiles) ---------------------------------------------------------
+//  measured grain stage 17.2 -> 20.8 ms.  The static power-of-two tiles are radix 8 (+ radix-4 passes) and gain.)
+// ---- in-place pass (static power-of-two tiles) ------------------------------------------------------
 // In place: every thread pulls the inputs of its (at most BPT) butterflies into registers and transforms them, the
 // CTA synchronises, then the results go back into the SAME buffer at the autosort positions.  Two barriers per
 // pass, ONE tile buffer: half the shared memory of a ping-pong Stockham, i.e. more CTAs per SM, which is what these
-// latency-bound passes need (measured on the FIR stage: 19.2 -> 15.3 ms).  tw = table of w_F^i (i < F), forward
+// latency-bound passes need (measured on 256 x 256 FIR-stage tiles: 19.2 -> 15.3 ms).  tw = table of w_F^i (i < F), forward
 // sign.  Integer divisions by the per-pass constants go through host-computed magic multipliers.
 template <int R, int CM, int BPT>
 MS_DEV void stockham_pass_ip(cpx* MS_RESTRICT buf, const TileGeom& g, int per_vec, int Ns, int tws,
@@ -268,27 +268,20 @@ MS_DEV void stockham_pass_ip(cpx* MS_RESTRICT buf, const TileGeom& g, int per_ve
     }
     c.sync();
 }
-// Static 256-point transform (radices 8, 8, 4) with literal geometry, so the magic divisions, strides and padded
-// addresses fold into immediates.  Used by the 256 x 256 (65536-point) transforms of the FIR stage, whose tiles are
-// always full: CNT vectors, CNT * 32 threads.
+// Literal geometry: the magic divisions, strides and padded addresses fold into immediates.
 template <unsigned D> struct MsMagic { static constexpr unsigned v = D <= 1 ? 0u : (unsigned)(0x100000000ull / (D ? D : 1)) + 1u; };
 #define ms_magic_c(D) (MsMagic<(D)>::v)
 // Static power-of-two transforms of CNT vectors of length F, F * CNT elements = 8 per thread (CNT * F / 8 threads),
-// in place: 128 = 8.4.4, 256 = 8.8.4, 512 = 8.8.8, 1024 = 8.8.4.4.  Used by the in-tile Bluestein columns.
+// in place: 128 = 8.4.4, 1024 = 8.8.4.4.  Used by the block-wide in-tile Bluestein columns (B1 = 256 and 512 are warp-local).
 template <int CM, int F, int CNT>
 MS_DEV cpx* tile_fft_pow2(cpx* a, const TileGeom& g, const cpx* MS_RESTRICT tw, const Ctx& c) {
+    static_assert(F == 128 || F == 1024, "static in-place tiles: 128 or 1024 points");
     constexpr unsigned mc = ms_magic_c(CNT);
     constexpr int P = F / 8;
     stockham_pass_ip<8, CM, 1>(a, g, P, 1, P, ms_magic_c(1), ms_magic_c(P), mc, tw, c);
     if (F == 128) {
         stockham_pass_ip<4, CM, 2>(a, g, 32, 8, 4, ms_magic_c(8), ms_magic_c(32), mc, tw, c);
         stockham_pass_ip<4, CM, 2>(a, g, 32, 32, 1, ms_magic_c(32), ms_magic_c(32), mc, tw, c);
-    } else if (F == 256) {
-        stockham_pass_ip<8, CM, 1>(a, g, 32, 8, 4, ms_magic_c(8), ms_magic_c(32), mc, tw, c);
-        stockham_pass_ip<4, CM, 2>(a, g, 64, 64, 1, ms_magic_c(64), ms_magic_c(64), mc, tw, c);
-    } else if (F == 512) {
-        stockham_pass_ip<8, CM, 1>(a, g, 64, 8, 8, ms_magic_c(8), ms_magic_c(64), mc, tw, c);
-        stockham_pass_ip<8, CM, 1>(a, g, 64, 64, 1, ms_magic_c(64), ms_magic_c(64), mc, tw, c);
     } else {        // 1024
         stockham_pass_ip<8, CM, 1>(a, g, 128, 8, 16, ms_magic_c(8), ms_magic_c(128), mc, tw, c);
         stockham_pass_ip<4, CM, 2>(a, g, 256, 64, 4, ms_magic_c(64), ms_magic_c(256), mc, tw, c);
@@ -296,15 +289,6 @@ MS_DEV cpx* tile_fft_pow2(cpx* a, const TileGeom& g, const cpx* MS_RESTRICT tw, 
     }
     return a;
 }
-template <int CM, int CNT>
-MS_DEV cpx* tile_fft_256(cpx* a, const TileGeom& g, const cpx* MS_RESTRICT tw, const Ctx& c) {
-    constexpr unsigned mc = ms_magic_c(CNT);
-    stockham_pass_ip<8, CM, 1>(a, g, 32, 1, 32, ms_magic_c(1), ms_magic_c(32), mc, tw, c);
-    stockham_pass_ip<8, CM, 1>(a, g, 32, 8, 4, ms_magic_c(8), ms_magic_c(32), mc, tw, c);
-    stockham_pass_ip<4, CM, 2>(a, g, 64, 64, 1, ms_magic_c(64), ms_magic_c(64), mc, tw, c);
-    return a;
-}
-
 // ---- warp-local 256-point forward FFT ---------------------------------------------------------------------
 // in: v[q] = x[lane + 32 q];  out: v[m] = X[lane + 32 m].  sw: the warp's shared-memory row (FF_RS entries).
 // The caller guarantees that nobody else touches sw and that the warp is converged.

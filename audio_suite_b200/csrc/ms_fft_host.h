@@ -10,16 +10,13 @@ static const int MS_TILE_MAX = sizeof(real) == 4 ? 8192 : 4096;
 #ifndef MS_FFT_MINB
 #define MS_FFT_MINB 2
 #endif
-#ifndef MS_SQ_MINB
-#define MS_SQ_MINB 5
-#endif
 #ifndef MS_SB_MINB
 #define MS_SB_MINB 5
 #endif
-template <int LD, int ST, int TWID, int SQ = 0, int SB = 0> struct ColsK {
-    static constexpr int MAXT = ((SQ && sizeof(real) == 8) || SB) ? 256 : 512;      // static tiles: 2048 elements, 256 threads
-    static constexpr int MINB = SB ? MS_SB_MINB : (SQ && sizeof(real) == 8) ? MS_SQ_MINB : MS_FFT_MINB;   // 2 x 512: <= 64 registers
-    static MS_DEV void run(const FftJob* jobs, const Ctx& c) { fft_cols_body<LD, ST, TWID, SQ, SB>(jobs, c); }
+template <int LD, int ST, int TWID, int SB = 0> struct ColsK {
+    static constexpr int MAXT = SB ? 256 : 512;      // static tiles: 2048 elements, 256 threads
+    static constexpr int MINB = SB ? MS_SB_MINB : MS_FFT_MINB;   // 2 x 512: <= 64 registers
+    static MS_DEV void run(const FftJob* jobs, const Ctx& c) { fft_cols_body<LD, ST, TWID, SB>(jobs, c); }
 };
 #ifndef MS_WB_MINB
 #define MS_WB_MINB 4
@@ -42,10 +39,10 @@ template <int LD, int ST, int TWID> struct ColsWarp512K {           // in-tile B
     static constexpr int MINB = MS_WB5_MINB;
     static MS_DEV void run(const FftJob* jobs, const Ctx& c) { fft_cols_warp512_body<LD, ST, TWID>(jobs, c); }
 };
-template <int LD, int MODE, int ST, int SQ = 0> struct RowsK {
-    static constexpr int MAXT = (SQ && sizeof(real) == 8) ? 256 : 512;
-    static constexpr int MINB = (SQ && sizeof(real) == 8) ? MS_SQ_MINB : MS_FFT_MINB;
-    static MS_DEV void run(const FftJob* jobs, const Ctx& c) { fft_rows_body<LD, MODE, ST, SQ>(jobs, c); }
+template <int LD, int MODE, int ST> struct RowsK {
+    static constexpr int MAXT = 512;
+    static constexpr int MINB = MS_FFT_MINB;
+    static MS_DEV void run(const FftJob* jobs, const Ctx& c) { fft_rows_body<LD, MODE, ST>(jobs, c); }
 };
 #ifndef MS_SPECOP_MINB
 #define MS_SPECOP_MINB 6          // 40 registers (the cold operator branches spill): 1.98 -> 1.62 ms over the sweep; 7 and 8 were slower
@@ -55,8 +52,6 @@ struct SpecOpK {                                                    // spectral 
     static constexpr int MINB = MS_SPECOP_MINB;
     static MS_DEV void run(const FftJob* jobs, const Ctx& c) { spec_op_body(jobs, c); }
 };
-// tile width of the static 256 x 256 kernels: what plan_direct picks for 65536 points in this precision
-static const int MS_SQ = (sizeof(real) == 4 ? 8192 : 4096) / 2 / 256;
 struct GenChirpK {
     static constexpr int MAXT = 256;
     static constexpr int MINB = 1;
@@ -193,17 +188,8 @@ private:
     // Per-element cost of the in-tile Bluestein columns by convolution length (<= 128, 256, 512, 1024) and of one radix-2
     // level of the rows pass, relative to the warp-local 256 kernel.  Measured on B200 (C5 sweep, f64, per padded element):
     // 128: 1.4, 256: 1.0, 512 (warp-local): 1.45, 1024 (block-wide tile): 2.45 -- so a longer convolution has to buy a much
-    // better padding ratio to be chosen (step 31.2 -> 30.8 ms against the analytic cost).  Development switch
-    // MS_PLAN_W="c128,c256,c512,c1024,rows" overrides; MS_PLAN_W=0 selects the analytic cost.
-    static const double* mixed_weights() {
-        static double w[5] = {1.4, 1.0, 1.45, 2.45, 0.02}; static int init = 0;
-        if (!init) {
-            init = 1;
-            const char* e = getenv("MS_PLAN_W");
-            if (e && sscanf(e, "%lf,%lf,%lf,%lf,%lf", &w[0], &w[1], &w[2], &w[3], &w[4]) != 5) w[0] = -1;
-        }
-        return w;
-    }
+    // better padding ratio to be chosen (step 31.2 -> 30.8 ms against an analytic cost in passes per element).
+    static constexpr double MIXED_W[5] = {1.4, 1.0, 1.45, 2.45, 0.02};
     static bool plan_direct(int n, FftJob& J) {
         if (!ms_is_smooth(n)) return false;
         J.M = n;
@@ -220,7 +206,7 @@ private:
         if (!best) return false;
         J.F1 = best; J.F2 = n / best;
         J.T = 16; J.G = 16;
-        // smooth n with 256 | n (not a power of two: those belong to the FIR stage's static kernels): columns of exactly 256
+        // smooth n with 256 | n (not a power of two: those keep the generic tile): columns of exactly 256
         // rows run as one warp-local transform each -- a third of the generic tile's cost per element
         if ((n & (n - 1)) && n % 256 == 0 && n / 256 >= 16 && n / 256 <= MS_TILE_MAX / 4) {
             J.F1 = 256; J.F2 = n / 256; J.T = 8;
@@ -246,16 +232,12 @@ private:
             const int b1 = ms_conv_len(2 * f1 - 1);
             if (b1 * 4 > MS_TILE_MAX) continue;
             const int T = std::max(1, std::min(16, tile_target / b1)), G = std::max(1, std::min(16, tile_target / f2));
-            double lg2 = 0, lgb = 0;
+            double lg2 = 0;
             for (int t = f2; t > 1; t >>= 1) lg2 += 1;
-            for (int t = b1; t > 1; t >>= 1) lgb += 1;
-            double cost = lg2 + 2.0 * lgb * (double)b1 / (double)f1 + (T < 8 ? 16.0 / T : 0) + (G < 8 ? 16.0 / G : 0);
-            if (mixed_weights()[0] > 0) {
-                // measured form: padded elements per useful one times the per-element cost of that columns kernel
-                const double* w = mixed_weights();
-                const double cb = b1 <= 128 ? w[0] : b1 == 256 ? w[1] : b1 == 512 ? w[2] : b1 == 1024 ? w[3] : w[3] * (double)b1 / 1024.0;
-                cost = w[4] * lg2 + cb * (double)b1 / (double)f1 + (T < 8 ? 16.0 / T : 0) + (G < 8 ? 16.0 / G : 0);
-            }
+            // padded elements per useful one times the per-element cost of that columns kernel
+            const double* w = MIXED_W;
+            const double cb = b1 <= 128 ? w[0] : b1 == 256 ? w[1] : b1 == 512 ? w[2] : b1 == 1024 ? w[3] : w[3] * (double)b1 / 1024.0;
+            const double cost = w[4] * lg2 + cb * (double)b1 / (double)f1 + (T < 8 ? 16.0 / T : 0) + (G < 8 ? 16.0 / G : 0);
             if (!best || cost < best_cost) { best = f2; best_cost = cost; }
         }
         if (!best) return false;
@@ -349,48 +331,25 @@ private:
         return 0;
     }
 
-    template <int LD, int ST, int TWID, int SQ = 0>
+    template <int LD, int ST, int TWID>
     static int launch_cols(int ept, unsigned gx, unsigned gy, int nthr, size_t smem, ms_stream_t st, const FftJob* jd) {
-        return L<ColsK<LD, ST, TWID, SQ>>(gx, gy, nthr, smem, st, jd);
+        return L<ColsK<LD, ST, TWID>>(gx, gy, nthr, smem, st, jd);
     }
     // in-tile Bluestein columns with static convolution length (sb = sb_id): 256 threads, one tile buffer
     template <int LD, int ST, int TWID>
     static int launch_cols_sb(int sb, unsigned gx, unsigned gy, ms_stream_t st, const FftJob* jd) {
         const size_t smem = MS_JOB_SMEM + sizeof(cpx) * (size_t)(MS_SB_TILE + MS_SB_TILE / 8 + 4);
         switch (sb) {
-            case 1: return L<ColsK<LD, ST, TWID, 0, 128>>(gx, gy, 256, smem, st, jd);
-            case 2:
-                if (sb_warp()) return L<ColsWarpK<LD, ST, TWID>>(gx, gy, 256, MS_JOB_SMEM + sizeof(cpx) * (size_t)(8 * WB_RS), st, jd);
-                return L<ColsK<LD, ST, TWID, 0, 256>>(gx, gy, 256, smem, st, jd);
-            case 3:
-                if (sb_warp() && LdPlain<LD>::v) return L<ColsWarp512K<LD, ST, TWID>>((gx + 1) / 2, gy, 256, MS_JOB_SMEM + sizeof(cpx) * (size_t)(8 * WB5_RS), st, jd);
-                return L<ColsK<LD, ST, TWID, 0, 512>>(gx, gy, 256, smem, st, jd);
-            case 5:
-                if (LdPlain<LD>::v) return L<ColsWarpPlainK<LD, ST, TWID>>(gx, gy, 256, MS_JOB_SMEM + sizeof(cpx) * (size_t)(8 * WB_RS), st, jd);
-                return -1;
-            default: return L<ColsK<LD, ST, TWID, 0, 1024>>(gx, gy, 256, smem, st, jd);
+            case 1: return L<ColsK<LD, ST, TWID, 128>>(gx, gy, 256, smem, st, jd);
+            case 2: return L<ColsWarpK<LD, ST, TWID>>(gx, gy, 256, MS_JOB_SMEM + sizeof(cpx) * (size_t)(8 * WB_RS), st, jd);
+            case 3: return L<ColsWarp512K<LD, ST, TWID>>((gx + 1) / 2, gy, 256, MS_JOB_SMEM + sizeof(cpx) * (size_t)(8 * WB5_RS), st, jd);
+            case 5: return L<ColsWarpPlainK<LD, ST, TWID>>(gx, gy, 256, MS_JOB_SMEM + sizeof(cpx) * (size_t)(8 * WB_RS), st, jd);
+            default: return L<ColsK<LD, ST, TWID, 1024>>(gx, gy, 256, smem, st, jd);
         }
     }
-    // development switch MS_SPEC_PASS=0: the operators inside the load functor of the inverse columns (round 1 form)
-    static bool spec_pass() { static int v = -1; if (v < 0) { const char* e = getenv("MS_SPEC_PASS"); v = (e && e[0] == '0') ? 0 : 1; } return v != 0; }
-    // development switch MS_SB_WARP=0: the block-wide B1 = 256 kernel instead of the warp-local one
-    static bool sb_warp() { static int v = -1; if (v < 0) { const char* e = getenv("MS_SB_WARP"); v = (e && e[0] == '0') ? 0 : 1; } return v != 0; }
-    template <int LD, int MODE, int ST, int SQ = 0>
+    template <int LD, int MODE, int ST>
     static int launch_rows(int ept, unsigned gx, unsigned gy, int nthr, size_t smem, ms_stream_t st, const FftJob* jd) {
-        return L<RowsK<LD, MODE, ST, SQ>>(gx, gy, nthr, smem, st, jd);
-    }
-    // shared memory of the static kernels: the job + ONE tile (the static passes run in place)
-    static size_t sq_smem(bool cols) {
-        FftJob t; t.T = t.G = MS_SQ; t.F1 = t.F2 = 256; t.B1 = 0;
-        return MS_JOB_SMEM + ((cols ? cols_smem(t) : rows_smem(t)) - MS_JOB_SMEM) / 2;
-    }
-    // every job of [b, e) is a plain 256 x 256 transform with the static tile width: the FIR stage's 65536-point blocks
-    static bool all_square(const std::vector<FftJob>& jobs, size_t b, size_t e) {
-        for (size_t i = b; i < e; ++i) {
-            const FftJob& J = jobs[i];
-            if (J.F1 != 256 || J.F2 != 256 || J.T != MS_SQ || J.G != MS_SQ || J.B1 || J.ch_hi) return false;
-        }
-        return e > b;
+        return L<RowsK<LD, MODE, ST>>(gx, gy, nthr, smem, st, jd);
     }
 
     struct ClassShape { LaunchShape cols, rows; };
@@ -436,21 +395,12 @@ private:
                 else if (cls == 1) {
                     // (summing the few non-zero input rows of the tap vector directly in the rows kernel, instead of
                     //  the columns pass, was measured SLOWER on B200: 7.8 ms vs 2.95 + 3.79 ms for the C5 sweep)
-                    if (all_square(jobs, b, e)) {
-                        rc = launch_cols<LD_REALPAD, ST_WORK, 1, MS_SQ>(C.ept, C.gx, gy, C.nthr, sq_smem(true), st, jd);
-                        if (!rc) rc = launch_rows<LD_WORK, MODE_RAW, ST_HMUL, MS_SQ>(R.ept, R.gx, gy, R.nthr, sq_smem(false), st, jd);
-                    } else {
                     rc = launch_cols<LD_REALPAD, ST_WORK, 1>(C.ept, C.gx, gy, C.nthr, C.smem, st, jd);
                     if (!rc) rc = launch_rows<LD_WORK, MODE_RAW, ST_HMUL>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd);
-                    }
                 } else MS_FAIL("filter spectrum needs a direct length");
             } else if (what == 4) {
                 if (cls == 0) rc = launch_rows<LD_OLS, MODE_CONV, ST_OLS>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd);
-                else if (cls == 1 && all_square(jobs, b, e)) {
-                    rc = launch_cols<LD_OLS, ST_WORK, 1, MS_SQ>(C.ept, C.gx, gy, C.nthr, sq_smem(true), st, jd);
-                    if (!rc) rc = launch_rows<LD_WORK, MODE_CONV, ST_WORK, MS_SQ>(R.ept, R.gx, gy, R.nthr, sq_smem(false), st, jd);
-                    if (!rc) rc = launch_cols<LD_WORK, ST_OLS, 0, MS_SQ>(C.ept, C.gx, gy, C.nthr, sq_smem(true), st, jd);
-                } else if (cls == 1) {
+                else if (cls == 1) {
                     rc = launch_cols<LD_OLS, ST_WORK, 1>(C.ept, C.gx, gy, C.nthr, C.smem, st, jd);
                     if (!rc) rc = launch_rows<LD_WORK, MODE_CONV, ST_WORK>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd);
                     if (!rc) rc = launch_cols<LD_WORK, ST_OLS, 0>(C.ept, C.gx, gy, C.nthr, C.smem, st, jd);
@@ -478,7 +428,7 @@ private:
                     rc = sb ? launch_cols_sb<LD_PAIR, ST_WORK, 1>(sb, C.gx, gy, st, jd)
                             : launch_cols<LD_PAIR, ST_WORK, 1>(C.ept, C.gx, gy, C.nthr, C.smem, st, jd);
                     if (!rc) rc = launch_rows<LD_WORK, MODE_NAT, ST_Z>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd);
-                } else if (spec_pass()) {
+                } else {
                     // operators in their own elementwise pass (Z -> work), then the inverse in place in `work`: a columns
                     // tile reads exactly the positions it writes back
                     int nmax = 0;
@@ -487,10 +437,6 @@ private:
                     rc = L<SpecOpK>(gxo, gy, SPECOP_NTHR, MS_JOB_SMEM, st, jd);
                     if (!rc) rc = sb ? launch_cols_sb<LD_WORK, ST_WORK, 1>(sb, C.gx, gy, st, jd)
                                      : launch_cols<LD_WORK, ST_WORK, 1>(C.ept, C.gx, gy, C.nthr, C.smem, st, jd);
-                    if (!rc) rc = launch_rows<LD_WORK, MODE_NAT, ST_PAIR>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd);
-                } else {
-                    rc = (sb && sb != 5) ? launch_cols_sb<LD_SPEC, ST_WORK, 1>(sb, C.gx, gy, st, jd)
-                                         : launch_cols<LD_SPEC, ST_WORK, 1>(C.ept, C.gx, gy, C.nthr, C.smem, st, jd);
                     if (!rc) rc = launch_rows<LD_WORK, MODE_NAT, ST_PAIR>(R.ept, R.gx, gy, R.nthr, R.smem, st, jd);
                 }
             } else if (cls == 2) {

@@ -329,11 +329,11 @@ MS_DEV void spec_op_body(const FftJob* MS_RESTRICT jobs, const Ctx& c) {
 }
 
 // ---- columns kernel --------------------------------------------------------------------------------
-// SQ != 0: static geometry F1 = F2 = 256, T = G = SQ, plain mixed radix (the 65536-point transforms of the FIR stage)
 // SB != 0: in-tile Bluestein with static convolution length B1 = SB and T = MS_SB_TILE / SB full columns, in place
 #define MS_SB_TILE 2048
 template <int LD, int ST, int TWID, int SB>
 MS_DEV void fft_cols_bluestein_static(const FftJob& J, const Ctx& c) {
+    static_assert(!SB || LdPlain<LD>::v, "static Bluestein columns: plain loads only");   // (SB = 0: never called)
     constexpr int T = MS_SB_TILE / (SB ? SB : 1);
     const int F1 = J.F1, F2 = J.F2;
     const int col0 = c.bx * T;
@@ -341,27 +341,17 @@ MS_DEV void fft_cols_bluestein_static(const FftJob& J, const Ctx& c) {
     cpx* s = (cpx*)(c.smem + MS_JOB_SMEM);
     TileGeom g; g.cnt = T; g.vs = 1; g.es = T; g.colmajor = 1;
     constexpr int all = MS_SB_TILE;
-    if (LdPlain<LD>::v) {
-        for (int e0 = c.tid; e0 < all; e0 += 4 * c.nthr) {
-            cpx ld[4];
+    for (int e0 = c.tid; e0 < all; e0 += 4 * c.nthr) {
+        cpx ld[4];
 #pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int e = e0 + u * c.nthr, i = e / T, v = e - i * T;
-                ld[u] = (e < all && i < F1) ? job_load<LD>(J, i * F2 + col0 + v) : c_zero();
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int e = e0 + u * c.nthr, i = e / T, v = e - i * T;
-                if (e < all) s[tile_addr(g, v, i)] = i < F1 ? c_mul(ld[u], __ldg(&J.b1_chirp[i])) : c_zero();
-            }
+        for (int u = 0; u < 4; ++u) {
+            const int e = e0 + u * c.nthr, i = e / T, v = e - i * T;
+            ld[u] = (e < all && i < F1) ? job_load<LD>(J, i * F2 + col0 + v) : c_zero();
         }
-    } else {
-#pragma unroll 2
-        for (int e = c.tid; e < all; e += c.nthr) {
-            const int i = e / T, v = e - i * T;
-            cpx val = c_zero();
-            if (i < F1) val = c_mul(job_load<LD>(J, i * F2 + col0 + v), __ldg(&J.b1_chirp[i]));
-            s[tile_addr(g, v, i)] = val;
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int e = e0 + u * c.nthr, i = e / T, v = e - i * T;
+            if (e < all) s[tile_addr(g, v, i)] = i < F1 ? c_mul(ld[u], __ldg(&J.b1_chirp[i])) : c_zero();
         }
     }
     c.sync();
@@ -404,28 +394,18 @@ MS_DEV void fft_cols_bluestein_warp256(const FftJob& J, const Ctx& c) {
     if (col0 >= F2) return;
     cpx* s = (cpx*)(c.smem + MS_JOB_SMEM);
     const int lane = c.tid & 31, warp = c.tid >> 5;
-    // rows 0 .. 127 may hold data (F1 <= 128), rows 128 .. 255 are the zero padding of the convolution.  The load functor of
-    // the inverse (the whole spectral operator) is NOT unrolled: four inlined copies spill.
-    if (LD == LD_PAIR || LD == LD_WORK || LD == LD_CPX) {
-        cpx ld[4];                                              // plain loads: all in flight before the first store
+    // rows 0 .. 127 may hold data (F1 <= 128), rows 128 .. 255 are the zero padding of the convolution
+    static_assert(LdPlain<LD>::v, "warp-local Bluestein columns: plain loads only");
+    cpx ld[4];                                                  // all loads in flight before the first store
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int e = c.tid + 256 * i, row = e >> 3, v = e & 7;
-            ld[i] = row < F1 ? job_load<LD>(J, row * F2 + col0 + v) : c_zero();
-        }
+    for (int i = 0; i < 4; ++i) {
+        const int e = c.tid + 256 * i, row = e >> 3, v = e & 7;
+        ld[i] = row < F1 ? job_load<LD>(J, row * F2 + col0 + v) : c_zero();
+    }
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int e = c.tid + 256 * i, row = e >> 3, v = e & 7;
-            s[v * WB_RS + ms_pad(row)] = row < F1 ? c_mul(ld[i], __ldg(&J.b1_chirp[row])) : c_zero();
-        }
-    } else {
-#pragma unroll 1
-        for (int i = 0; i < 4; ++i) {
-            const int e = c.tid + 256 * i, row = e >> 3, v = e & 7;
-            cpx val = c_zero();
-            if (row < F1) val = c_mul(job_load<LD>(J, row * F2 + col0 + v), __ldg(&J.b1_chirp[row]));
-            s[v * WB_RS + ms_pad(row)] = val;
-        }
+    for (int i = 0; i < 4; ++i) {
+        const int e = c.tid + 256 * i, row = e >> 3, v = e & 7;
+        s[v * WB_RS + ms_pad(row)] = row < F1 ? c_mul(ld[i], __ldg(&J.b1_chirp[row])) : c_zero();
     }
     c.sync();
     cpx v[8];
@@ -595,22 +575,22 @@ MS_DEV void fft_cols_warp_body(const FftJob* MS_RESTRICT jobs, const Ctx& c) {
     fft_cols_bluestein_warp256<LD, ST, TWID>(J, c);
 }
 
-template <int LD, int ST, int TWID, int SQ, int SB>
+template <int LD, int ST, int TWID, int SB>
 MS_DEV void fft_cols_body(const FftJob* MS_RESTRICT jobs, const Ctx& c) {
     const FftJob& J = stage_job(jobs, c);
     if (SB) { fft_cols_bluestein_static<LD, ST, TWID, SB>(J, c); return; }
-    const int T = SQ ? SQ : J.T, F1 = SQ ? 256 : J.F1, F2 = SQ ? 256 : J.F2;
+    const int T = J.T, F1 = J.F1, F2 = J.F2;
     const int col0 = c.bx * T;
     if (col0 >= F2) return;
-    const int cnt = SQ ? SQ : ((F2 - col0) < T ? (F2 - col0) : T);
-    const int rows = SQ ? 256 : (J.B1 ? J.B1 : F1);           // vector length held in the tile
+    const int cnt = (F2 - col0) < T ? (F2 - col0) : T;
+    const int rows = J.B1 ? J.B1 : F1;                         // vector length held in the tile
     cpx* s = (cpx*)(c.smem + MS_JOB_SMEM);
     cpx* const sA = s;
-    cpx* s2 = s + (ms_pad((rows - 1) * T + T - 1) + 2);       // (unused by the static in-place tiles)
+    cpx* s2 = s + (ms_pad((rows - 1) * T + T - 1) + 2);
     TileGeom g; g.cnt = cnt; g.vs = 1; g.es = T; g.colmajor = 1;
     const int total = F1 * cnt;
-    const unsigned mgc = SQ ? ms_magic_c(SQ ? SQ : 1) : ms_magic_dev(cnt);
-    if (!SQ && J.B1) {
+    const unsigned mgc = ms_magic_dev(cnt);
+    if (J.B1) {
         // length-F1 DFT of every column as chirp * IFFT_B1(FFT_B1(x * chirp) * spec)
         const int all = rows * cnt;
 #pragma unroll 2
@@ -660,7 +640,7 @@ MS_DEV void fft_cols_body(const FftJob* MS_RESTRICT jobs, const Ctx& c) {
         }
     }
     c.sync();
-    s = SQ ? tile_fft_256<1, SQ ? SQ : 1>(s, g, J.tw1, c) : tile_fft<1>(s, s2, g, J.p1, J.tw1, c);
+    s = tile_fft<1>(s, s2, g, J.p1, J.tw1, c);
     if (TWID && c.nthr % cnt == 0) {
         // the thread keeps its column: stepped twiddles as in the static Bluestein tiles
         const int k10 = ms_fastdiv(c.tid, mgc);
@@ -685,19 +665,19 @@ MS_DEV void fft_cols_body(const FftJob* MS_RESTRICT jobs, const Ctx& c) {
 }
 
 // ---- rows kernel -----------------------------------------------------------------------------------
-template <int LD, int MODE, int ST, int SQ>
+template <int LD, int MODE, int ST>
 MS_DEV void fft_rows_body(const FftJob* MS_RESTRICT jobs, const Ctx& c) {
     const FftJob& J = stage_job(jobs, c);
-    const int G = SQ ? SQ : J.G, F1 = SQ ? 256 : J.F1, F2 = SQ ? 256 : J.F2;
+    const int G = J.G, F1 = J.F1, F2 = J.F2;
     const int row0 = c.bx * G;
     if (row0 >= F1) return;
-    const int cnt = SQ ? SQ : ((F1 - row0) < G ? (F1 - row0) : G);
+    const int cnt = (F1 - row0) < G ? (F1 - row0) : G;
     cpx* s = (cpx*)(c.smem + MS_JOB_SMEM);
     cpx* const sA = s;
     TileGeom g; g.cnt = cnt; g.vs = (ms_pad(F2) + 1) | 1; g.es = 1; g.colmajor = 0;
-    cpx* s2 = s + (G * g.vs + 2);                                 // (unused by the static in-place tiles)
+    cpx* s2 = s + (G * g.vs + 2);
     const int total = F2 * cnt;
-    const unsigned mgF = SQ ? ms_magic_c(256) : J.p2.mg_F, mgc = SQ ? ms_magic_c(SQ ? SQ : 1) : ms_magic_dev(cnt);
+    const unsigned mgF = J.p2.mg_F, mgc = ms_magic_dev(cnt);
     if (LdPlain<LD>::v) {
         for (int e0 = c.tid; e0 < total; e0 += 4 * c.nthr) {
             cpx ld[4];
@@ -720,7 +700,7 @@ MS_DEV void fft_rows_body(const FftJob* MS_RESTRICT jobs, const Ctx& c) {
         }
     }
     c.sync();
-    s = SQ ? tile_fft_256<0, SQ ? SQ : 1>(s, g, J.tw2, c) : tile_fft<0>(s, s2, g, J.p2, J.tw2, c);
+    s = tile_fft<0>(s, s2, g, J.p2, J.tw2, c);
     if (MODE == MODE_NAT) {
         for (int e = c.tid; e < total; e += c.nthr) {
             const int k2 = ms_fastdiv(e, mgc), r = e - k2 * cnt;
@@ -740,7 +720,7 @@ MS_DEV void fft_rows_body(const FftJob* MS_RESTRICT jobs, const Ctx& c) {
         }
         c.sync();
         cpx* other = (s == sA) ? s2 : sA;
-        s = SQ ? tile_fft_256<0, SQ ? SQ : 1>(s, g, J.tw2, c) : tile_fft<0>(s, other, g, J.p2, J.tw2, c);
+        s = tile_fft<0>(s, other, g, J.p2, J.tw2, c);
 #pragma unroll 4
         for (int e = c.tid; e < total; e += c.nthr) {
             const int r = ms_fastdiv(e, mgF), i = e - r * F2;

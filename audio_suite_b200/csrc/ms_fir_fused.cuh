@@ -14,11 +14,8 @@
 // (512 contiguous bytes per warp instruction).  The strided side of each phase goes through a transposing tile in
 // shared memory (8 vectors x 256) so that global accesses are 64- / 128-byte segments.
 //
-// On the GPU the three phases run inside ONE persistent kernel launched as thread-block clusters: the CTAs of a
-// cluster share a unit, split the 32 tiles of each phase and meet at the hardware cluster barrier between phases;
-// the scratch block is 1 MB per CLUSTER (not per unit), is rewritten for every unit and therefore lives in the
-// 126 MB L2 -- x is read from HBM once and y written once.  The same phase bodies are also launchable one phase per
-// kernel (scratch per unit): that is what the CPU block emulator runs, and the A/B baseline on the GPU.
+// Each phase is its own launch, grid = (tiles, units): CTA (t, u) does tile t of unit u, and unit u owns scratch block
+// u.  The launch boundary is the barrier between phases.  The CPU block emulator runs the same launches.
 
 #ifdef MS_HOST_EMUL
 #define MS_LDCG(p) (*(p))
@@ -343,34 +340,3 @@ MS_DEV void fir_sort_taps_body(const FirSortJob* MS_RESTRICT jobs, const int* MS
         if (off >= 0 && off < FF_N * FF_N && (off & 255) == r) { soff[at] = off; sgain[at] = __ldg(&tap_gain[t]); ++at; }
     }
 }
-
-#ifndef MS_HOST_EMUL
-// ---- persistent cluster kernel ------------------------------------------------------------------------------------------
-// grid = clusters * CL CTAs of FF_NTHR threads; cluster k takes units k, k + clusters, ...; its CTAs split the 32 tiles
-// of each phase (tile = rank, rank + CL, ...: the SAME tiles in P1 and P3, so a CTA only overwrites scratch columns it
-// has itself finished reading) and meet at the cluster barrier between phases.  Scratch: 65536 complex per cluster.
-MS_DEV void ff_cluster_sync() {
-    __threadfence();
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-MS_DEV unsigned ff_cluster_rank() { unsigned r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-MS_DEV unsigned ff_cluster_id() { unsigned r; asm volatile("mov.u32 %0, %%clusterid.x;" : "=r"(r)); return r; }
-MS_DEV unsigned ff_nclusters() { unsigned r; asm volatile("mov.u32 %0, %%nclusterid.x;" : "=r"(r)); return r; }
-template <int CL>
-__global__ void __launch_bounds__(FF_NTHR, 3) fir_cluster_kernel(const FirUnit* __restrict__ units, int n_units, FirTables T, cpx* scratch) {
-    extern __shared__ float4 ms_dyn_smem[];
-    Ctx c;
-    c.tid = threadIdx.x; c.nthr = blockDim.x; c.bx = blockIdx.x; c.by = 0;
-    c.smem = (char*)ms_dyn_smem;
-    const int rank = (int)ff_cluster_rank(), cid = (int)ff_cluster_id(), ncl = (int)ff_nclusters();
-    cpx* S = scratch + (size_t)cid * (FF_N * FF_N);
-    for (int u = cid; u < n_units; u += ncl) {
-        const FirUnit& U = units[u];
-        for (int t = rank; t < FF_TILES; t += CL) fir_p1_tile(U, T, S, t, c);
-        ff_cluster_sync();
-        for (int t = rank; t < FF_TILES2; t += CL) fir_p2_tile<false>(U, T, S, t, c);
-        ff_cluster_sync();
-        for (int t = rank; t < FF_TILES; t += CL) fir_p3_tile(U, T, S, t, c);
-    }
-}
-#endif

@@ -33,7 +33,7 @@ def stage_of(launches):
             continue
         elif "AdsrTableK" in n or "OlaK" in n:
             stage = "overlap_add"
-        elif "ErScatterK" in n or "FirP1K" in n or "FirP2K" in n or "FirP3K" in n or "fir_cluster_kernel" in n:
+        elif "ErScatterK" in n or "FirP1K" in n or "FirP2K" in n or "FirP3K" in n:
             stage = "fir_overlap_save"
         elif "PostMaxK" in n or "PostWriteK" in n or "RollK" in n:
             stage = "post"

@@ -37,7 +37,7 @@ w("`roofline` of the dominant stage (%s): achieved %.1f GB/s of %.1f (frac %.4f)
       rf["kernel"], rf["achieved"], rf["peak"], rf["frac"], rf["algorithmic_bytes"] / 1e9, (rf["traffic"] or 0) / 1e9, rf["traffic_note"]))
 w("### Every launch of one step, timed live (CUDA event after each launch via `ms_set_launch_hook`; the length classes of a spectral stage run one after the other in this mode)\n")
 w("`ColsWarpK / ColsWarp512K / ColsWarpPlainK<LD, ST, TWID>`: warp-local column transforms (in-tile Bluestein of 256 / 512, plain 256); "
-  "`ColsK<LD, ST, TWID, SQ, SB>` / `RowsK<LD, MODE, ST, SQ>`: block-wide tiles; `SpecOpK`: the spectral operators, elementwise.\n")
+  "`ColsK<LD, ST, TWID, SB>` / `RowsK<LD, MODE, ST>`: block-wide tiles; `SpecOpK`: the spectral operators, elementwise.\n")
 w("| # kernel | ms |\n|---|---|")
 for k, v in d["kernels_ms"].items():
     w("| %s | %.3f |" % (k, v))

@@ -18,9 +18,9 @@ for line in sass.splitlines():
     m = re.match(r"\s+/\*([0-9a-f]+)\*/\s+(.*?);", line)
     if m and cur is not None:
         cur.append((m.group(1), m.group(2).strip()))
-KEEP = ("ColsWarpK<0", "ColsWarpK<2", "ColsWarp512K<0", "ColsWarp512K<2", "ColsWarpPlainK<0", "ColsWarpPlainK<2", "SpecOpK", "RowsK<0, 0, 2, 0>",
-        "RowsK<0, 0, 4, 0>", "FirP1K", "FirP2K", "FirP3K", "FirSortK", "OlaK", "PostMaxK", "PostWriteK", "SynthNormalK", "SynthDustK",
-        "synth_normal_cluster_kernel<4>", "fir_cluster_kernel<8>", "PartialLockK", "ErScatterK", "DecimateK")
+KEEP = ("ColsWarpK<0", "ColsWarpK<2", "ColsWarp512K<0", "ColsWarp512K<2", "ColsWarpPlainK<0", "ColsWarpPlainK<2", "SpecOpK", "RowsK<0, 0, 2>",
+        "RowsK<0, 0, 4>", "FirP1K", "FirP2K", "FirP3K", "FirSortK", "OlaK", "PostMaxK", "PostWriteK", "SynthNormalK", "SynthDustK",
+        "synth_normal_cluster_kernel<4>", "PartialLockK", "ErScatterK", "DecimateK")
 COLS = [("inst", None), ("FP64", r"^(@!?U?P\d+ )?D(FMA|ADD|MUL|SETP|MNMX)"), ("LDS", r"\bLDS"), ("STS", r"\bSTS"), ("LDG", r"\bLDG"), ("STG", r"\bSTG"),
         ("BAR", r"\bBAR\."), ("WARPSYNC", r"\bWARPSYNC"), ("SHFL", r"\bSHFL"), ("CGABAR", r"UCGABAR"), ("DSMEM (UPRMT / SR_SWINHI)", r"UPRMT|SR_SWINHI"),
         ("LDL", r"\bLDL"), ("STL", r"\bSTL"), ("ATOM", r"\bATOM|\bRED\."), ("UTMA / UBLKCP", r"UTMA|UBLKCP"), ("MMA", r"MMA")]
@@ -44,7 +44,7 @@ out = ["# SASS census of the shipped libmicrosound_b200.so (round 2, final build
        "ColsWarpPlainK, FirP1K/P2K/P3K); the hardware cluster barrier `UCGABAR_ARV` / `UCGABAR_WAIT` and the distributed-shared-memory accesses",
        "(PTX `mapa` + `ld.shared::cluster` become `UPRMT` of the CTA rank into the shared-window address, `S2UR SR_SWINHI` and a generic `LD.E`) in",
        "`synth_normal_cluster_kernel` -- the cluster form of the synthesis kernel that the DEFAULT path launches for small",
-       "batches -- and in the measured-and-rejected `fir_cluster_kernel`; `SHFL` in the reductions / scans; no `ATOM` / `RED` in ErScatterK and",
+       "batches; `SHFL` in the reductions / scans; no `ATOM` / `RED` in ErScatterK and",
        "PartialLockK (deterministic gather forms; PostMaxK keeps one order-independent atomicMax per CTA); `LDL` / `STL` = register spills (FirP2K).",
        "There is no `UTMA*` / `UBLKCP`: tiles are staged through registers with all loads of a tile in flight before the first dependent store",
        "(DESIGN.md section 4) -- the two ends of the FIR pipeline read / write real samples at 8-byte granularity, which the 16-byte alignment",
@@ -77,6 +77,5 @@ excerpt("warp-level barriers inside the transforms -- ColsWarp512K (two 512-poin
 excerpt("warp-level barriers inside the FFT phases -- FirP2K", "FirP2K", [r"WARPSYNC", r"BAR\."], 8)
 excerpt("block maximum by warp shuffles -- PostMaxK", "PostMaxK", [r"SHFL"], 5)
 excerpt("prefix scan by warp shuffles -- SynthNormalK", "SynthNormalK", [r"SHFL"], 5)
-excerpt("hardware cluster barrier between the phases -- fir_cluster_kernel<8> (built, measured slower, not the default)", "fir_cluster_kernel<8>", [r"UCGABAR", r"MEMBAR", r"CCTL"], 6)
 open(os.path.join(ROOT, "profiles", "sass_r02_census.md"), "w").write("\n".join(out) + "\n")
 print("\n".join(out[:40]))

@@ -4,17 +4,9 @@ overlap-add + ADSR and the stereo / clip / normalise tail -- against plain float
 Every check drives the C ABI directly with hand-built records, on whichever device it is given (the block emulator in
 the CPU suite, the B200 in the GPU suite).  In float32 every input is rounded to float32 before the reference sees it,
 so reference and kernel start from the same data.  Buffers carry sentinels around each render's range: reads outside
-the range show up as wrong values, writes outside it as overwritten sentinels.
-
-fir_mode_main() performs the FIR checks at full size on cuda:0 under whatever MS_FIR_MODE the environment holds (the
-CUDA build reads that switch once per process, so the GPU tests call it in one subprocess per mode) and prints one JSON
-line with the per-case errors, the kernels that ran and a digest of the outputs."""
+the range show up as wrong values, writes outside it as overwritten sentinels."""
 import ctypes as C
-import hashlib
-import json
-import os
 import re
-import sys
 
 import numpy as np
 
@@ -182,9 +174,9 @@ def fir_cases(big):
     return c
 
 
-def fir_cluster_batch(n_renders=100):
-    """300 fused units (three per render) sharing one IR spectrum, with and without taps:
-    more units than resident clusters (444 / CL), so every cluster walks several units through its scratch block."""
+def fir_many_units_batch(n_renders=100):
+    """300 fused units (three per render) sharing one IR spectrum, with and without taps: one launch per phase covers
+    every unit, each with its own scratch block."""
     rng = np.random.default_rng(404)
     hop = 65536 - 8160 + 1
     base = fir_case("cluster-0", rng, 5 * hop + 1000, 6000, 320, 2160, 65536, dup=12)
@@ -257,19 +249,17 @@ def fir_run(dev, precision, cases, runs=1):
     return outs, starts, log
 
 
-def fir_expected_route(cases, mode):
-    """Kernel base names each case must have launched: fused 65536-point units (one launch per phase, or the cluster
-    kernel), or the spectral engine's rows / columns behind the dense tap scatter."""
-    fused = [cs["B"] == 65536 and mode != 0 for cs in cases]
+def fir_expected_route(cases):
+    """Kernel base names each case must have launched: fused 65536-point units (one launch per phase), or the spectral
+    engine's rows / columns behind the dense tap scatter."""
+    fused = [cs["B"] == 65536 for cs in cases]
     want, absent = set(), set()
     if any(fused):
-        want |= {"FirP1K", "FirP2K", "FirP3K"} if mode in (0, 1) else {"fir_cluster_kernel"}
+        want |= {"FirP1K", "FirP2K", "FirP3K"}
         if any(f and len(cs["offs"]) for f, cs in zip(fused, cases)):
             want.add("FirSortK")
     else:
-        absent |= {"FirP1K", "FirP2K", "FirP3K", "FirSortK", "fir_cluster_kernel"}
-    if mode not in (0, 1):
-        absent |= {"FirP1K", "FirP2K", "FirP3K"}
+        absent |= {"FirP1K", "FirP2K", "FirP3K", "FirSortK"}
     legacy = [not f for f in fused]
     if any(legacy):
         want.add("RowsK")
@@ -300,28 +290,17 @@ def check_fir_outputs(precision, cases, out, starts, ref=fir_reference, refs=Non
     return errs
 
 
-def check_fir(dev, precision, big=False, mode=1, cluster=False, ref_cache=None):
+def check_fir(dev, precision, big=False, many=False):
     """Each case alone (its route asserted), then all of them as one batch run twice (bitwise-identical repeats), and
-    optionally the many-unit batch.  Returns {"errors": ..., "kernels": ..., "digest": ...}."""
+    optionally the many-unit batch.  Returns {"errors": ..., "kernels": ...}."""
     cases = fir_cases(big)
-    refs = []
-    for cs in cases:
-        path = os.path.join(ref_cache, "%s_%s.npy" % (cs["name"], precision)) if ref_cache else None
-        if path and os.path.exists(path):
-            refs.append(np.load(path))
-            continue
-        r = fir_reference(_as_ref(cs["ir"], precision), cs["offs"], _as_ref(cs["gains"], precision), _as_ref(cs["x"], precision),
-                          cs["x_begin"], cs["x_end"])
-        if path:
-            np.save(path, r)
-        refs.append(r)
+    refs = [fir_reference(_as_ref(cs["ir"], precision), cs["offs"], _as_ref(cs["gains"], precision), _as_ref(cs["x"], precision),
+                          cs["x_begin"], cs["x_end"]) for cs in cases]
     errors, kernels = {}, set()
     for cs, r in zip(cases, refs):
         (out,), starts, log = fir_run(dev, precision, [cs])
-        want, absent = fir_expected_route([cs], mode)
-        assert want <= log.base() and not (absent & log.base()), (cs["name"], mode, sorted(log.base()))
-        if mode not in (0, 1) and cs["B"] == 65536:
-            assert "fir_cluster_kernel<%d>" % mode in log.names, (cs["name"], log.names)
+        want, absent = fir_expected_route([cs])
+        assert want <= log.base() and not (absent & log.base()), (cs["name"], sorted(log.base()))
         errors.update(check_fir_outputs(precision, [cs], out, starts, refs=[r], label="alone"))
         kernels |= set(log.names)
     # one batch: the classes interleaved (stable sort by class, per-render offsets), IRs shared and duplicated
@@ -332,18 +311,16 @@ def check_fir(dev, precision, big=False, mode=1, cluster=False, ref_cache=None):
     assert np.array_equal(outs[0], outs[1], equal_nan=True), "second ms_fir_run on one handle differs"
     berr = check_fir_outputs(precision, batch, outs[0], starts, refs=[refs[i] for i in order], label="batch")
     errors.update({"batch:" + k: v for k, v in berr.items()})
-    h = hashlib.sha256(outs[0].tobytes())
-    if cluster:
-        cb = fir_cluster_batch()
-        outs, starts, log = fir_run(dev, precision, cb, runs=2)
+    if many:
+        mb = fir_many_units_batch()
+        outs, starts, log = fir_run(dev, precision, mb, runs=2)
         assert np.array_equal(outs[0], outs[1], equal_nan=True), "second ms_fir_run on the many-unit batch differs"
-        want, absent = fir_expected_route(cb, mode)
-        assert want <= log.base() and not (absent & log.base()), (mode, sorted(log.base()))
-        cerr = check_fir_outputs(precision, cb, outs[0], starts, ref=fir_reference_fft, label="cluster batch")
-        errors["cluster-batch-worst"] = max(cerr.values())
+        want, absent = fir_expected_route(mb)
+        assert want <= log.base() and not (absent & log.base()), sorted(log.base())
+        merr = check_fir_outputs(precision, mb, outs[0], starts, ref=fir_reference_fft, label="many-unit batch")
+        errors["many-unit-batch-worst"] = max(merr.values())
         kernels |= set(log.names)
-        h.update(outs[0].tobytes())
-    return {"errors": errors, "kernels": sorted(kernels), "digest": h.hexdigest()}
+    return {"errors": errors, "kernels": sorted(kernels)}
 
 
 # ---- 2. overlap-add + ADSR (ms_adsr_tables, ms_overlap_add) ---------------------------------------------------------------
@@ -645,14 +622,3 @@ def check_in_situ(dev, params_list, precision="f64"):
         return errs
     finally:
         br.close()
-
-
-# ---- the GPU FIR modes: one process per MS_FIR_MODE ------------------------------------------------------------------------
-def fir_mode_main(ref_cache=None):
-    dev = engine.CudaDevice(0)
-    mode = int(os.environ.get("MS_FIR_MODE", "1"))
-    res = {}
-    for precision in ("f64", "f32"):
-        res[precision] = check_fir(dev, precision, big=True, mode=mode, cluster=True, ref_cache=ref_cache)
-    print(json.dumps(dict(mode=mode, **res)))
-

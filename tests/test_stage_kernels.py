@@ -1,23 +1,15 @@
 """The time-domain stages every render runs after the grains -- FIR (reflection cloud + impulse response, overlap-save),
 overlap-add + ADSR, stereo / clip / normalise -- checked stage by stage against float64 restatements (stage_checks.py):
 directly through the C ABI at the edges of each kernel, and in situ on real renders, each stage on the device's own
-input.  The CPU tests run the kernel bodies on the block emulator at small sizes; the gpu tests repeat them at full size
-and run the FIR under every MS_FIR_MODE (one process each: the CUDA build reads the switch once per process).  Every
-test prints its per-case errors; the tolerances and the errors measured on a B200 are listed in stage_checks.py."""
-import functools
-import json
-import os
-import subprocess
-import sys
-
+input.  The CPU tests run the kernel bodies on the block emulator at small sizes; the gpu tests repeat them at full size,
+the FIR with a batch of many fused units as well.  Every test prints its per-case errors; the tolerances and the errors
+measured on a B200 are listed in stage_checks.py."""
 import numpy as np
 import pytest
 
 import kernel_checks as K
 import stage_checks as S
 from audio_suite_b200 import configs
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _report(title, errors):
@@ -56,15 +48,12 @@ def _check_in_situ(dev, title, params):
 
 
 # ---- CPU: block emulator --------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("mode", [1, 0])
 @pytest.mark.parametrize("precision", ["f64", "f32"])
-def test_fir_stage_emulated(emul, precision, mode, monkeypatch):
+def test_fir_stage_emulated(emul, precision):
     """Every block class, tap sets reaching the self-partnered rows 0 / 128 and the 4096-tap limit, shared delays,
-    support edges, one mixed batch run twice; mode 0 sends the 65536-point blocks through the legacy sequence (the
-    emulator reads MS_FIR_MODE at ms_fir_create)."""
-    monkeypatch.setenv("MS_FIR_MODE", str(mode))
-    res = S.check_fir(emul, precision, big=False, mode=mode)
-    _report("FIR %s MS_FIR_MODE=%d" % (precision, mode), res["errors"])
+    support edges, one mixed batch run twice."""
+    res = S.check_fir(emul, precision, big=False)
+    _report("FIR %s" % precision, res["errors"])
 
 
 @pytest.mark.parametrize("precision", ["f64", "f32"])
@@ -84,34 +73,13 @@ def test_stages_in_situ_emulated(emul, case):
 
 
 # ---- GPU --------------------------------------------------------------------------------------------------------------------
-@pytest.fixture(scope="module")
-def fir_ref_cache(tmp_path_factory):
-    return str(tmp_path_factory.mktemp("fir_ref"))
-
-
-@functools.lru_cache(maxsize=None)
-def _fir_mode_run(mode, ref_cache):
-    code = "import sys; sys.path[:0] = [%r, %r]; import stage_checks; stage_checks.fir_mode_main(%r)" % (
-        ROOT, os.path.join(ROOT, "tests"), ref_cache)
-    env = dict(os.environ, MS_FIR_MODE=str(mode))
-    p = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, cwd=ROOT)
-    assert p.returncode == 0, "MS_FIR_MODE=%d:\n%s" % (mode, p.stderr[-6000:])
-    return json.loads(p.stdout.strip().splitlines()[-1])
-
-
 @pytest.mark.gpu
-@pytest.mark.parametrize("mode", [1, 0, 4, 8, 16])
-def test_fir_stage_every_mode(cuda_dev, fir_ref_cache, mode):
-    """Full-size cases plus a batch of 300 fused units (more than the resident clusters, so clusters walk several
-    units through one reused scratch block).  Clusters run the same tile bodies as mode 1: bitwise-equal output."""
-    res = _fir_mode_run(mode, fir_ref_cache)
+def test_fir_stage(cuda_dev):
+    """Full-size cases plus a batch of 300 fused units sharing one IR spectrum, run twice (bitwise-equal repeats)."""
     for precision in ("f64", "f32"):
-        _report("FIR %s MS_FIR_MODE=%d" % (precision, mode), res[precision]["errors"])
-        print("  kernels:", ", ".join(k for k in res[precision]["kernels"] if k.startswith(("Fir", "fir", "ErScatter"))))
-    if mode in (4, 8, 16):
-        one = _fir_mode_run(1, fir_ref_cache)
-        for precision in ("f64", "f32"):
-            assert res[precision]["digest"] == one[precision]["digest"], (mode, precision)
+        res = S.check_fir(cuda_dev, precision, big=True, many=True)
+        _report("FIR %s" % precision, res["errors"])
+        print("  kernels:", ", ".join(k for k in res["kernels"] if k.startswith(("Fir", "ErScatter"))))
 
 
 @pytest.mark.gpu

@@ -392,9 +392,9 @@ def fir_pair_run(dev, precision, cases, runs=1):
     return outs, rows, starts, log
 
 
-def check_pairs(dev, precision, cases, mode=1, fft=False):
+def check_pairs(dev, precision, cases, fft=False):
     """The batch against float64 convolution per channel, two runs bitwise equal, every row bitwise equal to the same row
-    run alone; the pair kernel ran exactly when the mode and the block class call for it.  Returns {"errors", "kernels"}."""
+    run alone; the pair kernel ran exactly when the block class calls for it.  Returns {"errors", "kernels"}."""
     outs, rows, starts, log = fir_pair_run(dev, precision, cases, runs=2)
     assert np.array_equal(outs[0], outs[1], equal_nan=True), "second ms_fir_run on one handle differs"
     ref = S.fir_reference_fft if fft else S.fir_reference
@@ -404,18 +404,16 @@ def check_pairs(dev, precision, cases, mode=1, fft=False):
     alone, a_starts, _ = S.fir_run(dev, precision, [dict(cs, share=None) for cs in rows])
     for cs, s, sa in zip(rows, starts, a_starts):
         n = len(cs["x"])
-        assert np.array_equal(outs[0][s:s + n], alone[0][sa:sa + n]), (precision, mode, cs["name"], "differs from the lone row")
+        assert np.array_equal(outs[0][s:s + n], alone[0][sa:sa + n]), (precision, cs["name"], "differs from the lone row")
     fused_pair = any("ir_r" in cs and cs["B"] == 65536 for cs in cases)
-    assert ("FirP2PairK" in log.base()) == (fused_pair and mode == 1), (mode, sorted(log.base()))
+    assert ("FirP2PairK" in log.base()) == fused_pair, sorted(log.base())
     return {"errors": errors, "kernels": sorted(set(log.names))}
 
 
 @pytest.mark.parametrize("precision", ["f64", "f32"])
-@pytest.mark.parametrize("mode", ["1", "0"])
-def test_fir_pairs_emulated(emul, precision, mode, monkeypatch):
-    monkeypatch.setenv("MS_FIR_MODE", mode)
-    res = check_pairs(emul, precision, pair_cases(), mode=int(mode))
-    print("FIR pairs %s mode %s: worst %.2e" % (precision, mode, max(res["errors"].values())))
+def test_fir_pairs_emulated(emul, precision):
+    res = check_pairs(emul, precision, pair_cases())
+    print("FIR pairs %s: worst %.2e" % (precision, max(res["errors"].values())))
 
 
 def _workspace(dev, precision, cases):
@@ -471,7 +469,6 @@ def test_fir_pairs_thread_schedule():
     for seed in (None, "1", "7"):
         env = dict(os.environ)
         env.pop("MS_EMUL_SHUFFLE", None)
-        env.pop("MS_FIR_MODE", None)
         if seed:
             env["MS_EMUL_SHUFFLE"] = seed
         p = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, cwd=ROOT)
@@ -699,31 +696,11 @@ def test_mixed_batch_gpu(cuda_dev):
         assert np.array_equal(a[i], d.astype(a[i].dtype)) or np.array_equal(a[i].astype(np.float64), d), i
 
 
-def fir_mode_main():
-    """Stereo batch output digests under the environment's MS_FIR_MODE (read once per process by the CUDA build)."""
-    dev = engine.CudaDevice(0)
-    res = {}
-    for precision in ("f64", "f32"):
-        r = check_pairs(dev, precision, pair_cases(big=True), mode=int(os.environ.get("MS_FIR_MODE", "1")), fft=True)
-        outs, _, _, _ = fir_pair_run(dev, precision, pair_cases(big=True))
-        import hashlib
-        res[precision] = dict(worst=max(r["errors"].values()), digest=hashlib.sha256(outs[0].tobytes()).hexdigest())
-    print(json.dumps(res))
-
-
 @pytest.mark.gpu
-def test_fir_modes_gpu(cuda_dev):
-    code = "import sys; sys.path[:0] = [%r, %r]; import test_stereo_ir; test_stereo_ir.fir_mode_main()" % (ROOT, os.path.join(ROOT, "tests"))
-    res = {}
-    for mode in ("1", "0", "4", "8", "16"):
-        env = dict(os.environ, MS_FIR_MODE=mode)
-        p = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, cwd=ROOT)
-        assert p.returncode == 0, "MS_FIR_MODE=%s:\n%s" % (mode, p.stderr[-6000:])
-        res[mode] = json.loads(p.stdout.strip().splitlines()[-1])
-        print("MS_FIR_MODE=%s: %s" % (mode, {k: "%.2e" % v["worst"] for k, v in res[mode].items()}))
-    for mode in ("4", "8", "16"):
-        for precision in ("f64", "f32"):
-            assert res[mode][precision]["digest"] == res["1"][precision]["digest"], (mode, precision)
+def test_fir_pairs_gpu(cuda_dev):
+    for precision in ("f64", "f32"):
+        r = check_pairs(cuda_dev, precision, pair_cases(big=True), fft=True)
+        print("FIR pairs %s: worst %.2e" % (precision, max(r["errors"].values())))
 
 
 @pytest.mark.gpu

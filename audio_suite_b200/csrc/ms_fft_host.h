@@ -255,6 +255,7 @@ private:
         J.M = (int)M;
         if (M <= MS_SMALL_MAX) { J.M = ms_conv_len((int)need); J.F1 = 1; J.F2 = J.M; J.T = 1; J.G = 1; return true; }
         int l1 = std::min(lg / 2, 9);
+        while ((M >> l1) > MS_TILE_MAX) ++l1;          // f64 at M = 2^22: 1024 x 4096 (columns of 1024 rows, T = 2)
         J.F1 = 1 << l1; J.F2 = (int)(M >> l1);
         if (J.F2 > MS_TILE_MAX) return false;
         J.T = 16;

@@ -653,18 +653,13 @@ def render_batch(params_list, device=None, precision="auto", host_out=None, chun
     # the launching thread shares the interpreter with the planning threads: with the default 5 ms switch interval every
     # return from a ctypes / CUDA call could wait that long for the lock (measured: 5-7 ms per slice set-up instead of 2)
     si = sys.getswitchinterval()
-    sys.setswitchinterval(float(_os_env("MS_SWITCH") or 1e-4))
+    sys.setswitchinterval(1e-4)
     try:
         return _render_batch(params_list, device, precision, host_out, chunk, depth, workers, piece, ramp)
     finally:
         sys.setswitchinterval(si)
         if was:
             gc.enable()
-
-
-def _os_env(name):
-    import os
-    return os.environ.get(name, "")
 
 
 def _render_batch(params_list, device=None, precision="auto", host_out=None, chunk=384, depth=3, workers=None, piece=32, ramp=True):
@@ -690,9 +685,6 @@ def _render_batch(params_list, device=None, precision="auto", host_out=None, chu
         #  128,384 -> 77.1: every slice costs 1-2 ms of host work, and the host is what paces the first third of the sweep)
         head = [max(piece, c // 4), max(piece, 3 * c // 4)]
         tail = [max(piece, c // 2), max(piece, c // 4), max(piece, c // 4)]
-        if _os_env("MS_RAMP"):                     # development switch: "head sizes / tail sizes", e.g. "64,128,256/256,128,64"
-            h_, t_ = _os_env("MS_RAMP").split("/")
-            head, tail = [int(x) for x in h_.split(",") if x], [int(x) for x in t_.split(",") if x]
         body = max(0, n - sum(head) - sum(tail))
         chunk = head + [c] * (body // c) + ([body % c] if body % c else []) + tail
     if not hasattr(dev, "torch"):                   # host emulator device (tests): one slice after the other

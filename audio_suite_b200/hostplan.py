@@ -205,22 +205,20 @@ _SIDE_COL = [FIELDS.index(k) for k in ("gen_mode", "unfold_mode", "event_process
 def default_threads():
     """Native planning threads per slice: the cores this process may use, less two for the launching and the prefetching
     thread, shared between the ranks of the node."""
-    t = int(os.environ.get("MS_PLAN_THREADS", "0"))
-    if t > 0:
-        return t
     # (more than four slowed the launching thread's own slice set-up on the 16-core B200 hosts: 86.7 -> 79.4 ms per sweep)
     return max(1, min(4, (len(os.sched_getaffinity(0)) - 2) // max(1, int(os.environ.get("LOCAL_WORLD_SIZE", "1")))))
 
 
-def plan_chunk(params_list, threads=1):
+def plan_chunk(params_list, threads=None):
     """Packed Tables (tables.Tables) of a list of supported renders -- what tables.pack_chunk(plan_render(p) ...) returns.
-    `threads`: the native call plans blocks of 32 renders on that many threads and appends them in order (same tables)."""
+    `threads` (default: default_threads()): the native call plans blocks of 32 renders on that many threads and appends
+    them in order (same tables)."""
     from . import tables as T
     l = lib()
     R = len(params_list)
     rows, lane_ptr, lane_t, lane_v, irs, ir_len, btab = _marshal(params_list)
     h = l.ms_hp_plan(rows.ctypes.data, R, lane_ptr.ctypes.data, lane_t.ctypes.data, lane_v.ctypes.data, ir_len.ctypes.data,
-                     btab.ctypes.data, int(btab.shape[1]), max(1, int(threads)))
+                     btab.ctypes.data, int(btab.shape[1]), max(1, int(default_threads() if threads is None else threads)))
     try:
         bad = C.c_int(-1)
         err = l.ms_hp_error(h, C.byref(bad))
@@ -253,8 +251,3 @@ def plan_chunk(params_list, threads=1):
     t.pool_n, t.mono_n, t.frames, t.h_total, t.max_h, t.max_out_n, t.env_n = (int(v) for v in sc[:7])
     t.alg = dict(zip(("synth", "tilt_spectral", "grain_spectral", "overlap_add", "fir_in", "fir_taps", "post"), (int(v) for v in sc[7:])))
     return t
-
-
-def plan_slice(params_list, threads=None):
-    """plan_chunk with the default thread count (the native call splits the slice itself)."""
-    return plan_chunk(params_list, default_threads() if threads is None else threads)

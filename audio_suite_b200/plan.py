@@ -28,9 +28,6 @@ MODE_GAUSS, MODE_DUST, MODE_NOISE, MODE_SKEW, MODE_RES, MODE_PLAIN, MODE_WAVELET
 WAVELET_FLOOR = 128                 # M:319
 _MODE_ID = {m: i for i, m in enumerate(BASIC_MODES)}
 
-_NEXT_ROW_FLAGS = ()
-_NEXT_ROW_MODES = ()
-
 
 # --------------------------------------------------------------------------- breakpoint lanes (M:452-482)
 _BP_CACHE = {}
@@ -277,17 +274,8 @@ def grain_length(gen_sr, micro_ms, floor=16):
     return int(max(floor, round(gen_sr * micro_ms / 1000.0)))      # M:221 (gen_basic, floor 16), M:319 (wavelet atoms, 128)
 
 
-def check_supported(params):
-    for flag in _NEXT_ROW_FLAGS:
-        if params[flag]:
-            raise NotImplementedError(f"microsound_b200: '{flag}' is not on the accelerated path yet (SURVEY 8f)")
-    if params["gen_mode"] in _NEXT_ROW_MODES:
-        raise NotImplementedError(f"microsound_b200: generator '{params['gen_mode']}' is not on the accelerated path yet (SURVEY 8f)")
-
-
 def plan_render(params) -> RenderPlan:
     """Scalar half of render() (M:589-646, 742-753, 760-781)."""
-    check_supported(params)
     cap = ir_tap_cap(params)
     stereo_ir = ir_stereo(params)
     export = export_ratio(params)

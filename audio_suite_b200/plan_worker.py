@@ -10,11 +10,6 @@ import sys
 
 
 def main():
-    import os
-    try:                                             # planning yields the cores to the parent's launches / copies when asked to
-        os.nice(int(os.environ.get("MS_PLAN_NICE", "0")))
-    except Exception:
-        pass
     from audio_suite_b200 import plan as P, tables as T
     inp, out = sys.stdin.buffer, sys.stdout.buffer
     while True:
@@ -23,16 +18,14 @@ def main():
             return
         (size,) = struct.unpack("<Q", head)
         chunk = pickle.loads(inp.read(size))
-        # a dict {"pieces": [[params, ...], ...]} is answered piece by piece (streamed batches); a plain list is one piece
-        for piece in (chunk["pieces"] if isinstance(chunk, dict) else [chunk]):
-            try:
-                reply = ("ok", T.pack_chunk([P.plan_render(p) for p in piece]))
-            except BaseException as e:                     # the parent re-raises
-                reply = ("err", e)
-            blob = pickle.dumps(reply, protocol=pickle.HIGHEST_PROTOCOL)
-            out.write(struct.pack("<Q", len(blob)))
-            out.write(blob)
-            out.flush()
+        try:
+            reply = ("ok", T.pack_chunk([P.plan_render(p) for p in chunk]))
+        except BaseException as e:                     # the parent re-raises
+            reply = ("err", e)
+        blob = pickle.dumps(reply, protocol=pickle.HIGHEST_PROTOCOL)
+        out.write(struct.pack("<Q", len(blob)))
+        out.write(blob)
+        out.flush()
 
 
 if __name__ == "__main__":

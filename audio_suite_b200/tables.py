@@ -19,11 +19,13 @@ from __future__ import annotations
 
 import math
 import os
+import pickle
+import struct
 from dataclasses import dataclass, field, fields
 
 import numpy as np
 
-from . import _abi, decimate, plan as P
+from . import _abi, decimate, hostplan, plan as P
 
 _SPEC_OP_BYTES = np.dtype(_abi.SpecOp).itemsize
 _SPEC_JOB = np.dtype(_abi.SpecJob)
@@ -562,39 +564,10 @@ def pair_jobs(items):
 
 
 # --------------------------------------------------------------------------- worker pool
-class _Pending:
-    """Results of _WorkerPool.submit, retrievable in any order while the workers are still busy."""
-
-    def __init__(self, n):
-        import threading
-        self.results, self.ready, self.error, self.cv, self.threads = [None] * n, [False] * n, None, threading.Condition(), []
-
-    def put(self, i, value):
-        with self.cv:
-            self.results[i], self.ready[i] = value, True
-            self.cv.notify_all()
-
-    def fail(self, err):
-        with self.cv:
-            if self.error is None:
-                self.error = err
-            self.cv.notify_all()
-
-    def get(self, i):
-        with self.cv:
-            while not self.ready[i] and self.error is None:
-                self.cv.wait()
-            if not self.ready[i]:
-                raise self.error
-            out, self.results[i] = self.results[i], None
-            return out
-
-
 class _WorkerPool:
-    """Persistent `python -m audio_suite_b200.plan_worker` subprocesses, one feeder thread each."""
+    """Persistent `python -m audio_suite_b200.plan_worker` subprocesses, spoken to with length-prefixed pickles."""
 
     def __init__(self, size):
-        import os
         import subprocess
         import sys
         root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -604,19 +577,6 @@ class _WorkerPool:
         self.size = size
         self.procs = [subprocess.Popen([sys.executable, "-m", "audio_suite_b200.plan_worker"], stdin=subprocess.PIPE,
                                        stdout=subprocess.PIPE, env=env) for _ in range(size)]
-        # one worker per core, leaving the first cores of the affinity mask to the parent (kernel launches, table
-        # uploads, the copy stream): measured on the 16-core B200 hosts, workers floating over all cores stall
-        # the parent's CUDA calls for tens of ms at a time
-        try:
-            cores = sorted(os.sched_getaffinity(0))
-            spare = int(os.environ.get("MS_PLAN_SPARE_CORES", "2")) if len(cores) >= 8 else 0
-            usable = cores[spare:] or cores
-            # (pinning only helps when this process owns the box; ranks of a torchrun job share it unpinned)
-            if os.environ.get("MS_PLAN_PIN", "0") == "1":
-                for i, p in enumerate(self.procs):
-                    os.sched_setaffinity(p.pid, {usable[i % len(usable)]})
-        except Exception:
-            pass
         try:                                    # 1 MiB pipes: a request or a packed piece fits without blocking the writer
             import fcntl
             for p in self.procs:
@@ -625,62 +585,22 @@ class _WorkerPool:
         except Exception:
             pass
 
-    def submit(self, chunks, prep=None):
-        """Start planning `chunks` (lists of parameter dicts); returns a _Pending whose get(i) blocks until
-        chunk i is packed.  Chunks are handed out in order, so early chunks finish first.  `prep` (optional)
-        is applied to a chunk by the feeder thread right before it is sent."""
-        import pickle
-        import struct
-        import threading
-        pend = _Pending(len(chunks))
-        todo = list(enumerate(chunks))
-        lock = threading.Lock()
+    def send(self, w, obj):
+        blob = pickle.dumps(obj, protocol=pickle.HIGHEST_PROTOCOL)
+        f = self.procs[w].stdin
+        f.write(struct.pack("<Q", len(blob)))
+        f.write(blob)
+        f.flush()
 
-        def serve(proc):
-            # two requests in flight per worker: the worker finds its next piece already in the pipe when it
-            # finishes one, instead of waiting for this thread to be scheduled on a box whose cores are all busy
-            from collections import deque
-            inflight = deque()
-
-            def send_next():
-                with lock:
-                    if not todo or pend.error is not None:
-                        return
-                    i, chunk = todo.pop(0)
-                if prep is not None:
-                    chunk = prep(chunk)
-                blob = pickle.dumps(chunk, protocol=pickle.HIGHEST_PROTOCOL)
-                proc.stdin.write(struct.pack("<Q", len(blob)))
-                proc.stdin.write(blob)
-                proc.stdin.flush()
-                inflight.append(i)
-            try:
-                send_next()
-                send_next()
-                while inflight:
-                    i = inflight.popleft()
-                    head = proc.stdout.read(8)
-                    if len(head) < 8:
-                        raise RuntimeError("planning worker died")
-                    status, payload = pickle.loads(proc.stdout.read(struct.unpack("<Q", head)[0]))
-                    if status != "ok":
-                        raise payload
-                    pend.put(i, payload)
-                    send_next()
-            except BaseException as e:
-                pend.fail(e)
-        pend.threads = [threading.Thread(target=serve, args=(p,), daemon=True) for p in self.procs]
-        for t in pend.threads:
-            t.start()
-        return pend
-
-    def map(self, chunks):
-        pend = self.submit(chunks)
-        try:
-            return [pend.get(i) for i in range(len(chunks))]
-        except BaseException:
-            self.close()
-            raise
+    def recv(self, w):
+        f = self.procs[w].stdout
+        head = f.read(8)
+        if len(head) < 8:
+            raise RuntimeError("planning worker died")
+        status, payload = pickle.loads(f.read(struct.unpack("<Q", head)[0]))
+        if status != "ok":
+            raise payload
+        return payload
 
     def close(self):
         for p in self.procs:
@@ -715,14 +635,16 @@ def _pool(workers):
 def default_workers():
     """Planning worker processes per rank: the cores this process may run on, shared between the ranks of the box
     (torchrun sets LOCAL_WORLD_SIZE), minus two per rank for the parent (kernel launches, uploads, copy stream)."""
-    import os
-    forced = int(os.environ.get("MS_PLAN_WORKERS", "0"))
-    if forced:
-        return forced
     cores = len(os.sched_getaffinity(0))
     ranks = max(1, int(os.environ.get("LOCAL_WORLD_SIZE", "1")))
     share = cores // ranks
     return min(32, max(1, share - 2 if share >= 8 else share - 1 if share >= 3 else share))
+
+
+def _native(params_list):
+    """True when the native planner takes all of these renders.  MS_PLAN_PYTHON=1 sends every render to the Python
+    planner, the specification the native one is tested against."""
+    return hostplan.lib() is not None and not os.environ.get("MS_PLAN_PYTHON") and all(hostplan.supported(p) for p in params_list)
 
 
 def plan_stream(params_list, chunk, workers=None, piece=32):
@@ -740,13 +662,8 @@ def plan_stream(params_list, chunk, workers=None, piece=32):
         cuts.append((a, min(n, a + c)))
         a += c
     # slices whose renders all belong to the native planner's family are planned in-process by libms_hostplan.so
-    # (hostplan.plan_slice: no pickling, ~10x the Python planner's speed); the others go to the worker processes
-    from . import hostplan
-    have_native = hostplan.lib() is not None and not os.environ.get("MS_PLAN_PYTHON")
-
-    def is_native(a, b):
-        return have_native and all(hostplan.supported(p) for p in params_list[a:b])
-    if have_native and len(cuts) > 1 and workers > 1 and is_native(*cuts[0]):
+    # (hostplan.plan_chunk: no pickling, ~10x the Python planner's speed); the others go to the worker processes
+    if len(cuts) > 1 and workers > 1 and _native(params_list[cuts[0][0]:cuts[0][1]]):
         # Optimistic native path: the first slice is planned before anything else is looked at; then two Python threads
         # alternate over the remaining slices (one converts the parameters of slice k+1 while the native call of slice k --
         # which releases the GIL and plans blocks of renders on its own threads -- runs).  Slices come out in order.  The
@@ -770,10 +687,10 @@ def plan_stream(params_list, chunk, workers=None, piece=32):
         if rest is not None:
             yield from plan_stream(params_list[cuts[rest][0]:], sizes[rest:] if len(sizes) > rest else sizes[-1:], workers=workers, piece=piece)
         return
-    native = [is_native(a, b) for a, b in cuts]
+    native = [_native(params_list[a:b]) for a, b in cuts]
     if workers <= 1 or all(native):
         for (a, b), nat in zip(cuts, native):
-            yield hostplan.plan_slice(params_list[a:b]) if nat else pack_chunk([P.plan_render(p) for p in params_list[a:b]])
+            yield hostplan.plan_chunk(params_list[a:b]) if nat else pack_chunk([P.plan_render(p) for p in params_list[a:b]])
         return
     bounds = []
     for (a, b), nat in zip(cuts, native):
@@ -782,31 +699,12 @@ def plan_stream(params_list, chunk, workers=None, piece=32):
     # Static round-robin assignment: piece i belongs to worker i % W and is answered in order; the parent reads the
     # answers in piece order straight from the pipes (1 MiB pipes let a worker run a few pieces ahead).  Impulse
     # responses are digested before pickling (P._slim_params).
-    import pickle
-    import struct
     pool = _pool(workers)
     W = len(pool.procs)
-
-    def send(w, obj):
-        blob = pickle.dumps(obj, protocol=pickle.HIGHEST_PROTOCOL)
-        f = pool.procs[w].stdin
-        f.write(struct.pack("<Q", len(blob)))
-        f.write(blob)
-        f.flush()
 
     def slim(i):
         a, b = flat[i]
         return [P._slim_params(p) for p in params_list[a:b]]
-
-    def recv(w):
-        f = pool.procs[w].stdout
-        head = f.read(8)
-        if len(head) < 8:
-            raise RuntimeError("planning worker died")
-        status, payload = pickle.loads(f.read(struct.unpack("<Q", head)[0]))
-        if status != "ok":
-            raise payload
-        return payload
     # Requests go out piece by piece, round-robin (piece i -> worker i % W), from a FEEDER THREAD: the thread that
     # reads the answers never blocks on a write.  (Writing from the reading thread can deadlock: a request larger than
     # the free space of a worker's stdin pipe blocks the parent while that worker is itself blocked writing an answer
@@ -818,7 +716,7 @@ def plan_stream(params_list, chunk, workers=None, piece=32):
     def feed():
         try:
             for i in range(len(flat)):
-                send(i % W, slim(i))
+                pool.send(i % W, slim(i))
         except BaseException as e:          # a closed pool (abandoned generator) ends the feeder quietly;
             feed_err.append(e)              # anything else (e.g. an unpicklable parameter) must not leave the reader waiting
             if not isinstance(e, (BrokenPipeError, ValueError, OSError)):
@@ -829,9 +727,9 @@ def plan_stream(params_list, chunk, workers=None, piece=32):
         k = 0
         for (a, b), bs in zip(cuts, bounds):
             if bs is None:
-                yield hostplan.plan_slice(params_list[a:b])
+                yield hostplan.plan_chunk(params_list[a:b])
                 continue
-            parts = [recv((k + t) % W) for t in range(len(bs))]
+            parts = [pool.recv((k + t) % W) for t in range(len(bs))]
             k += len(bs)
             yield merge_chunks(parts)
         feeder.join()
@@ -842,21 +740,17 @@ def plan_stream(params_list, chunk, workers=None, piece=32):
         raise
 
 
-def plan_and_pack(params_list, workers=None):
-    """Returns (Tables, plans or None).  Small batches are planned in-process (plans kept for progress /
-    inspection); large ones by a persistent pool of worker processes that return packed chunks."""
-    import os
-    from . import hostplan
+def plan_and_pack(params_list, workers=None, min_batch=256):
+    """Returns (Tables, plans or None).  Renders of the native planner's family are planned by it; batches of fewer than
+    `min_batch` renders are planned in-process (plans kept for progress / inspection); larger ones by the worker processes,
+    as one slice of plan_stream."""
     n = len(params_list)
-    if hostplan.lib() is not None and not os.environ.get("MS_PLAN_PYTHON") and all(hostplan.supported(p) for p in params_list):
-        return hostplan.plan_slice(params_list), None
-    if workers is None:
-        workers = default_workers()
-    min_batch = int(os.environ.get("MS_PLAN_MIN_BATCH", "256"))
-    if n < min_batch or workers <= 1:
+    if _native(params_list):
+        return hostplan.plan_chunk(params_list), None
+    workers = default_workers() if workers is None else workers
+    if n == 0 or n < min_batch or workers <= 1:
         plans = [P.plan_render(p) for p in params_list]
         return pack_chunk(plans), plans
-    slim = [P._slim_params(p) for p in params_list]      # do not pickle multi-MB impulse responses per render
     per = max(min(32, max(1, n // workers)), (n + 2 * workers - 1) // (2 * workers))
-    chunks = _pool(workers).map([slim[i:i + per] for i in range(0, n, per)])
-    return merge_chunks(chunks), None
+    [tb] = plan_stream(params_list, n, workers, piece=per)      # runs it to its end: closed at its yield, it shuts the pool down
+    return tb, None

@@ -95,10 +95,10 @@ def test_batch_equals_single_renders(emul):
         assert np.max(np.abs(got.astype(np.float64) - one)) < 1e-6     # pairing changes rounding only
 
 
-def test_pooled_planning_matches_in_process(emul, monkeypatch):
-    """Large batches are planned and packed by worker processes in relocatable chunks; the merged tables
-    must render exactly what the single-chunk path renders."""
-    from audio_suite_b200 import engine
+def test_pooled_and_streamed_planning_match_in_process(emul):
+    """Large batches are planned and packed by worker processes in relocatable chunks, streamed (render_batch) or as one
+    batch (plan_and_pack); the merged tables must render exactly what the single-chunk path renders."""
+    from audio_suite_b200 import engine, tables as T
     ps = [configs.with_defaults(seed=10 + s, out_dur_s=0.05 + 0.01 * (s % 2), gen_mode=m, time_unfold=u, space_ir_on=True,
                                 _ir_audio=configs.synth_ir(0.02, 48000, 3))
           for s, (m, u) in enumerate([("Gaussian click", 25.0), ("Noise burst", 30.0), ("Dust impulses", 25.0),
@@ -117,10 +117,9 @@ def test_pooled_planning_matches_in_process(emul, monkeypatch):
     ramped = engine.render_batch(ps, device=emul, chunk=[1, 2, 3], workers=2, piece=2)  # slice schedule 1, 2, 3, 3: short first slices
     for a, c in zip(one, ramped):
         assert a.shape == c.shape and np.max(np.abs(a.astype(np.float64) - c.astype(np.float64))) < 1e-6
-    monkeypatch.setenv("MS_PLAN_MIN_BATCH", "2")
-    monkeypatch.setenv("MS_PLAN_WORKERS", "3")
-    br = engine.BatchRenderer(ps, device=emul)                                       # plan_and_pack through the pool
-    assert br.plans is None
+    tb, plans = T.plan_and_pack(ps, workers=3, min_batch=2)                          # through the pool
+    assert plans is None
+    br = engine.BatchRenderer(device=emul, tables=tb)
     br.run()
     pooled = [br.output(r) for r in range(br.n_renders)]
     br.close()

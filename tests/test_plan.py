@@ -127,14 +127,21 @@ def test_pooled_planning_keeps_the_whole_ir_for_the_fragment_generator():
 
 def test_streamed_planning_does_not_deadlock_on_large_requests():
     """ADVICE r1 (tables.py plan_stream): requests larger than the pipe (a 4 MB `_img_gray` per piece) used to block the
-    parent on a write while the worker blocked on its answer.  Requests now leave from a feeder thread."""
+    parent on a write while the worker blocked on its answer.  Requests now leave from a feeder thread, for streamed
+    batches and for the pooled batches of plan_and_pack (BatchRenderer(params_list)) alike."""
     import threading
     from audio_suite_b200 import tables as T
     img = np.random.default_rng(3).integers(0, 256, (2048, 2048)).astype(np.uint8)
-    ps = [configs.with_defaults(gen_mode="Image scanline", seed=i, out_dur_s=0.05, _img_gray=img) for i in range(96)]
-    got = []
-    th = threading.Thread(target=lambda: got.extend(T.plan_stream(ps, 32, workers=2, piece=16)), daemon=True)
-    th.start()
-    th.join(120)
-    T.shutdown_pool()
-    assert not th.is_alive() and len(got) == 3 and sum(len(t.post) for t in got) == 96
+    ps = [configs.with_defaults(gen_mode="Image scanline", seed=i, out_dur_s=0.05, _img_gray=img) for i in range(300)]
+    for plan, renders, slices in ((lambda: T.plan_stream(ps[:96], 32, workers=2, piece=16), 96, 3),
+                                  (lambda: [T.plan_and_pack(ps, workers=2)[0]], 300, 1)):
+        got = []
+        th = threading.Thread(target=lambda: got.extend(plan()), daemon=True)
+        th.start()
+        th.join(120)
+        stuck = th.is_alive()
+        if stuck:                        # a writer blocked on a full pipe holds its lock: closing the pipe would hang too
+            for proc in T._POOL.procs:
+                proc.kill()
+        T.shutdown_pool()
+        assert not stuck and len(got) == slices and sum(len(t.post) for t in got) == renders

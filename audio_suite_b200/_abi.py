@@ -123,6 +123,10 @@ class ExportRender(C.Structure):
                 ("rate", C.c_int32 * 4)]             # up, down, half, taps per phase
 
 
+class PcmRender(C.Structure):
+    _fields_ = [("key", C.c_uint32 * 2), ("fmt", C.c_int32 * 2)]            # Philox key; bits, dither
+
+
 _P, _I, _Z = C.c_void_p, C.c_int, C.c_size_t
 _COMMON = {
     "ms_version": (C.c_int, []),
@@ -165,6 +169,7 @@ _STAGES = {
     "ms_fir_destroy": (None, [_P]),
     "ms_post": (_I, [_P, _I, _I, _P, _P, _P, _P]),
     "ms_post_export": (_I, [_P, _P, _I, _I, _I, _P, _P, _P, _P, _P]),
+    "ms_post_pcm": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "ms_roll": (_I, [_P, _P, _I, _I, _P]),
     "ms_polyphase_decimate": (_I, [_P, C.c_int64, _I, _I, _P, _I, _I, _P, C.c_int64, _P]),
 }

@@ -122,7 +122,8 @@ enum { F_base_sr, F_out_dur_s, F_time_unfold, F_peak, F_sat_drive, F_stereo_on, 
        F_mb_b1, F_mb_b2, F_mb_b3, F_mb_u1, F_mb_u2, F_mb_u3, F_mb_roll, F_bandlimit_on, F_bandlimit_out_hz, F_bandlimit_roll_hz,
        F_event_process, F_grains_per_sec, F_max_grains, F_grain_amp_rand, F_grain_offset_on, F_grain_offset_max_ms,
        F_lane_density, F_lane_unfold, F_lane_cutoff, F_lane_stretch, F_er_cloud_on, F_er_taps, F_er_max_ms, F_space_ir_on, F_ir_id,
-       F_ir_r_id, F_env_a, F_env_d, F_env_s, F_env_r, F_env_curve, F_bessel_id, F_export_sr, F_COUNT };
+       F_ir_r_id, F_env_a, F_env_d, F_env_s, F_env_r, F_env_curve, F_bessel_id, F_export_sr,
+       F_export_bits, F_export_dither, F_COUNT };
 enum { MODE_GAUSS = 0, MODE_DUST = 1, MODE_NOISE = 2, MODE_SKEW = 3, MODE_RES = 4, MODE_PLAIN = 5 };
 
 struct Lanes { const int64_t* ptr; const double* t; const double* v; };
@@ -189,6 +190,8 @@ struct Plan {
     std::vector<int64_t> out_at, out_n, y_at, last, srs, ir_order;
     std::vector<ms_export_render> exp;              // renders with export_sr: resampler rows ...
     std::vector<int64_t> export_of, ratios, bank_at; // ... their render indices; distinct (up, down) in order of first use
+    std::vector<ms_pcm_render> pcm;                 // renders with export_format: PCM rows ...
+    std::vector<int64_t> pcm_of;                    // ... their render indices
     int64_t pool_n, mono_n, frames, h_total, max_h, max_out_n, env_n, n_ir, n_bank;
     int64_t alg[7];                                 // synth, tilt_spectral, grain_spectral, overlap_add, fir_in, fir_taps, post
     std::string error; int error_render;
@@ -203,10 +206,12 @@ static bool same_env(const EnvKey& k, const EnvKey& o) {
 struct Scal {
     std::vector<int64_t> mono_at, fir_of, fir_r_of, st_dl, st_dr;      // fir_r_of: the right channel's row (space_ir_stereo), or -1
     std::vector<int64_t> ex_up, ex_down;                                 // export_sr as up / down in lowest terms (0: none)
+    std::vector<int64_t> pcm_bits, pcm_dither;                           // export_format as bits (0: float32), export_dither
+    std::vector<uint64_t> seed;
     std::vector<int> stereo_on, bessel_id;
     std::vector<double> st_theta, drive, peak;
     void resize(size_t n) {
-        ex_up.assign(n, 0); ex_down.assign(n, 0);
+        ex_up.assign(n, 0); ex_down.assign(n, 0); pcm_bits.assign(n, 0); pcm_dither.assign(n, 0); seed.assign(n, 0);
         mono_at.resize(n); fir_of.assign(n, -1); fir_r_of.assign(n, -1); st_dl.resize(n); st_dr.resize(n); stereo_on.resize(n); bessel_id.resize(n);
         st_theta.resize(n); drive.resize(n); peak.resize(n);
     }
@@ -461,6 +466,8 @@ static int plan_range(Plan& P, Scal& SC, const double* rows, int r0, int r1, con
         drive[r] = p[F_sat_drive]; peak[r] = p[F_peak]; bessel_id[r] = (int)p[F_bessel_id];
         const long long ex_sr = (long long)p[F_export_sr];          // validated by plan.export_ratio; 0: none
         if (ex_sr > 0) { const long long g = std::gcd(base_sr, ex_sr); SC.ex_up[r] = ex_sr / g; SC.ex_down[r] = base_sr / g; }
+        SC.pcm_bits[r] = (int64_t)p[F_export_bits]; SC.pcm_dither[r] = (int64_t)p[F_export_dither];      // validated by plan.pcm_format
+        SC.seed[r] = (uint64_t)seed;
         P.out_n[r] = n_out;
     }
     return 0;
@@ -512,6 +519,7 @@ static void append_part(Plan& P, Scal& S, const Plan& Q, const Scal& QS, std::ve
     append(S.stereo_on, QS.stereo_on); append(S.st_dl, QS.st_dl); append(S.st_dr, QS.st_dr); append(S.st_theta, QS.st_theta);
     append(S.drive, QS.drive); append(S.peak, QS.peak); append(S.bessel_id, QS.bessel_id);
     append(S.ex_up, QS.ex_up); append(S.ex_down, QS.ex_down);
+    append(S.pcm_bits, QS.pcm_bits); append(S.pcm_dither, QS.pcm_dither); append(S.seed, QS.seed);
     P.pool_n += Q.pool_n; P.mono_n += Q.mono_n; P.h_total += Q.h_total;
     P.max_h = std::max(P.max_h, Q.max_h); P.max_out_n = std::max(P.max_out_n, Q.max_out_n);
     for (int k = 0; k < 7; ++k) P.alg[k] += Q.alg[k];
@@ -587,8 +595,17 @@ static void finish_plan(Plan& P, const Scal& S, const double* bessel, int n_coef
             e.rate[0] = (int32_t)up; e.rate[1] = (int32_t)down; e.rate[2] = (int32_t)half; e.rate[3] = (int32_t)taps;
             P.exp.push_back(e); P.export_of.push_back(r);
         }
+        // export_format: the frames are stored as PCM bytes in ceil(n_x / 2) (16 bits) or ceil(3 n_x / 4) (24 bits) slots
+        int64_t slots = n_x;
+        if (S.pcm_bits[r] > 0) {
+            ms_pcm_render q;
+            q.key[0] = (uint32_t)S.seed[r]; q.key[1] = (uint32_t)(S.seed[r] >> 32);
+            q.fmt[0] = (int32_t)S.pcm_bits[r]; q.fmt[1] = (int32_t)S.pcm_dither[r];
+            P.pcm.push_back(q); P.pcm_of.push_back(r);
+            slots = q.fmt[0] == 16 ? (n_x + 1) / 2 : (3 * n_x + 3) / 4;
+        }
         P.out_at[r] = P.frames; P.y_at[r] = y;
-        P.frames += n_x;
+        P.frames += slots;
         P.out_n[r] = n_x;
         P.alg[6] += n;
     }
@@ -673,7 +690,7 @@ void* ms_hp_plan(const double* rows, int n_renders, const int64_t* lane_ptr, con
 const char* ms_hp_error(void* h, int* render) { Plan* P = (Plan*)h; *render = P->error_render; return P->error.c_str(); }
 // sizes: element counts of every exported array, in the order of ms_hp_export
 enum { HP_SY, HP_OLA_R, HP_ENV_REPS, HP_OLA_E, HP_FIR, HP_POST, HP_TAPS, HP_DUST, HP_TILT, HP_GRAIN, HP_ROT, HP_ODD, HP_IRS, HP_EXPORT,
-       HP_RATIOS, HP_NSIZES };
+       HP_RATIOS, HP_PCM, HP_NSIZES };
 void ms_hp_sizes(void* h, int64_t* sizes, int64_t* scalars /*pool_n mono_n frames h_total max_h max_out_n env_n, alg[7]*/) {
     Plan* P = (Plan*)h;
     sizes[HP_SY] = (int64_t)P->sy1.size(); sizes[HP_OLA_R] = (int64_t)P->ola_r.size(); sizes[HP_ENV_REPS] = (int64_t)P->env_reps.size();
@@ -681,6 +698,7 @@ void ms_hp_sizes(void* h, int64_t* sizes, int64_t* scalars /*pool_n mono_n frame
     sizes[HP_TAPS] = (int64_t)P->tap_off.size(); sizes[HP_DUST] = (int64_t)P->dust_pos.size(); sizes[HP_TILT] = (int64_t)P->tilt.size();
     sizes[HP_GRAIN] = (int64_t)P->grain.size(); sizes[HP_ROT] = (int64_t)P->rot.size(); sizes[HP_ODD] = (int64_t)P->odd.size() / 4;
     sizes[HP_IRS] = (int64_t)P->ir_order.size(); sizes[HP_EXPORT] = (int64_t)P->exp.size(); sizes[HP_RATIOS] = (int64_t)P->bank_at.size();
+    sizes[HP_PCM] = (int64_t)P->pcm.size();
     scalars[0] = P->pool_n; scalars[1] = P->mono_n; scalars[2] = P->frames; scalars[3] = P->h_total; scalars[4] = P->max_h;
     scalars[5] = P->max_out_n; scalars[6] = P->env_n;
     for (int i = 0; i < 7; ++i) scalars[7 + i] = P->alg[i];
@@ -689,7 +707,7 @@ void ms_hp_export(void* h, void* sy1, void* sy2, void* ola_r, void* env_reps, vo
                   int32_t* tap_off, double* tap_delay, double* tap_raw, int32_t* dust_pos, double* dust_val,
                   void* tilt, void* grain, void* rot,
                   int64_t* odd, int64_t* ir_order, int64_t* out_at, int64_t* out_n, int64_t* y_at, int64_t* last, int64_t* srs,
-                  void* exp, int64_t* export_of, int64_t* ratios) {
+                  void* exp, int64_t* export_of, int64_t* ratios, void* pcm, int64_t* pcm_of) {
     Plan* P = (Plan*)h;
     auto cp = [](void* d, const void* s, size_t b) { if (b) memcpy(d, s, b); };
     cp(sy1, P->sy1.data(), P->sy1.size() * sizeof(ms_synth_evt)); cp(sy2, P->sy2.data(), P->sy2.size() * sizeof(ms_synth_evt));
@@ -705,6 +723,7 @@ void ms_hp_export(void* h, void* sy1, void* sy2, void* ola_r, void* env_reps, vo
     cp(last, P->last.data(), P->last.size() * 8); cp(srs, P->srs.data(), P->srs.size() * 8);
     cp(exp, P->exp.data(), P->exp.size() * sizeof(ms_export_render)); cp(export_of, P->export_of.data(), P->export_of.size() * 8);
     cp(ratios, P->ratios.data(), P->ratios.size() * 8);
+    cp(pcm, P->pcm.data(), P->pcm.size() * sizeof(ms_pcm_render)); cp(pcm_of, P->pcm_of.data(), P->pcm_of.size() * 8);
 }
 void ms_hp_free(void* h) { delete (Plan*)h; }
 }

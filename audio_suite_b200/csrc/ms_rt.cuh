@@ -27,6 +27,7 @@
   static inline float2 __ldg(const float2* p) { return *p; }
   static inline int __ldg(const int* p) { return *p; }
   static inline float __fmaf_rn(float a, float b, float c) { return std::fma(a, b, c); }
+  static inline unsigned int __umulhi(unsigned int a, unsigned int b) { return (unsigned int)(((unsigned long long)a * b) >> 32); }
   static inline double cospi(double a) { return std::cos(M_PI * a); }
   namespace msemu { void yield_barrier(); void yield_warp_barrier(); }
   struct Ctx {

@@ -229,9 +229,60 @@ MS_DEV void post_max_body(const PostRender* MS_RESTRICT renders, real* mono, uns
 #endif
     }
 }
+// ---- EXTENSION: integer PCM output (include/microsound_b200.h, ms_post_pcm) ----
+// The write passes below take the store as a compile-time policy: BITS 0 stores float2 frames (ms_post, ms_post_export:
+// the code they always had), BITS 16 / 24 store PCM, with DITHER on or off (the dither-off passes hold no Philox code).
+typedef ms_pcm_render PcmRender;
+#define PCM_TILE_BYTES (6 * OLA_TILE)        // pcm24: one tile of 1024 frames staged in shared memory
+// Philox4x32-10 (Salmon et al., SC'11; Random123's philox4x32 with 10 rounds): the counter c becomes the output words
+MS_DEV void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        if (r) { k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
+        c[0] = hi1 ^ c[1] ^ k0; c[1] = lo1; c[2] = hi0 ^ c[3] ^ k1; c[3] = lo0;
+    }
+}
+// q = clamp(rint(x S + d), -S, S - 1), S = 2^(BITS - 1), in double: x S is exact, so there is one rounding
+template <int BITS> MS_DEV int pcm_quant(double x, double d) {
+    const double S = (double)(1 << (BITS - 1));
+    return (int)fmin(fmax(rint(x * S + d), -S), S - 1.0);
+}
+// output frame i of a PCM render of n frames: dither, quantise, store (pcm16: one 32-bit word per frame at o; pcm24: 6 bytes
+// at slot j of the staged tile, written as three 16-bit halves)
+template <int BITS, bool DITHER>
+MS_DEV void pcm_frame(const PcmRender& P, long long n, long long i, double l, double r, unsigned char* o, char* stage, int j) {
+    double dl = 0.0, dr = 0.0;
+    if (DITHER) {
+        uint32_t w[4] = {(uint32_t)i, (uint32_t)((unsigned long long)i >> 32), 0x64697468u, 0u};
+        philox4x32_10(w, P.key[0], P.key[1]);
+        dl = ((double)w[0] - (double)w[1]) * 2.3283064365386963e-10;     // 2^-32: exact, triangular on (-1, 1)
+        dr = ((double)w[2] - (double)w[3]) * 2.3283064365386963e-10;
+    }
+    const uint32_t ql = (uint32_t)pcm_quant<BITS>(l, dl), qr = (uint32_t)pcm_quant<BITS>(r, dr);
+    if (BITS == 16) {
+        ((uint32_t*)o)[i] = (ql & 0xffffu) | (qr << 16);
+        if (i == n - 1 && (n & 1)) ((uint32_t*)o)[i + 1] = 0u;                      // the rest of the last slot
+    } else {
+        unsigned short* s = (unsigned short*)(stage + 6 * j);
+        s[0] = (unsigned short)ql; s[1] = (unsigned short)(((ql >> 16) & 0xffu) | ((qr & 0xffu) << 8)); s[2] = (unsigned short)(qr >> 8);
+    }
+}
+// pcm24: the staged tile of cnt frames, from frame f0 (a multiple of OLA_TILE, so byte 6 f0 is 8-aligned), as 8-byte words;
+// the last word's bytes past the tile are zero (they lie in the render's own last slot)
+MS_DEV void pcm24_flush(char* stage, unsigned char* o, long long f0, int cnt, const Ctx& c) {
+    const int nb = 6 * cnt, nw = (nb + 7) >> 3;
+    if (c.tid < 8 * nw - nb) stage[nb + c.tid] = 0;
+    c.sync();
+    unsigned long long* d = (unsigned long long*)(o + 6 * f0);
+    const unsigned long long* s = (const unsigned long long*)stage;
+    for (int w = c.tid; w < nw; w += c.nthr) d[w] = s[w];
+}
 // pass 2: write interleaved stereo, clipped and scaled to the requested peak (modes 1-3 read the right channel at rbuf)
-MS_DEV void post_write_body(const PostRender* MS_RESTRICT renders, const real* MS_RESTRICT mono, const unsigned long long* MS_RESTRICT maxbits,
-                            float2* MS_RESTRICT out, const Ctx& c) {
+template <int BITS, bool DITHER>
+MS_DEV void post_write_body(const PostRender* MS_RESTRICT renders, const PcmRender* MS_RESTRICT pcms, const real* MS_RESTRICT mono,
+                            const unsigned long long* MS_RESTRICT maxbits, float2* MS_RESTRICT out, const Ctx& c) {
     const PostRender& R = renders[c.by];
     const int t0 = c.bx * OLA_TILE;
     if (t0 >= R.n) return;
@@ -253,10 +304,23 @@ MS_DEV void post_write_body(const PostRender* MS_RESTRICT renders, const real* M
         lv[q] = i < t1 ? y[li] : (real)0.;
         rv[q] = i < t1 ? rsrc[i] : (real)0.;
     }
+    if constexpr (BITS == 0) {
 #pragma unroll
-    for (int q = 0; q < OLA_TILE / OLA_NTHR; ++q) {
-        const int i = t0 + c.tid + OLA_NTHR * q;
-        if (i < t1) o[i] = make_float2((float)(soft_clip(lv[q], drive, inv_t) * scale), (float)(soft_clip(rv[q], drive, inv_t) * scale));
+        for (int q = 0; q < OLA_TILE / OLA_NTHR; ++q) {
+            const int i = t0 + c.tid + OLA_NTHR * q;
+            if (i < t1) o[i] = make_float2((float)(soft_clip(lv[q], drive, inv_t) * scale), (float)(soft_clip(rv[q], drive, inv_t) * scale));
+        }
+    } else {
+        const PcmRender P = pcms[c.by];
+        if (P.fmt[0] != BITS || P.fmt[1] != (DITHER ? 1 : 0)) return;
+        unsigned char* ob = (unsigned char*)o;
+#pragma unroll
+        for (int q = 0; q < OLA_TILE / OLA_NTHR; ++q) {
+            const int i = t0 + c.tid + OLA_NTHR * q;
+            if (i < t1) pcm_frame<BITS, DITHER>(P, R.n, i, (double)(soft_clip(lv[q], drive, inv_t) * scale), (double)(soft_clip(rv[q], drive, inv_t) * scale),
+                                                ob, c.smem, i - t0);
+        }
+        if (BITS == 24) pcm24_flush(c.smem, ob, t0, t1 - t0, c);
     }
 }
 // ---- EXTENSION: export sample rate, the write pass of an exporting render (include/microsound_b200.h, ms_post_export) ----
@@ -270,9 +334,10 @@ MS_DEV void post_write_body(const PostRender* MS_RESTRICT renders, const real* M
 typedef ms_export_render ExportRender;
 #define EXP_TILE 1024                // output frames per CTA
 #define EXP_CH 2048                  // input frames per round of the staged window
-MS_DEV void post_export_body(const PostRender* MS_RESTRICT renders, const ExportRender* MS_RESTRICT exps, const real* MS_RESTRICT mono,
-                             const unsigned long long* MS_RESTRICT maxbits, const real* MS_RESTRICT bank, float2* MS_RESTRICT out,
-                             const Ctx& c) {
+template <int BITS, bool DITHER>
+MS_DEV void post_export_body(const PostRender* MS_RESTRICT renders, const ExportRender* MS_RESTRICT exps, const PcmRender* MS_RESTRICT pcms,
+                             const real* MS_RESTRICT mono, const unsigned long long* MS_RESTRICT maxbits, const real* MS_RESTRICT bank,
+                             float2* MS_RESTRICT out, const Ctx& c) {
     const PostRender& R = renders[c.by];
     const ExportRender E = exps[c.by];
     const long long out_n = E.out_end - E.out;
@@ -342,10 +407,22 @@ MS_DEV void post_export_body(const PostRender* MS_RESTRICT renders, const Export
             aL[k] = l; aR[k] = r;
         }
     }
-    float2* o = out + E.out + m0;
+    if constexpr (BITS == 0) {
+        float2* o = out + E.out + m0;
 #pragma unroll
-    for (int k = 0; k < NQ; ++k)
-        if (rq[k] >= 0) o[c.tid + OLA_NTHR * k] = make_float2((float)aL[k], (float)aR[k]);
+        for (int k = 0; k < NQ; ++k)
+            if (rq[k] >= 0) o[c.tid + OLA_NTHR * k] = make_float2((float)aL[k], (float)aR[k]);
+    } else {
+        // the dither is drawn here, after the accumulation: its registers do not compete with the tap loop's
+        const PcmRender P = pcms[c.by];
+        if (P.fmt[0] != BITS || P.fmt[1] != (DITHER ? 1 : 0)) return;
+        unsigned char* ob = (unsigned char*)(out + E.out);
+        if (BITS == 24) c.sync();                // the staged window is read by every thread: its space becomes the tile's
+#pragma unroll
+        for (int k = 0; k < NQ; ++k)
+            if (rq[k] >= 0) pcm_frame<BITS, DITHER>(P, out_n, m0 + c.tid + OLA_NTHR * k, (double)aL[k], (double)aR[k], ob, c.smem, c.tid + OLA_NTHR * k);
+        if (BITS == 24) pcm24_flush(c.smem, ob, m0, cnt, c);
+    }
 }
 // circular shift used by the odd-length stereo path: dst[i] = src[(i + shift) mod n]
 MS_DEV void roll_body(const real* MS_RESTRICT src, real* MS_RESTRICT dst, int n, int shift, const Ctx& c) {

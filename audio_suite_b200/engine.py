@@ -14,6 +14,7 @@ Stage order (one batched launch sequence for all renders):
   reflection cloud (+) impulse response as one FIR, overlap-save ms_fir_*
   stereo diffusion, soft clip, normalise                         ms_post
   [... and for renders with `export_sr`: resampled to that rate]  ms_post_export
+  [... and for renders with `export_format`: stored as PCM]       ms_post_pcm
 """
 from __future__ import annotations
 
@@ -261,18 +262,38 @@ class BatchRenderer:
         self.n_env = len(t.env_reps)
         self.envpool = dev.empty(max(1, t.env_n), real)
         self.d_env_reps = dev.upload(t.env_reps) if self.n_env else None
-        # export_sr: the renders that have one run ms_post_export instead of ms_post, on the maxbits after the plain ones
-        self.n_export = len(t.export)
-        if self.n_export:
-            exporting = np.zeros(self.n_renders, bool)
-            exporting[t.export_of] = True
-            plain = t.post[~exporting]
+        # export_sr: the renders that have one run ms_post_export instead of ms_post, on the maxbits after the plain ones;
+        # export_format: PCM renders run ms_post_pcm after those, one call per (bits, dither, exporting) group
+        self.n_export, self.n_pcm = len(t.export), len(t.pcm)
+        self.pcm_groups = []
+        if self.n_export or self.n_pcm:
+            is_pcm = np.zeros(self.n_renders, bool)
+            is_pcm[t.pcm_of] = True
+            ex_row = np.full(self.n_renders, -1, np.int64)
+            ex_row[t.export_of] = np.arange(self.n_export)
+            plain = t.post[~is_pcm & (ex_row < 0)]
             self.n_plain, self.max_n_plain = len(plain), int(plain["n"].max()) if len(plain) else 0
             self.d_post = dev.upload(plain) if len(plain) else None
-            self.d_post_export, self.d_export = dev.upload(t.post[t.export_of]), dev.upload(t.export)
-            self.d_bank = dev.upload(t.bank.astype(real))
-            self.max_n_export = int(t.post["n"][t.export_of].max())
-            self.max_out_export = int((t.export["out_end"] - t.export["out"]).max())
+            fexp = np.flatnonzero(~is_pcm & (ex_row >= 0))
+            self.n_float_export = len(fexp)
+            if self.n_export:
+                self.d_bank = dev.upload(t.bank.astype(real))
+            if len(fexp):
+                e = t.export[ex_row[fexp]]
+                self.d_post_export, self.d_export = dev.upload(t.post[fexp]), dev.upload(e)
+                self.max_n_export = int(t.post["n"][fexp].max())
+                self.max_out_export = int((e["out_end"] - e["out"]).max())
+            mb = self.n_plain + len(fexp)
+            exporting, bits, dither = ex_row[t.pcm_of] >= 0, t.pcm["fmt"][:, 0], t.pcm["fmt"][:, 1]
+            for key in sorted(set(zip(exporting.tolist(), bits.tolist(), dither.tolist()))):
+                sel = (exporting == key[0]) & (bits == key[1]) & (dither == key[2])
+                rows = t.pcm_of[sel]
+                e = t.export[ex_row[rows]] if key[0] else None
+                self.pcm_groups.append(dict(
+                    n=len(rows), mb=mb, bits=key[1], dither=key[2], d_post=dev.upload(t.post[rows]), d_pcm=dev.upload(t.pcm[sel]),
+                    d_export=dev.upload(e) if key[0] else None, max_n=int(t.post["n"][rows].max()),
+                    max_out=int((e["out_end"] - e["out"]).max()) if key[0] else 0))
+                mb += len(rows)
         else:
             self.d_post = dev.upload(t.post)
         if self.any_dust:
@@ -472,16 +493,23 @@ class BatchRenderer:
             for (y_at, scratch, n, dr) in self.tables.odd.tolist():
                 _check(dev, lib.ms_roll(C.c_void_p(base + isz * y_at), C.c_void_p(base + isz * scratch), n, dr, st))
             self.rot_stage.run()
-        if not self.n_export:
+        if not self.n_export and not self.n_pcm:
             _check(dev, lib.ms_post(dev.ptr(self.d_post), self.n_renders, self.max_out_n, dev.ptr(self.mono),
                                     dev.ptr(self.maxbits), dev.ptr(self.out), st))
         else:
             if self.n_plain:
                 _check(dev, lib.ms_post(dev.ptr(self.d_post), self.n_plain, self.max_n_plain, dev.ptr(self.mono),
                                         dev.ptr(self.maxbits), dev.ptr(self.out), st))
-            mb = C.c_void_p(dev.ptr(self.maxbits).value + 8 * self.n_plain)
-            _check(dev, lib.ms_post_export(dev.ptr(self.d_post_export), dev.ptr(self.d_export), self.n_export, self.max_n_export,
-                                           self.max_out_export, dev.ptr(self.mono), mb, dev.ptr(self.d_bank), dev.ptr(self.out), st))
+            if self.n_float_export:
+                mb = C.c_void_p(dev.ptr(self.maxbits).value + 8 * self.n_plain)
+                _check(dev, lib.ms_post_export(dev.ptr(self.d_post_export), dev.ptr(self.d_export), self.n_float_export,
+                                               self.max_n_export, self.max_out_export, dev.ptr(self.mono), mb, dev.ptr(self.d_bank),
+                                               dev.ptr(self.out), st))
+            for g in self.pcm_groups:
+                mb = C.c_void_p(dev.ptr(self.maxbits).value + 8 * g["mb"])
+                _check(dev, lib.ms_post_pcm(dev.ptr(g["d_post"]), dev.ptr(g["d_pcm"]), dev.ptr(g["d_export"]) if g["d_export"] is not None else None,
+                                            g["n"], g["max_n"], g["max_out"], g["bits"], g["dither"], dev.ptr(self.mono), mb,
+                                            dev.ptr(self.d_bank) if self.n_export else None, dev.ptr(self.out), st))
         mark("post")
 
     # ---- CUDA graph ------------------------------------------------------------------------------------
@@ -512,10 +540,17 @@ class BatchRenderer:
         self.graph.replay()
 
     # ---- results ---------------------------------------------------------------------------------------
+    def pcm_bits(self, r):
+        """16 or 24 when render r has `export_format` "pcm16" / "pcm24", else None."""
+        at = np.flatnonzero(self.tables.pcm_of == r)
+        return int(self.tables.pcm["fmt"][at[0], 0]) if at.size else None
+
     def output(self, r):
-        """float32 [out_n, 2] of render r (host copy; out_n frames at its export rate, if any)."""
-        n = int(self.tables.out_n[r])
-        return self.dev.download(self.out, 2 * int(self.tables.out_at[r]), 2 * n).reshape(n, 2)
+        """float32 [out_n, 2] of render r (host copy; out_n frames at its export rate, if any); with `export_format`, int16
+        [out_n, 2] (pcm16) or uint8 [out_n, 6] (pcm24) -- pcm_frames."""
+        n, bits = int(self.tables.out_n[r]), self.pcm_bits(r)
+        a = np.asarray(self.dev.download(self.out, 2 * int(self.tables.out_at[r]), 2 * P.output_slots(n, bits)))
+        return a.reshape(n, 2) if bits is None else pcm_frames(a.view(np.uint8), n, bits)
 
     def output_f64(self, r):
         """float64 [out_n, 2] of render r -- the float32 samples widened ON THE DEVICE (exact), as the reference returns them
@@ -604,7 +639,7 @@ def render(params, progress=None, device=None, precision="auto", cache=True):
         for ev in rp.events:
             if ev.placed and ev.index % 50 == 0:
                 progress(int(5 + 70 * (ev.index / max(1, n_evt))), f"Events {ev.index}/{n_evt}  {ev.note}".strip())      # M:758
-    audio = br.output_f64(0)
+    audio = br.output_f64(0) if not br.n_pcm else br.output(0)
     meta = br.meta(0)
     if key is not None and br.tables.frames <= _CACHE_MAX_FRAMES:
         _RENDER_CACHE[key] = (br, uses + 1)                            # most recent last
@@ -616,6 +651,12 @@ def render(params, progress=None, device=None, precision="auto", cache=True):
     if progress:
         progress(100, "Done.")
     return audio, meta
+
+
+def pcm_frames(buf, n, bits):
+    """The n frames of a PCM render from the bytes of its slots (a uint8 array starting at its first slot): int16 [n, 2]
+    for 16 bits, uint8 [n, 6] for 24 (each row L, R as three little-endian bytes of two's complement) -- views of `buf`."""
+    return buf[:4 * n].view(np.int16).reshape(n, 2) if bits == 16 else buf[:6 * n].reshape(n, 6)
 
 
 def _prefetch(gen, depth=2):
@@ -669,7 +710,9 @@ def _render_batch(params_list, device=None, precision="auto", host_out=None, chu
     integer segment maps) while the GPU renders slice k and slice k-1 drains to host memory on a copy
     stream, so planning, kernels and the device->host transfer overlap.  Returns a list of float32
     [out_n, 2] arrays, one per render, in order -- views into `host_out` (a pinned 1-D float32 torch tensor
-    of at least 2 * total frames) when it is given, else into a pinned buffer allocated here."""
+    of at least 2 * total frames) when it is given, else into a pinned buffer allocated here.  A render with
+    `export_format` takes ceil(out_n / 2) (pcm16) or ceil(3 out_n / 4) (pcm24) of those frames, and its array is
+    an int16 [out_n, 2] or uint8 [out_n, 6] view of their bytes (pcm_frames)."""
     from collections import deque
     import os as _os, time as _time
     from . import tables as T
@@ -696,16 +739,18 @@ def _render_batch(params_list, device=None, precision="auto", host_out=None, chu
             br.close()
         return outs
     torch = dev.torch
-    # frames of the whole batch (main_v2.py:590; at the export rate of renders with `export_sr`), memoised per distinct
-    # (duration, rate, export rate): a sweep repeats a few values
+    # frames of the whole batch (main_v2.py:590; at the export rate of renders with `export_sr`; in 8-byte slots, one
+    # float32 frame each, for renders with `export_format`), memoised per distinct (duration, rate, export rate, format):
+    # a sweep repeats a few values
     import operator
     frames_of, get_dur = {}, operator.itemgetter("out_dur_s", "base_sr")
     total = 0
     for p in params_list:
-        key = get_dur(p) + (p.get("export_sr"),)
+        pcm = P.pcm_format(p)
+        key = get_dur(p) + (p.get("export_sr"), None if pcm is None else pcm[0])
         f = frames_of.get(key)
         if f is None:
-            f = frames_of[key] = P.export_frames(int(max(1, round(float(key[0]) * int(key[1])))), P.export_ratio(p))
+            f = frames_of[key] = P.output_slots(P.export_frames(int(max(1, round(float(key[0]) * int(key[1])))), P.export_ratio(p)), key[3])
         total += f
     if host_out is None:
         host_out = torch.empty(2 * total, dtype=torch.float32).pin_memory()
@@ -737,8 +782,11 @@ def _render_batch(params_list, device=None, precision="auto", host_out=None, chu
             host_out[at:at + 2 * tb.frames].copy_(br.out[:2 * tb.frames], non_blocking=True)
             drained = torch.cuda.Event()
             drained.record(copy)
-        for a, n in zip(tb.out_at.tolist(), tb.out_n.tolist()):
-            views.append((at + 2 * a, n))
+        bits = [None] * len(tb.out_n)
+        for r, b in zip(tb.pcm_of.tolist(), tb.pcm["fmt"][:, 0].tolist()):
+            bits[r] = b
+        for a, n, b in zip(tb.out_at.tolist(), tb.out_n.tolist(), bits):
+            views.append((at + 2 * a, n, b))
         at += 2 * tb.frames
         live.append((br, drained))
         t_enq = _time.perf_counter()
@@ -760,4 +808,6 @@ def _render_batch(params_list, device=None, precision="auto", host_out=None, chu
         import sys as _sys
         print("\n".join(trace) + "\n  drained at t=%.1f ms" % (1e3 * (_time.perf_counter() - t_start)), file=_sys.stderr, flush=True)
     flat = host_out.numpy()
-    return [flat[a:a + 2 * n].reshape(n, 2) for a, n in views]
+    raw, i16 = flat.view(np.uint8), flat.view(np.int16)             # (pcm_frames' views, in two numpy calls per render)
+    return [flat[a:a + 2 * n].reshape(n, 2) if b is None else i16[2 * a:2 * a + 2 * n].reshape(n, 2) if b == 16
+            else raw[4 * a:4 * a + 6 * n].reshape(n, 6) for a, n, b in views]

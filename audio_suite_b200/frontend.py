@@ -135,9 +135,27 @@ def write_wav_float32(path, audio, sample_rate):
         f.write(b"RIFF" + struct.pack("<I", len(body)) + body)
 
 
+def write_wav_pcm(path, data, sample_rate):
+    """RIFF/WAVE, WAVE_FORMAT_PCM, stereo, from what a render with `export_format` returns: int16 [n, 2] is written as 16 bit,
+    uint8 [n, 6] (L, R as three little-endian bytes each) as 24 bit -- the bytes as they are."""
+    a = np.asarray(data)
+    if a.dtype == np.int16 and a.ndim == 2 and a.shape[1] == 2:
+        bits, data_bytes = 16, np.ascontiguousarray(a, dtype="<i2").tobytes()
+    elif a.dtype == np.uint8 and a.ndim == 2 and a.shape[1] == 6:
+        bits, data_bytes = 24, np.ascontiguousarray(a).tobytes()
+    else:
+        raise ValueError(f"write_wav_pcm takes int16 [n, 2] or uint8 [n, 6], not {a.dtype} {a.shape}")
+    ch, block = 2, 2 * bits // 8
+    fmt = struct.pack("<HHIIHH", 1, ch, int(sample_rate), int(sample_rate) * block, block, bits)
+    body = b"WAVE" + b"fmt " + struct.pack("<I", len(fmt)) + fmt + b"data" + struct.pack("<I", len(data_bytes)) + data_bytes
+    with open(path, "wb") as f:
+        f.write(b"RIFF" + struct.pack("<I", len(body)) + body)
+
+
 def batch_render(base_params, seeds, unfolds, stretches, folder, device=None, precision="auto", progress=None):
     """The batch dialog's sweep (main_v2.py:1524-1593) through the streamed GPU batch: returns [(reference name, path)].
-    With `export_sr` in the parameters the files are written, and named, at that rate.
+    With `export_sr` in the parameters the files are written, and named, at that rate; with `export_format` "pcm16" /
+    "pcm24" they are 16- / 24-bit PCM files (write_wav_pcm), else 32-bit float.
     `progress(done, total, name)` mirrors the dialog's progress bar / status line."""
     from . import engine
     plist = batch_params(base_params, seeds, unfolds, stretches)
@@ -148,7 +166,10 @@ def batch_render(base_params, seeds, unfolds, stretches, folder, device=None, pr
         out_sr = int(p["base_sr"]) if export_ratio(p) is None else int(p["export_sr"])      # the optional key `export_sr`
         name = batch_name(p["seed"], p["time_unfold"], p["partial_stretch"], out_sr)
         path = os.path.join(folder, name + ".wav")
-        write_wav_float32(path, audio, out_sr)
+        if audio.dtype == np.float32:
+            write_wav_float32(path, audio, out_sr)
+        else:
+            write_wav_pcm(path, audio, out_sr)
         written.append((name, path))
         if progress:
             progress(i + 1, total, name)

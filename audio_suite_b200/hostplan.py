@@ -24,11 +24,12 @@ FIELDS = ("base_sr", "out_dur_s", "time_unfold", "peak", "sat_drive", "stereo_on
           "mb_b1", "mb_b2", "mb_b3", "mb_u1", "mb_u2", "mb_u3", "mb_roll", "bandlimit_on", "bandlimit_out_hz", "bandlimit_roll_hz",
           "event_process", "grains_per_sec", "max_grains", "grain_amp_rand", "grain_offset_on", "grain_offset_max_ms",
           "bp_density", "bp_unfold", "bp_cutoff", "bp_stretch", "er_cloud_on", "er_taps", "er_max_ms", "space_ir_on", "_ir",
-          "_ir_r", "env_a", "env_d", "env_s", "env_r", "env_curve", "_bessel", "export_sr")
+          "_ir_r", "env_a", "env_d", "env_s", "env_r", "env_curve", "_bessel", "export_sr",
+          "export_format", "export_dither")
 _MODE = {m: float(i) for i, m in enumerate(BASIC_MODES)}
 _PROCESS = {"Single": 0.0, "Poisson": 1.0}
 _OFF_FLAGS = ("partial_lock_on", "cep_warp_on", "res_bank_on", "wg_on", "event_feedback_on", "spectral_imprint_on")
-_HP_NAMES = ("sy1", "ola_r", "env_reps", "ola_e", "fir", "post", "tap_off", "dust_pos", "tilt", "grain", "rot", "odd", "irs", "export", "ratios")   # ms_hp_sizes
+_HP_NAMES = ("sy1", "ola_r", "env_reps", "ola_e", "fir", "post", "tap_off", "dust_pos", "tilt", "grain", "rot", "odd", "irs", "export", "ratios", "pcm")   # ms_hp_sizes
 
 _lib = None
 
@@ -47,7 +48,7 @@ def lib():
             l.ms_hp_error.restype = C.c_char_p
             l.ms_hp_error.argtypes = [C.c_void_p, C.POINTER(C.c_int)]
             l.ms_hp_sizes.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
-            l.ms_hp_export.argtypes = [C.c_void_p] * 26
+            l.ms_hp_export.argtypes = [C.c_void_p] * 28
             l.ms_hp_free.argtypes = [C.c_void_p]
             l.ms_hp_pcg64_seed.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
             l.ms_hp_draws.argtypes = [C.c_int64, C.c_int, C.c_uint64, C.c_int, C.c_void_p]
@@ -148,6 +149,7 @@ def _marshal(params_list):
     # the non-numeric fields: one small tuple per render; a sweep repeats the same strings / IR object, so the converted
     # values are memoised per distinct tuple (arrays enter by id(); the objects themselves are kept alive by `params_list`)
     uniq, uniq_of, idx = [], {}, []
+    pcm_rows, pcm_vals = [], []
     widths = rows[:, 6].tolist()
     gs = _get_side
     for r, p in enumerate(params_list):
@@ -161,6 +163,11 @@ def _marshal(params_list):
         ex = p.get("export_sr")                                  # optional key, 0 = none (also when equal to base_sr)
         if ex is not None:
             rows[r, _EXPORT_COL] = 0.0 if P.export_ratio(p) is None else float(ex)
+        if p.get("export_format") is not None:                   # optional key: bits (0 = float32) and dither
+            pcm = P.pcm_format(p)
+            if pcm is not None:
+                pcm_rows.append(r)
+                pcm_vals.append(pcm)
         key = gs(p) + (cap, stereo, id(ir), id(dig), widths[r])
         k = uniq_of.get(key)
         if k is None:
@@ -186,6 +193,8 @@ def _marshal(params_list):
             uniq.append((_MODE[gen_mode], 0.0 if unfold_mode == _CLASSIC else 1.0, _PROCESS[process],
                          lane_id(l0), lane_id(l1), lane_id(l2), lane_id(l3), ir_id, ir_r_id, b))
         idx.append(k)
+    if pcm_rows:
+        rows[np.ix_(pcm_rows, _PCM_COL)] = pcm_vals
     rows[:, _SIDE_COL] = np.array(uniq, dtype=np.float64).reshape(len(uniq), len(_SIDE_COL))[np.array(idx, dtype=np.intp)]
     lane_ptr = np.zeros(len(lanes) + 1, np.int64)
     for i, pts in enumerate(lanes):
@@ -199,6 +208,7 @@ def _marshal(params_list):
 
 
 _EXPORT_COL = FIELDS.index("export_sr")
+_PCM_COL = [FIELDS.index("export_format"), FIELDS.index("export_dither")]
 _SIDE_COL = [FIELDS.index(k) for k in ("gen_mode", "unfold_mode", "event_process", "bp_density", "bp_unfold", "bp_cutoff", "bp_stretch", "_ir", "_ir_r", "_bessel")]
 
 
@@ -238,8 +248,10 @@ def plan_chunk(params_list, threads=None):
         t.out_at, t.out_n, t.y_at = np.zeros(R, np.int64), np.zeros(R, np.int64), np.zeros(R, np.int64)
         t.last, t.srs = np.zeros(R, T.LAST), np.zeros((R, 2), np.int64)
         t.export, t.export_of, ratios = np.zeros(n["export"], t.export.dtype), np.zeros(n["export"], np.int64), np.zeros((n["ratios"], 2), np.int64)
+        t.pcm, t.pcm_of = np.zeros(n["pcm"], t.pcm.dtype), np.zeros(n["pcm"], np.int64)
         args = [t.sy1, t.sy2, t.ola_r, t.env_reps, t.ola_e, t.fir, t.post, t.tap_off, delay, raw, t.dust_pos, t.dust_val,
-                t.tilt, t.grain, t.rot, t.odd, ir_order, t.out_at, t.out_n, t.y_at, t.last, t.srs, t.export, t.export_of, ratios]
+                t.tilt, t.grain, t.rot, t.odd, ir_order, t.out_at, t.out_n, t.y_at, t.last, t.srs, t.export, t.export_of, ratios,
+                t.pcm, t.pcm_of]
         l.ms_hp_export(h, *[a.ctypes.data for a in args])
     finally:
         l.ms_hp_free(h)

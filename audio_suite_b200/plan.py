@@ -263,6 +263,7 @@ class RenderPlan:
     drive: float = 1.0
     peak: float = 0.98
     export: Optional[tuple] = None          # (up, down) of the optional key `export_sr`, or None: delivered at base_sr
+    pcm: Optional[tuple] = None             # (bits, dither, seed mod 2^64) of the optional key `export_format`, or None: float32
     progress_msgs: list = field(default_factory=list)
 
 
@@ -279,6 +280,7 @@ def plan_render(params) -> RenderPlan:
     cap = ir_tap_cap(params)
     stereo_ir = ir_stereo(params)
     export = export_ratio(params)
+    pcm = pcm_format(params)
     base_sr = int(params["base_sr"])
     out_dur = float(params["out_dur_s"])
     out_n = int(max(1, round(out_dur * base_sr)))
@@ -443,6 +445,8 @@ def plan_render(params) -> RenderPlan:
     rp.drive = float(params["sat_drive"])
     rp.peak = float(params["peak"])
     rp.export = export
+    if pcm is not None:
+        rp.pcm = pcm + (seed % (1 << 64),)
     return rp
 
 
@@ -506,6 +510,32 @@ def export_ratio(params):
 def export_frames(n, ratio):
     """Frames of a render of n frames at base_sr after the export resampler: ceil(n up / down)."""
     return n if ratio is None else -(-n * ratio[0] // ratio[1])
+
+
+PCM_FORMATS = {"pcm16": 16, "pcm24": 24}
+
+
+def pcm_format(params):
+    """The optional keys `export_format` and `export_dither` (EXTENSION; the reference returns float samples): integer PCM
+    quantised on the GPU after everything else (include/microsound_b200.h, ms_post_pcm).  Returns (bits, dither) -- bits 16
+    or 24 for "pcm16" / "pcm24", dither 1 for TPDF dither (the default), 0 without -- or None for float32 output (the key
+    absent, None or "float32"; `export_dither` is then not looked at).  Any other value raises ValueError."""
+    fmt = params.get("export_format", None)
+    if fmt is None or isinstance(fmt, str) and fmt == "float32":
+        return None
+    bits = PCM_FORMATS.get(fmt) if isinstance(fmt, str) else None
+    if bits is None:
+        raise ValueError(f"export_format must be None, 'float32', 'pcm16' or 'pcm24', not {fmt!r}")
+    dither = params.get("export_dither", True)
+    if not isinstance(dither, (bool, np.bool_)):
+        raise ValueError(f"export_dither must be a bool, not {dither!r}")
+    return bits, int(bool(dither))
+
+
+def output_slots(n, bits=None):
+    """8-byte slots of the output arena that n frames take: one float32 frame each, ceil(n / 2) for pcm16 and ceil(3 n / 4)
+    for pcm24 (6 bytes a frame).  Every render starts on a slot."""
+    return n if bits is None else (n + 1) // 2 if bits == 16 else (3 * n + 3) // 4
 
 
 _PAIR_CACHE = {}

@@ -11,8 +11,9 @@ Every table is a record array with the layout of its struct in include/microsoun
 workspace can supply (the `z*` spectrum offsets, scratch offsets) stay 0 here and are filled on upload.
 
 Buffers (offsets in elements): pool (real; per-event signals), mono (real; per chunk:
-[OLA plane | FIR plane | right channels / odd-length scratch / right-channel FIR outputs]), out (float32 frames, at the
-export rate of renders with `export_sr`), hpool (real; combined FIR taps), taps (reflection delays/gains), irs
+[OLA plane | FIR plane | right channels / odd-length scratch / right-channel FIR outputs]), out (8-byte slots: one float32
+frame each, or the PCM bytes of renders with `export_format` -- P.output_slots; at the export rate of renders with
+`export_sr`), hpool (real; combined FIR taps), taps (reflection delays/gains), irs
 (deduplicated IR taps), dust (impulses), bank (polyphase banks of the export resampler, one per ratio and chunk).
 """
 from __future__ import annotations
@@ -125,13 +126,15 @@ class Tables:
     export: np.ndarray = _empty(_abi.ExportRender)   # renders with an export rate, in render order ...
     export_of: np.ndarray = _empty(np.int64)         # ... and their render indices
     bank: np.ndarray = _empty(np.float64)            # polyphase banks of the export resampler (decimate.polyphase_bank)
+    pcm: np.ndarray = _empty(_abi.PcmRender)         # renders with integer PCM output, in render order ...
+    pcm_of: np.ndarray = _empty(np.int64)            # ... and their render indices
     pool_n: int = 0
     mono_n: int = 0
-    frames: int = 0
+    frames: int = 0                                  # slots of the output arena
     h_total: int = 0
     max_h: int = 0
     max_out_n: int = 0
-    out_at: np.ndarray = _empty(np.int64)            # per render: first frame
+    out_at: np.ndarray = _empty(np.int64)            # per render: first slot
     out_n: np.ndarray = _empty(np.int64)             # per render: frames (at the export rate, if any)
     y_at: np.ndarray = _empty(np.int64)
     last: np.ndarray = _empty(LAST)
@@ -159,6 +162,7 @@ RELOC = {
     ("out_at", None): ("frames", False), ("y_at", None): ("mono", False),
     ("export", "out"): ("frames", False), ("export", "out_end"): ("frames", False),
     ("export", "bank"): ("bank", False), ("export", "bank_end"): ("bank", False), ("export_of", None): ("renders", False),
+    ("pcm_of", None): ("renders", False),
     ("last", "micro"): ("pool", True), ("last", "grain"): ("pool", True),
 }
 for _t, _buf in (("tilt", "pool"), ("grain", "pool"), ("post_grain", "pool"), ("cep_items", "pool"), ("plock_items", "pool"),
@@ -399,6 +403,7 @@ def pack_chunk(plans) -> Tables:
     odd = []
     out_at, out_n, y_at = np.zeros(R, np.int64), np.zeros(R, np.int64), np.zeros(R, np.int64)
     export, export_of, banks, bank_at, n_bank = [], [], [], {}, 0
+    pcm, pcm_of = [], []
     fir_arr = np.array(fir, np.dtype(_abi.FirRender))
     for r, rp in enumerate(plans):
         n = rp.out_n
@@ -450,8 +455,12 @@ def pack_chunk(plans) -> Tables:
                 n_bank += bk.size
             export.append((frames, frames + n_x, at, at + bk.size, rp.export + (half, taps)))
             export_of.append(r)
+        if rp.pcm is not None:                   # export_format: the frames are stored as PCM bytes in fewer slots
+            bits, dither, seed = rp.pcm
+            pcm.append(((seed & 0xFFFFFFFF, seed >> 32), (bits, dither)))
+            pcm_of.append(r)
         out_at[r], out_n[r], y_at[r] = frames, n_x, y
-        frames += n_x
+        frames += P.output_slots(n_x, None if rp.pcm is None else rp.pcm[0])
         alg["post"] += n
     # envelopes shared by several renders are tabulated once (ms_adsr_tables) instead of one pow() per sample
     env_n = 0
@@ -487,6 +496,8 @@ def pack_chunk(plans) -> Tables:
     if export:
         t.export, t.export_of = np.array(export, t.export.dtype), np.array(export_of, np.int64)
         t.bank = np.concatenate(banks)
+    if pcm:
+        t.pcm, t.pcm_of = np.array(pcm, t.pcm.dtype), np.array(pcm_of, np.int64)
     t.pool_n, t.mono_n, t.frames, t.h_total, t.max_h = pool_n, 2 * plane + extra, frames, h_total, max_h
     t.max_out_n = max((rp.out_n for rp in plans), default=0)
     t.out_at, t.out_n, t.y_at, t.last = out_at, out_n, y_at, last

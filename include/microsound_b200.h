@@ -258,11 +258,31 @@ typedef struct {
  * no renormalisation after the resampler, so inter-sample peaks may exceed `peak`.  Row i of dev_export belongs to row i of
  * dev_renders.  max_n: largest n, max_out_n: largest out_end - out.  Allocates nothing, never synchronises. */
 typedef struct {
-    int64_t out, out_end;     /* output frames [out, out_end) */
+    int64_t out, out_end;     /* output frames [out, out_end); under ms_post_pcm, out is the first slot and out_end - out the
+                                 frame count */
     int64_t bank, bank_end;   /* the render's polyphase bank in the bank pool: up * taps coefficients */
     int32_t rate[4];          /* up, down, half, taps per phase */
 } ms_export_render;
 /* ms_post_export_f32 / ms_post_export_f64: declared below by MS_DECLARE_API */
+/* EXTENSION (the reference delivers float samples): integer PCM output.  ms_post_pcm runs the max pass of ms_post (the
+ * same kernel) on the renders of `dev_renders`, then a write pass that stores each output frame as signed `bits`-bit PCM
+ * instead of float32.  The input of the quantiser is the value the float path rounds to float32 -- soft_clip(.) * scale,
+ * or the resampler's sum when `dev_export` is not NULL (then row i of dev_export belongs to row i of dev_renders, and
+ * out_end - out is its frame count) -- widened to double.  With S = 2^(bits - 1), each channel of output frame i becomes
+ *     q = clamp(rint(x S + d), -S, S - 1)      (rint: round half to even; x S is exact, so one rounding)
+ * d = 0 without dither.  With dither, d is TPDF from Philox4x32-10 (Random123), a pure function of the key and i:
+ * counter (i mod 2^32, i >> 32, 0x64697468, 0), key (key[0], key[1]); of the output words w0..w3, d_L = (w0 - w1) 2^-32,
+ * d_R = (w2 - w3) 2^-32.  Stored form, at byte 8 * out of `out` (`out` counted in 8-byte slots, as a float frame is): little-
+ * endian two's complement, interleaved L, R -- 4 bytes a frame (bits 16) or 6 (bits 24).  A render of n frames (n of
+ * its ms_post_render row, or out_end - out of its export row) owns ceil(n / 2) (16) or ceil(3 n / 4) (24) slots; the
+ * bytes of those slots past its last frame are written as zero.  Every row must carry the call's `bits` (16 or 24) and
+ * `dither` (0 or 1) in `fmt`; a row that does not is left unwritten.  max_n: largest n, max_out_n: largest out_end - out
+ * (with dev_export).  Allocates nothing, never synchronises. */
+typedef struct {
+    uint32_t key[2];          /* Philox key: low and high 32 bits of the render's seed mod 2^64 */
+    int32_t fmt[2];           /* bits (16 or 24), dither (1: TPDF, 0: none) */
+} ms_pcm_render;
+/* ms_post_pcm_f32 / ms_post_pcm_f64: declared below by MS_DECLARE_API */
 
 /* ---- EXTENSION, not on the reference's path (SURVEY a14): band-limited polyphase decimation.  render() never decimates:
  *      the rate change is a relabel (main_v2.py:489-490), the band-limit is lowpass_fft (main_v2.py:39-59).  This stage
@@ -318,6 +338,9 @@ typedef struct {
     float* out, void* stream); \
     int ms_post_export##SFX(const ms_post_render* dev_renders, const ms_export_render* dev_export, int n_renders, int max_n, \
     int max_out_n, REAL* mono, uint64_t* maxbits, const REAL* bank, float* out, void* stream); \
+    int ms_post_pcm##SFX(const ms_post_render* dev_renders, const ms_pcm_render* dev_pcm, const ms_export_render* dev_export, \
+    int n_renders, int max_n, int max_out_n, int bits, int dither, REAL* mono, uint64_t* maxbits, const REAL* bank, void* out, \
+    void* stream); \
     int ms_roll##SFX(const REAL* src, REAL* dst, int n, int shift, void* stream); \
     int ms_polyphase_decimate##SFX(const REAL* x, int64_t x_stride, int n, int n_signals, const REAL* h, int taps, int q, \
     REAL* y, int64_t y_stride, void* stream);

@@ -172,6 +172,7 @@ _STAGES = {
     "ms_post_pcm": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "ms_roll": (_I, [_P, _P, _I, _I, _P]),
     "ms_polyphase_decimate": (_I, [_P, C.c_int64, _I, _I, _P, _I, _I, _P, C.c_int64, _P]),
+    "ms_resample_poly": (_I, [_P, C.c_int64, _I, _I, _P, _I, _I, _I, _I, _P, C.c_int64, _I, _P]),
 }
 PRECISIONS = ("f32", "f64")
 

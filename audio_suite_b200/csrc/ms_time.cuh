@@ -424,6 +424,69 @@ MS_DEV void post_export_body(const PostRender* MS_RESTRICT renders, const Export
         if (BITS == 24) pcm24_flush(c.smem, ob, m0, cnt, c);
     }
 }
+// ---- EXTENSION: batched rational resampler (include/microsound_b200.h, ms_resample_poly; `space_ir_sr` resamples the IR) ----
+// y[s][m] = sum_t x[s][q + t] bank[p][t + A], q = (m down) div up, p = (m down) mod up (zero outside [0, n)): the tap loop of
+// post_export_body for one plain signal.  grid = (ceil(n_out / RS_TILE), signals), OLA_NTHR threads; a thread owns the outputs
+// m0 + tid + OLA_NTHR k.  The window goes through shared memory in rounds of RS_CH samples, every load of a round issued
+// before its first store; each output adds the taps that fall in the round, in ascending t, into one accumulator, so the
+// sum does not depend on the rounds.  (A separate body, not post_export_body with a load policy: that one clips, scales and
+// reads two channels with the stereo roll on load, and keeping the post kernels' SASS unchanged forbids reshaping it.)
+#define RS_TILE 1024                 // outputs per CTA
+#define RS_CH 2048                   // input samples per round of the staged window
+MS_DEV void resample_poly_body(const real* MS_RESTRICT x, long long x_stride, int n, const real* MS_RESTRICT bank, int up, int down,
+                               int half, int taps, real* MS_RESTRICT y, long long y_stride, int n_out, const Ctx& c) {
+    const long long m0 = (long long)c.bx * RS_TILE;
+    if (m0 >= n_out) return;
+    const int cnt = (int)(n_out - m0 < RS_TILE ? n_out - m0 : RS_TILE);
+    const real* xs = x + (long long)c.by * x_stride;
+    const int A = half / up;
+    const long long w0 = m0 * down / up - A;                            // input sample of window slot 0
+    const int wlen = (int)((m0 + cnt - 1) * down / up + (taps - A) - w0);
+    constexpr int NQ = RS_TILE / OLA_NTHR, NL = RS_CH / OLA_NTHR;
+    int rq[NQ];                                  // window slot of q(m), -1: no output
+    const real* tp[NQ];                          // taps of the output's phase, at t = 0
+    real acc[NQ];
+#pragma unroll
+    for (int k = 0; k < NQ; ++k) {
+        const int i = c.tid + OLA_NTHR * k;
+        const long long md = (m0 + i) * down, q = md / up;
+        rq[k] = i < cnt ? (int)(q - w0) : -1;
+        tp[k] = bank + (md - q * up) * taps + A;
+        acc[k] = (real)0.;
+    }
+    real* win = (real*)c.smem;                   // RS_CH samples
+    for (int c0 = 0; c0 < wlen; c0 += RS_CH) {
+        const int clen = wlen - c0 < RS_CH ? wlen - c0 : RS_CH;
+        real v[NL];
+#pragma unroll
+        for (int k = 0; k < NL; ++k) {
+            const int j = c.tid + OLA_NTHR * k;
+            const long long J = w0 + c0 + j;
+            v[k] = (j < clen && J >= 0 && J < n) ? __ldg(&xs[J]) : (real)0.;
+        }
+        if (c0) c.sync();                        // the previous round has been read
+#pragma unroll
+        for (int k = 0; k < NL; ++k) {
+            const int j = c.tid + OLA_NTHR * k;
+            if (j < clen) win[j] = v[k];
+        }
+        c.sync();
+#pragma unroll
+        for (int k = 0; k < NQ; ++k) {
+            if (rq[k] < 0) continue;
+            const int d = rq[k] - c0;            // slot of x[q] in this round
+            const int t_lo = -A > -d ? -A : -d;
+            const int t_hi = taps - 1 - A < clen - 1 - d ? taps - 1 - A : clen - 1 - d;
+            real a = acc[k];
+            for (int t = t_lo; t <= t_hi; ++t) a += __ldg(&tp[k][t]) * win[d + t];
+            acc[k] = a;
+        }
+    }
+    real* ys = y + (long long)c.by * y_stride + m0;
+#pragma unroll
+    for (int k = 0; k < NQ; ++k)
+        if (rq[k] >= 0) ys[c.tid + OLA_NTHR * k] = acc[k];
+}
 // circular shift used by the odd-length stereo path: dst[i] = src[(i + shift) mod n]
 MS_DEV void roll_body(const real* MS_RESTRICT src, real* MS_RESTRICT dst, int n, int shift, const Ctx& c) {
     for (int i = c.bx * c.nthr + c.tid; i < n; i += c.nthr * 64) dst[i] = src[wrap_idx((long long)i + shift, n)];

@@ -67,6 +67,32 @@ def upfirdn_decimate(x, h, q, device, precision="f64"):
     return y[0] if np.ndim(x) == 1 else y
 
 
+def resample_poly(x, up, down, device, precision="f64", n_out=None):
+    """scipy.signal.resample_poly(x, up, down) along axis 0 of `x` ([n] or [n, signals]) on the device
+    (ms_resample_poly, with the filter of polyphase_bank).  Returns ceil(n up / down) rows, or only the first `n_out` of
+    them: every output is its own sum, so those rows are bitwise the rows of the full call."""
+    up, down = int(up), int(down)
+    api = _abi.Api(device.lib, precision)
+    real = np.float32 if precision == "f32" else np.float64
+    a = np.asarray(x)
+    x2 = np.ascontiguousarray(np.atleast_2d(a.T if a.ndim > 1 else a), dtype=real)        # [signals, n]
+    s, n = x2.shape
+    full = -(-n * up // down)
+    n_out = full if n_out is None else max(0, min(int(n_out), full))
+    half, taps, bank = polyphase_bank(up, down)
+    y = np.zeros((s, n_out), real)
+    if n_out and s:
+        dx, db = device.upload(x2), device.upload(bank.astype(real))
+        dy = device.zeros(s * n_out, real)
+        rc = api.ms_resample_poly(device.ptr(dx), n, n, s, device.ptr(db), up, down, half, taps, device.ptr(dy), n_out, n_out,
+                                  device.stream_ptr())
+        if rc != 0:
+            raise RuntimeError("microsound_b200: " + (device.lib.ms_last_error() or b"unknown error").decode())
+        device.synchronize()
+        y = np.asarray(device.download(dy, 0, s * n_out)).view(real).reshape(s, n_out)
+    return np.ascontiguousarray(y.T) if a.ndim > 1 else y[0]
+
+
 def decimate(x, q, device, precision="f64", taps=None):
     """resample_poly(x, 1, q) along the last axis: the Kaiser-windowed FIR above, group delay removed, ceil(n / q) outputs."""
     h = design_taps(q) if taps is None else np.asarray(taps, np.float64)

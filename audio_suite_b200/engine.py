@@ -7,6 +7,7 @@ main_v2.py:1578-1593) as one batched launch sequence on one GPU; `parallel.py` s
 the GPUs of a box.
 
 Stage order (one batched launch sequence for all renders):
+  [before planning, for renders with `space_ir_sr`: the IR resampled to base_sr]  ms_resample_poly
   synth (PCG64 + ziggurat normals, closed-form modes)            ms_synth_normal / ms_synth_dust
   [tilted-noise modes: rfft -> power-law tilt -> irfft, finish]  ms_spectral_* / ms_synth_tilt_finish
   grain spectral op: low-pass -> stretch -> multiband            ms_spectral_*
@@ -202,6 +203,7 @@ class BatchRenderer:
         if tables is not None:
             self.tables, self.plans = tables, None                            # already planned (tables.plan_stream)
         else:
+            params_list = resolve_ir_rate(params_list, self.dev)
             self.tables, self.plans = T.plan_and_pack(params_list, workers)  # plans is None for pooled batches
         self.t_plan = _time.perf_counter() - t0
         self.precision = choose_precision(self.plans) if precision == "auto" else precision
@@ -613,6 +615,54 @@ def _cache_key(params, dev, precision):
     return (items, _array_key(params.get("_ir_audio")), _array_key(params.get("_img_gray")), id(dev), precision)
 
 
+# ---- `space_ir_sr`: the impulse response resampled to base_sr on the device, in the calling process, before any planning (the
+#      planning workers and the native planner's threads never touch the device: they see the float64 result only).  One
+#      resample per distinct (IR, file rate, base_sr, kept rows, kind of device), cached like the planner's tap arrays.
+_IR_RATE_CACHE = {}
+
+
+def _resampled_ir(ir, ratio, rows, key, dev):
+    hit = _IR_RATE_CACHE.get(key)
+    if hit is not None and hit[0] is ir:
+        return hit[1]
+    from . import decimate
+    h = decimate.resample_poly(np.asarray(ir, dtype=np.float64), ratio[0], ratio[1], dev, "f64", n_out=rows)
+    if len(_IR_RATE_CACHE) > 64:
+        _IR_RATE_CACHE.clear()
+    _IR_RATE_CACHE[key] = (ir, h)
+    return h
+
+
+def resolve_ir_rate(params_list, device=None):
+    """`params_list` with every render whose `space_ir_sr` differs from base_sr (IR on and loaded) replaced by a shallow
+    copy carrying its resampled IR under plan.IR_RESAMPLED: resample_poly of every column of `_ir_audio`, float64 from the
+    f64 kernel in both precisions, only the rows plan.ir_rate_rows says the convolution can read.  `_ir_audio` stays as
+    given (the IR fragment generator reads it).  Every value of the key is validated before any device work; the list
+    and its dicts are not modified.  `device`: where to resample (a CudaDevice is opened when it is None and needed)."""
+    todo = []
+    for i, p in enumerate(params_list):
+        if p.get("space_ir_sr") is None:
+            continue
+        ratio = P.ir_rate(p)
+        ir = p.get("_ir_audio")
+        if ratio is not None and ir is not None and p["space_ir_on"] and P.IR_RESAMPLED not in p:
+            todo.append((i, ratio, P.ir_rate_rows(p)))
+    if not todo:
+        return params_list
+    dev = device or CudaDevice()
+    out, memo = list(params_list), {}
+    for i, ratio, rows in todo:
+        p = params_list[i]
+        ir = p["_ir_audio"]
+        k = (id(ir), ratio, rows)
+        h = memo.get(k)
+        if h is None:
+            key = (P.array_signature(ir), int(p["space_ir_sr"]), int(p["base_sr"]), rows, type(dev))
+            h = memo[k] = _resampled_ir(ir, ratio, rows, key, dev)
+        out[i] = {**p, P.IR_RESAMPLED: h}
+    return out
+
+
 def clear_render_cache():
     for br, _ in _RENDER_CACHE.values():
         br.close()
@@ -621,6 +671,7 @@ def clear_render_cache():
 
 def render(params, progress=None, device=None, precision="auto", cache=True):
     """Drop-in for reference render() (main_v2.py:588-792).  `cache=False` plans from scratch every time."""
+    [params] = resolve_ir_rate([params], device)
     key = _cache_key(params, device, precision) if (cache and device is None or (cache and hasattr(device, "torch"))) else None
     hit = _RENDER_CACHE.pop(key, None) if key is not None else None
     if hit is not None:
@@ -730,6 +781,7 @@ def _render_batch(params_list, device=None, precision="auto", host_out=None, chu
         tail = [max(piece, c // 2), max(piece, c // 4), max(piece, c // 4)]
         body = max(0, n - sum(head) - sum(tail))
         chunk = head + [c] * (body // c) + ([body % c] if body % c else []) + tail
+    params_list = resolve_ir_rate(params_list, dev)
     if not hasattr(dev, "torch"):                   # host emulator device (tests): one slice after the other
         outs = []
         for tb in T.plan_stream(params_list, chunk, workers=workers or 1, piece=piece):

@@ -75,18 +75,20 @@ def read_wav(path):
     return a, int(sr)
 
 
-def load_ir_wav(path, stereo=False):
+def load_ir_wav(path, stereo=False, with_rate=False):
     """What on_load_ir hands to render() as `_ir_audio` (main_v2.py:1401-1413): the file as float64, the mean over
     its channels, normalised to a 0.9 peak (normalize, main_v2.py:26-29: untouched when silent).  The file's sample
-    rate is ignored, as in the reference (it is only displayed there).  `stereo=True` (EXTENSION, for
-    `space_ir_stereo`) keeps every channel, float64 [frames, channels], with one gain for all of them so that their
-    balance stays as recorded; a one-channel file gives the same 1-D array either way."""
-    a, _ = read_wav(path)
+    rate is ignored, as in the reference (it is only displayed there); `with_rate=True` (EXTENSION) returns
+    `(ir, file_rate)`, the rate to pass as `space_ir_sr` so that the IR is resampled to base_sr.  `stereo=True`
+    (EXTENSION, for `space_ir_stereo`) keeps every channel, float64 [frames, channels], with one gain for all of them so
+    that their balance stays as recorded; a one-channel file gives the same 1-D array either way."""
+    a, sr = read_wav(path)
     a = a.astype(np.float64)
     if a.ndim > 1 and not stereo:
         a = a.mean(axis=1)
     m = float(np.max(np.abs(a))) if a.size else 0.0
-    return a if m <= 0 else a * (0.9 / m)
+    a = a if m <= 0 else a * (0.9 / m)
+    return (a, sr) if with_rate else a
 
 
 def parse_list(text, cast=float):

@@ -154,6 +154,8 @@ def _marshal(params_list):
     gs = _get_side
     for r, p in enumerate(params_list):
         ir, dig = p.get("_ir_audio"), p.get("_ir_digest")
+        if p.get("space_ir_sr") is not None:                     # optional key: the convolution reads the resampled IR
+            ir = P.conv_ir(p)
         cap = p.get("space_ir_tap_cap", P.IR_TAP_CAP)           # optional keys: not in the itemgetter
         if cap.__class__ is not int or cap < 1:
             cap = P.ir_tap_cap(p)

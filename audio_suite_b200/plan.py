@@ -281,6 +281,7 @@ def plan_render(params) -> RenderPlan:
     stereo_ir = ir_stereo(params)
     export = export_ratio(params)
     pcm = pcm_format(params)
+    ir_conv = conv_ir(params)
     base_sr = int(params["base_sr"])
     out_dur = float(params["out_dur_s"])
     out_n = int(max(1, round(out_dur * base_sr)))
@@ -434,8 +435,8 @@ def plan_render(params) -> RenderPlan:
     if params["space_ir_on"]:
         if digest is not None:
             rp.ir, rp.ir_r = digest["taps"], digest.get("taps_r")
-        elif ir_audio is not None:
-            rp.ir, rp.ir_r = ir_pair(ir_audio, int(params["space_ir_max_samps"]), cap, stereo_ir)
+        elif ir_conv is not None:
+            rp.ir, rp.ir_r = ir_pair(ir_conv, int(params["space_ir_max_samps"]), cap, stereo_ir)
     if params["stereo_on"] and out_n >= 64:   # M:426: shorter outputs are duplicated
         w = float(min(max(float(params["stereo_width"]), 0.0), 1.0))
         rp.stereo_on = True
@@ -505,6 +506,54 @@ def export_ratio(params):
         raise ValueError(f"export_sr {sr} from base_sr {base} is the ratio {up}/{down}: up and down must be at most "
                          f"{EXPORT_RATIO_LIMIT}")
     return up, down
+
+
+IR_RESAMPLED = "_ir_resampled"      # private key: the IR at base_sr under `space_ir_sr` (engine.resolve_ir_rate puts it there)
+
+
+def ir_rate(params):
+    """The optional key `space_ir_sr` (EXTENSION; the reference plays the IR at base_sr whatever its file rate): the rate
+    of `_ir_audio`.  The convolution then reads scipy.signal.resample_poly(ir, up, down) of every column, resampled to
+    base_sr on the device (engine.resolve_ir_rate), and the tap keys count rows of that.  Returns (up, down) in lowest
+    terms, or None when the key is absent, None or equal to int(base_sr).  Only an int >= 1 (numpy's included, not a
+    bool) is taken, with up and down at most EXPORT_RATIO_LIMIT."""
+    sr = params.get("space_ir_sr", None)
+    if sr is None:
+        return None
+    if isinstance(sr, (bool, np.bool_)) or not isinstance(sr, (int, np.integer)) or sr < 1:
+        raise ValueError(f"space_ir_sr must be an int >= 1 or None, not {sr!r}")
+    base, sr = int(params["base_sr"]), int(sr)
+    if sr == base:
+        return None
+    g = math.gcd(base, sr)
+    up, down = base // g, sr // g
+    if max(up, down) > EXPORT_RATIO_LIMIT:
+        raise ValueError(f"space_ir_sr {sr} to base_sr {base} is the ratio {up}/{down}: up and down must be at most "
+                         f"{EXPORT_RATIO_LIMIT}")
+    return up, down
+
+
+def ir_rate_rows(params):
+    """Rows of the resampled IR the convolution can read: min(space_ir_max_samps, max(cap, 8)) -- the "< 8 values" test
+    sees the slice before the cut to `space_ir_tap_cap`, so at least 8 rows are kept for it -- or None for all of them
+    (a negative space_ir_max_samps slices from the end)."""
+    max_samps, cap = int(params["space_ir_max_samps"]), ir_tap_cap(params)
+    if max_samps < 0:
+        return None
+    return max_samps if cap is None else min(max_samps, max(cap, 8))
+
+
+def conv_ir(params):
+    """The impulse response the convolution reads: `_ir_audio`, or under `space_ir_sr` (with the IR on) its resampled rows
+    at IR_RESAMPLED.  The planners never touch the device: a render whose IR has not been resampled is refused."""
+    ir = params.get("_ir_audio")
+    if ir_rate(params) is None or ir is None or not params["space_ir_on"]:
+        return ir
+    h = params.get(IR_RESAMPLED)
+    if h is None:
+        raise ValueError("space_ir_sr: the impulse response has not been resampled to base_sr "
+                         "(engine.resolve_ir_rate runs before planning)")
+    return h
 
 
 def export_frames(n, ratio):
@@ -722,16 +771,18 @@ def _slim_params(p):
     min(space_ir_max_samps, space_ir_tap_cap) rows, None when that slice has fewer than 8 values), "frag": gen_ir_fragment's
     source (M:335-340: the float64 mono mix of the WHOLE response, None when it has fewer than 32 values), "taps_r": the
     right channel under space_ir_stereo (`ir_pair`; "taps" is then the left one), else None}` -- so a
-    multi-second stereo IR is not pickled per render and both size tests are made on the original array.  The
+    multi-second stereo IR is not pickled per render and both size tests are made on the original array.  Under
+    `space_ir_sr` "taps" / "taps_r" come from the resampled IR (conv_ir) and "frag" from `_ir_audio`.  The
     digests are cached per IR object, so renders sharing an IR share the arrays (one pickle memo entry per piece)."""
     ir = p.get("_ir_audio")
     if ir is None or "_ir_digest" in p:
         return p
     q = dict(p)
     q["_ir_audio"] = None
+    q.pop(IR_RESAMPLED, None)
     frag = None
     if p["gen_mode"] == "IR fragment" and np.asarray(ir).size >= 32:
         frag = _mono64(ir)
-    taps, taps_r = ir_pair(ir, int(p["space_ir_max_samps"]), ir_tap_cap(p), ir_stereo(p)) if p["space_ir_on"] else (None, None)
+    taps, taps_r = ir_pair(conv_ir(p),int(p["space_ir_max_samps"]), ir_tap_cap(p), ir_stereo(p)) if p["space_ir_on"] else (None, None)
     q["_ir_digest"] = {"taps": taps, "taps_r": taps_r, "frag": frag}
     return q

@@ -290,6 +290,18 @@ typedef struct {
  *      is "parity unpinned" by the reference.  y[s][m] = sum_k h[k] x[s][m q - k] (zero-extended), m < ceil((n + taps - 1) / q);
  *      taps <= 4096; x_stride / y_stride: elements between consecutive signals. ---- */
 /* ms_polyphase_decimate_f32 / ms_polyphase_decimate_f64: declared below by MS_DECLARE_API */
+/* ---- EXTENSION (the reference plays an impulse response at base_sr whatever its file rate): a batched rational
+ *      resampler.  `space_ir_sr` resamples the IR to base_sr with it before the convolution.  For each of n_signals signals
+ *      of n samples (x_stride / y_stride: elements between consecutive signals) and 0 <= m < n_out,
+ *          y[s][m] = sum_j x[s][j] g[m down - j up + half]      (x zero outside [0, n); g zero outside [0, 2 half]),
+ *      scipy.signal.resample_poly(x, up, down)'s sum when g is its filter and n_out = ceil(n up / down); a smaller n_out
+ *      computes only the first outputs, each bitwise as in the full call.  `bank` is g as the polyphase bank of
+ *      ms_export_render: phase p holds `taps` = half / up + (up - 1 + half) / up + 1 coefficients, entry t + A being
+ *      g[p + half - t up] for t = -A .. taps - 1 - A, A = half / up; with q = (m down) div up, p = (m down) mod up,
+ *      y[s][m] = sum_t x[s][q + t] bank[p][t + A], added in ascending t.  Allocates nothing, never synchronises; bad
+ *      arguments (up, down < 1, half, n, n_signals, n_out < 0, taps that do not match, strides shorter than the signals)
+ *      return -1 with ms_last_error(). ---- */
+/* ms_resample_poly_f32 / ms_resample_poly_f64: declared below by MS_DECLARE_API */
 
 /* ---- entry points.  Every stage exists in two precisions with identical signatures except for the
  *      element type of the signal buffers: suffix _f32 (float) and _f64 (double).  The interleaved stereo
@@ -343,7 +355,9 @@ typedef struct {
     void* stream); \
     int ms_roll##SFX(const REAL* src, REAL* dst, int n, int shift, void* stream); \
     int ms_polyphase_decimate##SFX(const REAL* x, int64_t x_stride, int n, int n_signals, const REAL* h, int taps, int q, \
-    REAL* y, int64_t y_stride, void* stream);
+    REAL* y, int64_t y_stride, void* stream); \
+    int ms_resample_poly##SFX(const REAL* x, int64_t x_stride, int n, int n_signals, const REAL* bank, int up, int down, \
+    int half, int taps, REAL* y, int64_t y_stride, int n_out, void* stream);
 MS_DECLARE_API(_f32, float)
 MS_DECLARE_API(_f64, double)
 
